@@ -29,6 +29,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the tree may be read-only: no byte-code caches written into it
 
 BYTES_PER_PIXRES = 32.0   # 4 B pat_ref + 6*4 B steepest-descent values + 4 B new-frame texel (SURVEY.md §8(d))
 
@@ -297,6 +298,22 @@ def other_configs(ict, dev, cores):
 
 
 KERNEL_NAME = "k_track_r<4,2>"   # the reference-order kernel for psz 32, up to 4 points per track (ict_kernel_r.cu)
+DUMP_BYTES = 60 * 10 ** 6           # --dump-outputs stays below 64 MB, .npy headers included
+
+
+def dump_outputs(out_dir, arrays, suffix=""):
+    """Writes per-track arrays (first axis = track) as <out_dir>/<name><suffix>.npy in float64, at most DUMP_BYTES in
+    all: above that, the rows of a fixed seeded sample of tracks, whose indices go to track_index<suffix>.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.asarray(a, np.float64) for k, a in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    row_bytes = 8 * sum(a[0].size for a in arrays.values())
+    if n * row_bytes > DUMP_BYTES:
+        idx = np.sort(np.random.default_rng(0).choice(n, DUMP_BYTES // (row_bytes + 8), replace=False))
+        arrays = {k: a[idx] for k, a in arrays.items()}
+        arrays["track_index"] = idx.astype(np.float64)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + suffix + ".npy"), a)
 
 
 def main():
@@ -322,7 +339,14 @@ def main():
     ap.add_argument("--strong", action="store_true",
                     help="strong scaling: the 256 sequences of BASELINE configs[4] in total, split over the ranks")
     ap.add_argument("--no-fast", action="store_true", help="skip the fast_mode (tree-order kernels) leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the poses, iteration counts and pixel-residual counts of the last timed step as "
+                         "DIR/p_out.npy, iters.npy, npixres.npy (float64, one row per track)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
 
     rank, world = env_int("RANK", 0), env_int("WORLD_SIZE", 1)
     local_rank = env_int("LOCAL_RANK", 0)
@@ -438,6 +462,9 @@ def main():
     ms_kernel = float(np.mean([ev_k0[k].elapsed_time(ev_k1[k]) for k in range(a.steps)]))
     npix_step = int(d_npix.sum().item())
     iters_mean = float(d_iters.sum(dim=1).double().mean().item())
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, {"p_out": d_pout.cpu().numpy(), "iters": d_iters.cpu().numpy(),
+                                      "npixres": d_npix.cpu().numpy()}, "_rank%d" % rank if world > 1 else "")
 
     # ---- fast mode (opt-in tree-order kernels), device-resident, same workload: reported beside the headline -----
     fast = None
@@ -458,13 +485,12 @@ def main():
             step_fast()
         barrier()
         g0, g1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        nfast = max(3, a.steps)
         g0.record()
-        for _ in range(nfast):
+        for _ in range(a.steps):
             step_fast()
         g1.record()
         barrier()
-        fast = dict(ms=g0.elapsed_time(g1) / nfast, npix=int(f_npix.sum().item()), pout=f_pout, iters=f_iters)
+        fast = dict(ms=g0.elapsed_time(g1) / a.steps, npix=int(f_npix.sum().item()), pout=f_pout, iters=f_iters)
         tr_f.close()
 
     # ---- e2e: host buffers through the C ABI, H2D/D2H inside the timed region ----------------------------

@@ -20,18 +20,6 @@ def orc():
 
 
 @pytest.fixture(scope="session")
-def ref():
-    """The reference's own sources compiled against the stand-in headers; only where oracle/_ref was built."""
-    from oracle import oracle as O
-    if not O.RefLib.available():
-        if os.path.isdir("/root/reference"):
-            O.build("ref")
-        else:
-            pytest.skip("oracle/_ref not built and /root/reference absent")
-    return O.RefLib()
-
-
-@pytest.fixture(scope="session")
 def ict():
     import invcompcamtrack_b200 as ict
     ict.lib()

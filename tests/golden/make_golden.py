@@ -13,6 +13,10 @@ oracle/_ref and Python cv2):   python tests/golden/make_golden.py
                   the reference keeps BETWEEN TrackPose calls (ResetOdometer only runs from Set3Dpoints).
   drivers.npz     inputs and outputs of the reference's own main()s: run_track_nposes.cpp (text in/out, forward and
                   backward chains, NCC) and run_io_reprojection_test.cpp (binary in/out), compiled into oracle/_ref.
+  vs_ref.npz      what tests/test_oracle_vs_ref.py compares with: pyramids (digest + sample), traces, poses,
+                  reprojections and centred points of its seeded cases, camera levels and one batch.  This script
+                  records it from oracle/_ref.  The committed file holds the ORACLE's outputs instead: the reference's
+                  sources were not at hand when it was recorded (see that test's docstring).
 """
 import os
 import sys
@@ -245,6 +249,14 @@ def gen_drivers():
     print("run_io_reprojection_test golden:", pair_out)
 
 
+def gen_vs_ref(ref):
+    """Records from the reference only: an oracle recording would pin the oracle to itself."""
+    assert isinstance(ref, O.RefLib)
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    from helpers import ref_outputs
+    np.savez_compressed(os.path.join(HERE, "vs_ref.npz"), **ref_outputs(ref, O.OracleLib()))
+
+
 if __name__ == "__main__":
     O.build("ref")
     ref = O.RefLib()
@@ -254,4 +266,5 @@ if __name__ == "__main__":
     gen_getpatch(ref)
     gen_drivers()
     gen_drivers_stale()
+    gen_vs_ref(ref)
     print("golden fixtures written to", HERE)

@@ -1,4 +1,6 @@
 """Shared case builders for the parity tests."""
+import hashlib
+
 import numpy as np
 
 from invcompcamtrack_b200 import synth
@@ -194,3 +196,63 @@ def teacher_forced_errors(g, o):
             worst_dp = max(worst_dp, float(np.abs(gt_[k, 8:14] - dpo).max() / dp0))
             nrec += 1
     return worst_jtr, worst_dp, nrec
+
+
+# ---- the seeded cases on which the oracle is compared with the reference's own sources (tests/golden/vs_ref.npz) ----
+REF_CASES = [dict(seed=11), dict(seed=12, donorm=1), dict(seed=13, dopatchnorm=1), dict(seed=14, psz=4, npts=64),
+             dict(seed=15, psz=16, npts=12), dict(seed=16, psz=7, npts=20, donorm=1, dopatchnorm=1),
+             dict(seed=17, psz=32, npts=4, w=1920, h=1080), dict(seed=18, scale=4.0)]
+REF_CAMERAS = (((640, 480), (600.5, 610.25), (321.5, 239.25), 8), ((1920, 1080), (1920, 1920), (960, 540), 32))
+PYR_SAMPLE = 2048          # pyramid values stored per plane beside the digest of the whole plane
+
+
+def digest(*arrays):
+    h = hashlib.sha256()
+    for a in arrays:
+        h.update(np.ascontiguousarray(a).tobytes())
+    return h.hexdigest()
+
+
+def pyramid_sample_index(n, seed):
+    return np.sort(np.random.default_rng(seed).choice(n, size=min(PYR_SAMPLE, n), replace=False))
+
+
+def ref_outputs(lib, orc):
+    """Everything the comparison with the reference records, computed by lib (OracleLib or RefLib), as one dict of
+    arrays: per case k the digest of the seeded inputs, lib's pyramid of the first frame (digest + seeded sample), and
+    Set3Dpoints -> SetPose -> TrackPose on the oracle's pyramids (pose, every iteration's J^T r and delta_p, reference
+    reprojection, possibly centred points); camera levels; the poses of one 12-track batch."""
+    out = {}
+    for k, kw in enumerate(REF_CASES):
+        c = make_case(**kw)
+        lv_f, psz = c["lv_f"], c["psz"]
+        tot, off, sw, sh = O.pyramid_layout(c["w"], c["h"], lv_f, psz)
+        pa = lib.pyramid_build(c["A"].astype(np.float32), lv_f, psz)
+        pa_o = orc.pyramid_build(c["A"].astype(np.float32), lv_f, psz)
+        pb_o = orc.pyramid_build(c["B"].astype(np.float32), lv_f, psz)
+        od = O.Odometer(lib, c["op"], c["sc"].fc, c["sc"].cc, c["sc"].wh)
+        pts = c["pts"].copy()
+        od.set3dpoints(pts)
+        od.setpose(np.zeros(6), pa_o, pb_o, lv_f, off)
+        q = od.get2dpoints()
+        if isinstance(lib, O.RefLib):
+            p, sv = lib.track(od, 96)
+            jtr, dp = sv[:, 36:42], sv[:, 42:48]
+        else:
+            p, it, tr, npx = lib.track(od, 96)
+            jtr, dp = tr[:, 2:8], tr[:, 8:14]
+        od.close()
+        idx = pyramid_sample_index(pa[0].size, k)
+        out.update({"t%d_inputs" % k: digest(c["A"], c["B"], c["pts"]), "t%d_pyr" % k: digest(*pa),
+                    "t%d_pyr_sample" % k: np.stack([a[idx] for a in pa]), "t%d_p" % k: p, "t%d_jtr" % k: jtr,
+                    "t%d_dp" % k: dp, "t%d_q" % k: q, "t%d_pts" % k: pts})
+    for k, (wh, fc, cc, pad) in enumerate(REF_CAMERAS):
+        out["camera%d" % k] = lib.camera_levels(4, fc, cc, wh, pad)
+    c = make_case(seed=19, ntracks=12, npts=24)
+    pa = orc.pyramid_build(c["A"].astype(np.float32), c["lv_f"], c["psz"])
+    pb = orc.pyramid_build(c["B"].astype(np.float32), c["lv_f"], c["psz"])
+    batch = lib.track_batch(c["op"], c["sc"].fc, c["sc"].cc, c["sc"].wh, [pa[0], pb[0]], [pa[1], pb[1]],
+                            [pa[2], pb[2]], c["pt_off"], c["pts"].copy(), np.zeros(12, np.int32), np.ones(12, np.int32),
+                            np.zeros((12, 6)), nthreads=2)
+    out["batch_p_out"] = batch if isinstance(lib, O.RefLib) else batch["p_out"]
+    return out
