@@ -12,6 +12,8 @@ _ERR = {1: "ICT_ERR_NO_DEVICE", 2: "ICT_ERR_BAD_ARG", 3: "ICT_ERR_CUDA", 4: "ICT
 
 
 ROBUST_FULL_STEP, ROBUST_COMPOSE, ROBUST_FLOOR = 1, 2, 4
+# Tracker.set_sum_order (ict_tracker_set_sum_order)
+SUM_ORDER_FAST, SUM_ORDER_EIGEN_SSE, SUM_ORDER_GENERAL_TREE, SUM_ORDER_EIGEN_AVX = 0, 1, 2, 3
 
 
 class IctError(RuntimeError):
@@ -252,7 +254,13 @@ class Tracker:
         self.L = op.lv_f - op.lv_l + 1
 
     def set_sum_order(self, mode):
-        """1 (library default): Eigen packet order, bit-identical to the oracle; 0: fast mode (fixed-order tree sums)."""
+        """Order of the fp32 sums (include/ictrack.h):
+        1 (library default, SUM_ORDER_EIGEN_SSE): Eigen's packet order with 4-float SSE packets, bit-identical to the
+          oracle in its sum mode 0;
+        3 (SUM_ORDER_EIGEN_AVX): the same with 8-float AVX packets, bit-identical to the oracle in its sum mode 1 — a
+          reference built with -mavx against Eigen >= 3.3;
+        0 (SUM_ORDER_FAST): fast mode, fixed-order tree sums;  2: tree sums on the general kernel (tests).
+        Other values raise IctError (ICT_ERR_BAD_ARG)."""
         _check(lib().ict_tracker_set_sum_order(self.h_, int(mode)))
 
     def set_teacher(self, poses):

@@ -25,7 +25,8 @@ class OdometerClass {
 
   // not in the reference: iterations run per level by the last TrackPose (coarse to fine), -1 before the first call
   inline const int* LastIterations() const { return iters; }
-  // 0: fast tree reductions, 1: the reference's summation order (bit-identical results)
+  // the order of the fp32 sums (ict_tracker_set_sum_order): 1 (default) the reference's order with Eigen's 4-float SSE
+  // packets, 3 with its 8-float AVX packets (a reference built with -mavx), 0 fast tree reductions
   void SetSumOrder(int mode);
 
  private:

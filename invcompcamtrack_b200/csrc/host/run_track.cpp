@@ -8,7 +8,8 @@
 //   outfile (binary)                 6 f64 pose                                   (:83-97)
 //   images  binary PGM (P5) instead of whatever cv::imread accepts.
 // Written against the reference's class interface (CamClass / PoseClass / OdometerClass / util_constructpyramide);
-// the alignment itself runs on the GPU.  The reference's summation order is the default; ICT_SUM_ORDER=0 selects the fast mode.
+// the alignment itself runs on the GPU.  The reference's summation order (Eigen's 4-float SSE packets) is the default;
+// ICT_SUM_ORDER=3 selects that order with 8-float AVX packets (a reference built with -mavx), 0 the fast mode.
 #include <sys/time.h>
 
 #include <cstdint>

@@ -12,7 +12,8 @@
 // one NCC launch; only poses and correlations leave the device.  Two quirks of the reference are kept on purpose:
 // its NCC step sets op.dopatchnorm = true and never resets it (:281), so every sample after the first is TRACKED
 // with patch normalisation whatever the input file says; and Set3Dpoints runs once per sample, not per frame.
-// The reference's summation order is the default; ICT_SUM_ORDER=0 selects the fast mode.
+// The reference's summation order (Eigen's 4-float SSE packets) is the default; ICT_SUM_ORDER=3 selects that order with
+// 8-float AVX packets (a reference built with -mavx), 0 the fast mode.
 #include <algorithm>
 #include <cstdio>
 #include <cstdlib>

@@ -461,6 +461,7 @@ struct ict_tracker {
   std::vector<int64_t> h_off;
   bool have_2d = false;
   int sum_mode = 1;            // the reference's summation order is the default (ictrack.h, ict_tracker_set_sum_order)
+  int eigen_packet = 4;        // float packet width of that order: 4 (SSE, the default) or 8 (AVX, sum order 3)
   int force_general = 0;
   int knob_no_k2r = 0, knob_seq_launches = 0;   // ict_tracker_set_knob
   unsigned robust = 0;         // ict_tracker_set_robust
@@ -559,8 +560,11 @@ int ict_tracker_set_knob(ict_tracker* tr, const char* name, int value) {
 }
 
 int ict_tracker_set_sum_order(ict_tracker* tr, int mode) {
-  if (!tr || mode < 0 || mode > 2) return fail(ICT_ERR_BAD_ARG, "sum order must be 1 (reference order, default), 0 (fast tree order) or 2");
-  tr->sum_mode = mode == 1 ? 1 : 0;
+  if (!tr || mode < 0 || mode > 3)
+    return fail(ICT_ERR_BAD_ARG, "sum order must be 1 (reference order, 4-float packets, default), 3 (reference order, "
+                                 "8-float packets), 0 (fast tree order) or 2");
+  tr->sum_mode = (mode == 1 || mode == 3) ? 1 : 0;
+  tr->eigen_packet = mode == 3 ? 8 : 4;
   tr->force_general = mode == 2 ? 1 : 0;
   return ICT_OK;
 }
@@ -678,6 +682,7 @@ static int run_tracks(ict_tracker* tr, const ict_frames* fs, const int* rf_dev, 
   prm.T = tr->T;
   prm.t0 = 0;
   prm.sum_mode = tr->sum_mode;
+  prm.eigen_packet = tr->eigen_packet;
   prm.tma_ok = fs->tma_ok ? 1 : 0;
   prm.force_general = tr->force_general;
   prm.seq_n = tr->seq_n;
@@ -688,7 +693,8 @@ static int run_tracks(ict_tracker* tr, const ict_frames* fs, const int* rf_dev, 
   if (tr->robust && !(tr->sum_mode == 0 && !tr->force_general && v8_supported(tr->op, tr->max_pts)))
     return fail(ICT_ERR_UNSUPPORTED, "robustness modes need the fast mode (sum order 0), psz 8 and at most 240 points per track");
   if (tr->keep_state) {
-    // carried template state: implemented by the reference-order kernel for 8x8 patches (the drivers' configuration)
+    // carried template state: implemented by the reference-order kernel for 8x8 patches (the drivers' configuration),
+    // with either packet width (the carried template does not depend on the order of the sums)
     if (!(tr->sum_mode == 1 && !tr->force_general && tr->op.psz == 8 && kx8_supported(tr->op, tr->max_pts)))
       return fail(ICT_ERR_UNSUPPORTED, "keep_state needs the reference summation order, psz 8 and at most 224 points per track");
     const int P = tr->max_pts < tr->op.maxpttrack ? tr->max_pts : tr->op.maxpttrack;
@@ -711,7 +717,7 @@ static int run_tracks(ict_tracker* tr, const ict_frames* fs, const int* rf_dev, 
     if (rf_dev) return fail(ICT_ERR_UNSUPPORTED, "big tracks take fixed ref/new frames (use ict_track_sequence or T=1)");
     size_t wb = 0;                          // work buffers sized for the largest track, reused in stream order
     for (int t = 0; t < tr->T; ++t) {
-      const size_t w = bigtrack_work_bytes(tr->op, tr->h_off[t + 1] - tr->h_off[t]);
+      const size_t w = bigtrack_work_bytes(tr->op, tr->h_off[t + 1] - tr->h_off[t], tr->eigen_packet);
       wb = w > wb ? w : wb;
     }
     // lanes: as many as there are tracks, at most ICT_BIG_LANES, and only while their work buffers stay below 2 GB

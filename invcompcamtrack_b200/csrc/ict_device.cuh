@@ -730,34 +730,38 @@ __device__ __forceinline__ float warp_sum(float v) {
   return v;
 }
 
-// ---- reference-order reductions (Eigen 3.3 vectorised .sum(), 4-float packets, two accumulators) ----------------
-// Eight interleaved SEQUENTIAL fp32 chains (chain c adds v[c], v[8+c], ...), p0+p1, one odd packet, predux
+// ---- reference-order reductions (Eigen's vectorised .sum(), W-float packets, two accumulators) -------------------
+// W = 4 (SSE Packet4f, Eigen 3.3 built without AVX): eight interleaved SEQUENTIAL fp32 chains; W = 8 (AVX Packet8f):
+// sixteen.  Chain c adds v[c], v[2W+c], ... ; then p0+p1, one odd packet, for W = 8 predux4(lo + hi), predux
 // (a0+a2)+(a1+a3), scalar tail — see oracle/ictrack_oracle.c DEF_PACKET_SUM and ict_kernels.cu (sum_mode 1).
-// chain c of the two-accumulator body: sum over e = c, c+8, ... < as2 (values beyond `valid` are zeros)
-template <typename F>
+// chain c (< 2W) of the two-accumulator body: sum over e = c, c+2W, ... < as2 (values beyond `valid` are zeros)
+template <int W, typename F>
 __device__ __forceinline__ float eigen_chain(F v, int c, int as2, int valid) {
   if (c >= as2) return 0.0f;
   float s = c < valid ? v(c) : 0.0f;
   const int lim = as2 < valid ? as2 : valid;
-  for (int e = c + 8; e < lim; e += 8) s = s + v(e);
+  for (int e = c + 2 * W; e < lim; e += 2 * W) s = s + v(e);
   return s;
 }
-// combine the eight chains + the odd packet + the scalar tail exactly like redux_impl::run
-template <typename F>
+// combine the 2W chains + the odd packet + the scalar tail exactly like redux_impl::run
+template <int W, typename F>
 __device__ __forceinline__ float eigen_finish(const float* ch, F v, int N, int valid) {
-  const int as1 = (N / 4) * 4, as2 = (N / 8) * 8;
+  static_assert(W == 4 || W == 8, "Eigen float packets are 4 (SSE) or 8 (AVX) wide");
+  const int as1 = (N / W) * W, as2 = (N / (2 * W)) * (2 * W);
   auto val = [&](int e) { return e < valid ? v(e) : 0.0f; };
   float res;
   if (N == 0) return 0.0f;
   if (as1) {
-    float p0[4];
-    if (as1 > 4) {
-      for (int j = 0; j < 4; ++j) p0[j] = ch[j] + ch[4 + j];
+    float p0[W];
+    if (as1 > W) {
+      for (int j = 0; j < W; ++j) p0[j] = ch[j] + ch[W + j];
       if (as1 > as2)
-        for (int j = 0; j < 4; ++j) p0[j] = p0[j] + val(as2 + j);
+        for (int j = 0; j < W; ++j) p0[j] = p0[j] + val(as2 + j);
     } else {
-      for (int j = 0; j < 4; ++j) p0[j] = val(j);
+      for (int j = 0; j < W; ++j) p0[j] = val(j);
     }
+    if (W == 8)                                       // predux<Packet8f> = predux(lo + hi)
+      for (int j = 0; j < 4; ++j) p0[j] = p0[j] + p0[j + 4];
     res = (p0[0] + p0[2]) + (p0[1] + p0[3]);
     for (int e = as1; e < N; ++e) res = res + val(e);
   } else {
@@ -767,12 +771,12 @@ __device__ __forceinline__ float eigen_finish(const float* ch, F v, int N, int v
   return res;
 }
 // whole sum by ONE thread (patch means: N = psz*psz)
-template <typename F>
+template <int W, typename F>
 __device__ __forceinline__ float eigen_sum_serial(F v, int N) {
-  float ch[8];
-  const int as2 = (N / 8) * 8;
-  for (int c = 0; c < 8; ++c) ch[c] = eigen_chain(v, c, as2, N);
-  return eigen_finish(ch, v, N, N);
+  float ch[2 * W];
+  const int as2 = (N / (2 * W)) * (2 * W);
+  for (int c = 0; c < 2 * W; ++c) ch[c] = eigen_chain<W>(v, c, as2, N);
+  return eigen_finish<W>(ch, v, N, N);
 }
 
 

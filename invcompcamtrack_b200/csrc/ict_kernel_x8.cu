@@ -16,6 +16,11 @@
 // dopatchnorm in the reference order: the mean of a patch is Eigen's sum of its 64 values, i.e. the same eight
 // column chains followed by the redux tail; a patch lives in one warp, so the chain of column c runs through the four
 // lanes that hold its rows (three shuffles) and the tail through the last row group's lanes.
+//
+// With Eigen's 8-float packets (sum order 3, PK = 8) a sum has sixteen chains: chain c adds e = c, c + 16, ...  For 8x8
+// patches that is chain (row & 1) * 8 + col, four rows of one parity per patch; for 16x16 patches chain c is column
+// c.  In both cases a staged column of eight values holds two chains, the even positions and the odd ones, so the
+// chain lane (k, c) keeps two accumulators per quantity, each half as long, and adds them (p0 + p1) before the tail.
 #include "ict_kernels.cuh"
 #include "ict_device.cuh"
 #include "ict_kernel_v2.cuh"
@@ -30,16 +35,29 @@ void count_launch_external();
 #define X8_MAXR 32                      /* rounds per sum at most: 7 * 32 = 224 points per track */
 
 // Eigen's vectorised sum of the 64 values of a patch held two per lane (rows 2q, 2q+1 of column c; lane = 8q + c):
-// chain c = ((((v[0][c] + v[1][c]) + v[2][c]) + ...) + v[7][c]), then (c0+c4 + c2+c6) + (c1+c5 + c3+c7).
+// PK = 4: chain c = ((((v[0][c] + v[1][c]) + v[2][c]) + ...) + v[7][c]), then (c0+c4 + c2+c6) + (c1+c5 + c3+c7).
+// PK = 8: chains (even rows of c) and (odd rows of c), their sum per column, then the same tail.
 // Returns the sum in every lane.
+template <int PK>
 __device__ __forceinline__ float x8_patch_sum(float a, float b) {
   const unsigned FULL = 0xffffffffu;
   const int q = (threadIdx.x & 31) >> 3;
-  float s = a + b;                                        // rows 0, 1 (valid in row group 0)
+  float s;
+  if (PK == 4) {
+    s = a + b;                                            // rows 0, 1 (valid in row group 0)
 #pragma unroll
-  for (int step = 1; step < 4; ++step) {
-    const float t = __shfl_up_sync(FULL, s, 8);
-    if (q == step) s = (t + a) + b;
+    for (int step = 1; step < 4; ++step) {
+      const float t = __shfl_up_sync(FULL, s, 8);
+      if (q == step) s = (t + a) + b;
+    }
+  } else {
+    float se = a, so = b;                                 // rows 0 and 1 (valid in row group 0)
+#pragma unroll
+    for (int step = 1; step < 4; ++step) {
+      const float te = __shfl_up_sync(FULL, se, 8), to = __shfl_up_sync(FULL, so, 8);
+      if (q == step) { se = te + a; so = to + b; }
+    }
+    s = se + so;                                          // p0[c] + p1[c]
   }
   // lanes 24..31 hold the chains of columns 0..7
   const float p0 = s + __shfl_down_sync(FULL, s, 4);      // lanes 24..27: ch[c] + ch[c+4]
@@ -66,27 +84,47 @@ __device__ __forceinline__ void x8_load(const float* tile, int lane, X8Quads& q)
   q.y0 = q.y1 = make_float4(0.f, 0.f, 0.f, 0.f);
   if (lane < 16) { q.y0 = py[lo]; q.y1 = py[lo ^ 1]; }
 }
-__device__ __forceinline__ void x8_add(const X8Quads& q, bool first, float& sx, float& sy) {
-  sx = first ? q.x0.x : sx + q.x0.x;  sy = first ? q.y0.x : sy + q.y0.x;
-  sx = sx + q.x0.y; sy = sy + q.y0.y; sx = sx + q.x0.z; sy = sy + q.y0.z; sx = sx + q.x0.w; sy = sy + q.y0.w;
-  sx = sx + q.x1.x; sy = sy + q.y1.x; sx = sx + q.x1.y; sy = sy + q.y1.y; sx = sx + q.x1.z; sy = sy + q.y1.z; sx = sx + q.x1.w; sy = sy + q.y1.w;
+// s[0], s[1]: the chains of quantities kx and 4 + kx; with PK = 8 these take the even positions of the column and
+// s[2], s[3] the odd ones
+template <int PK>
+__device__ __forceinline__ void x8_add(const X8Quads& q, bool first, float* s) {
+  if (PK == 4) {
+    float sx = s[0], sy = s[1];
+    sx = first ? q.x0.x : sx + q.x0.x;  sy = first ? q.y0.x : sy + q.y0.x;
+    sx = sx + q.x0.y; sy = sy + q.y0.y; sx = sx + q.x0.z; sy = sy + q.y0.z; sx = sx + q.x0.w; sy = sy + q.y0.w;
+    sx = sx + q.x1.x; sy = sy + q.y1.x; sx = sx + q.x1.y; sy = sy + q.y1.y; sx = sx + q.x1.z; sy = sy + q.y1.z; sx = sx + q.x1.w; sy = sy + q.y1.w;
+    s[0] = sx; s[1] = sy;
+  } else {
+    float xe = s[0], ye = s[1], xo = s[2], yo = s[3];
+    xe = first ? q.x0.x : xe + q.x0.x;  ye = first ? q.y0.x : ye + q.y0.x;
+    xo = first ? q.x0.y : xo + q.x0.y;  yo = first ? q.y0.y : yo + q.y0.y;
+    xe = xe + q.x0.z; ye = ye + q.y0.z; xo = xo + q.x0.w; yo = yo + q.y0.w;
+    xe = xe + q.x1.x; ye = ye + q.y1.x; xo = xo + q.x1.y; yo = yo + q.y1.y;
+    xe = xe + q.x1.z; ye = ye + q.y1.z; xo = xo + q.x1.w; yo = yo + q.y1.w;
+    s[0] = xe; s[1] = ye; s[2] = xo; s[3] = yo;
+  }
 }
-template <int NP>
-__device__ __forceinline__ void x8_consume_round(const float* half, int lane, int j, int ntile, float& sx, float& sy) {
+// the two quantities' chains, combined per lane: the chain of column c (PK = 4) or p0[c] + p1[c] (PK = 8)
+template <int PK>
+__device__ __forceinline__ float2 x8_lane_chains(const float* s) {
+  return PK == 4 ? make_float2(s[0], s[1]) : make_float2(s[0] + s[2], s[1] + s[3]);
+}
+template <int NP, int PK>
+__device__ __forceinline__ void x8_consume_round(const float* half, int lane, int j, int ntile, float* s) {
   X8Quads cur, nxt;
   x8_load(half, lane, cur);
   if ((j + 1) * NP <= ntile) {
 #pragma unroll
     for (int w = 0; w < NP; ++w) {
       if (w + 1 < NP) x8_load(half + (w + 1) * X8_TILE, lane, nxt);
-      x8_add(cur, w == 0 && j == 0, sx, sy);
+      x8_add<PK>(cur, w == 0 && j == 0, s);
       cur = nxt;
     }
   } else {
     const int n = ntile - j * NP;
     for (int w = 0; w < n; ++w) {
       if (w + 1 < n) x8_load(half + (w + 1) * X8_TILE, lane, nxt);
-      x8_add(cur, w == 0 && j == 0, sx, sy);
+      x8_add<PK>(cur, w == 0 && j == 0, s);
       cur = nxt;
     }
   }
@@ -139,7 +177,7 @@ __device__ __forceinline__ float2 x_bilin(const XRows<TPP>& r, const float4 w) {
 // NP = 15: 512 threads, one CTA per SM — a producer's round is ~150 dependent unfused instructions (~900 cycles), so
 // the time of an iteration is rounds x 900 and twice the producers halve it; chosen when only one CTA fits an SM anyway
 // or when the batch is too small to fill the GPU twice (the reference's own use: one track per call).
-template <bool PN, int NP, int TPP>
+template <bool PN, int NP, int TPP, int PK>
 __global__ void __launch_bounds__((NP + 1) * 32, NP == 7 ? 2 : 1) k_track_x8(const TrackParams prm) {
   constexpr int N = 64 * TPP;          // pixels per patch
   extern __shared__ __align__(16) float smem[];
@@ -264,7 +302,7 @@ __global__ void __launch_bounds__((NP + 1) * 32, NP == 7 ? 2 : 1) k_track_x8(con
                          ry = x_load<TPP>(Dyr, o, tt, q2, cc, width);
         float2 r = x_bilin<TPP>(ri, pw);
         if (pnorm) {                     // utilities.cpp:187-188: tmp.sum() / novals, Eigen's order
-          const float m = x8_patch_sum(r.x, r.y) / N;
+          const float m = x8_patch_sum<PK>(r.x, r.y) / N;
           r.x = r.x - m;
           r.y = r.y - m;
         }
@@ -303,15 +341,16 @@ __global__ void __launch_bounds__((NP + 1) * 32, NP == 7 ? 2 : 1) k_track_x8(con
           ++ground;
         }
       } else {
-        float sx = 0.0f, sy = 0.0f;
+        float s4[4] = {0.0f, 0.0f, 0.0f, 0.0f};
         for (int j = 0; j < ROUNDS; ++j) {
           const int h = ground & 1;
           mbar_wait(&S.full[h], (ground >> 1) & 1);
-          x8_consume_round<NP>(s_ring + h * NP * X8_TILE, lane, j, Q, sx, sy);
+          x8_consume_round<NP, PK>(s_ring + h * NP * X8_TILE, lane, j, Q, s4);
           mbar_arrive(&S.empty[h]);
           ++ground;
         }
-        const float rx = kx_finish(sx), ry = kx_finish(sy);
+        const float2 ch = x8_lane_chains<PK>(s4);
+        const float rx = kx_finish(ch.x), ry = kx_finish(ch.y);
         if ((lane & 7) == 0) {
           const int q = 6 * pass + (lane >> 3);
           if (q < 21) S.Hsum[q] = rx;
@@ -334,7 +373,7 @@ __global__ void __launch_bounds__((NP + 1) * 32, NP == 7 ? 2 : 1) k_track_x8(con
     // ---- iterations (odometer.cpp:344-419) ----------------------------------------------------------------------------
     int it = 0;
     while (S.cont) {
-      float sx = 0.0f, sy = 0.0f;
+      float s4[4] = {0.0f, 0.0f, 0.0f, 0.0f};
       if (!chainw) {
         // 7. project_pt + new-frame placement of this warp's patches (7m + warp), lanes = patches
         {
@@ -383,7 +422,7 @@ __global__ void __launch_bounds__((NP + 1) * 32, NP == 7 ? 2 : 1) k_track_x8(con
             if (vis) {
               pn = x_bilin<TPP>(cur.ln, cur.lw);     // util_getPatch (utilities.cpp:55-113), unfused
               if (pnorm) {                           // utilities.cpp:111-112, Eigen's order
-                const float mn = x8_patch_sum(pn.x, pn.y) / N;
+                const float mn = x8_patch_sum<PK>(pn.x, pn.y) / N;
                 pn.x = pn.x - mn;
                 pn.y = pn.y - mn;
               }
@@ -419,14 +458,15 @@ __global__ void __launch_bounds__((NP + 1) * 32, NP == 7 ? 2 : 1) k_track_x8(con
             mbar_wait(&S.full[h], (ground >> 1) & 1);
           }
           const long long tq = trace ? clock64() : 0;
-          x8_consume_round<NP>(s_ring + h * NP * X8_TILE, lane, j, Q, sx, sy);
+          x8_consume_round<NP, PK>(s_ring + h * NP * X8_TILE, lane, j, Q, s4);
           if (trace) tcons += clock64() - tq;
           mbar_arrive(&S.empty[h]);
           ++ground;
         }
         const long long tc1 = trace ? clock64() : 0;
-        // 9a. sumsd[k]: Eigen's redux of the eight chains
-        const float rx = kx_finish(sx), ry = kx_finish(sy);
+        // 9a. sumsd[k]: Eigen's redux of the eight (sixteen) chains
+        const float2 ch = x8_lane_chains<PK>(s4);
+        const float rx = kx_finish(ch.x), ry = kx_finish(ch.y);
         if ((lane & 7) == 0) {
           S.sum[lane >> 3] = rx;
           if (lane < 16) S.sum[4 + (lane >> 3)] = ry;
@@ -518,21 +558,30 @@ bool kx8_supported(const ict_optparam& op, int max_pts) {
   return x8_form_ok(op, max_pts, KX_PROD) || x8_form_ok(op, max_pts, 15);
 }
 
-template <bool PN, int NP, int TPP>
+template <bool PN, int NP, int TPP, int PK>
 static cudaError_t launch_x8_t(const TrackParams& prm, size_t smem, cudaStream_t stream) {
   static bool attr_dev[64] = {};            // function attributes are per device
   int dev_ = 0;
   cudaGetDevice(&dev_);
   bool& attr_set = attr_dev[dev_ & 63];
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(k_track_x8<PN, NP, TPP>, cudaFuncAttributeMaxDynamicSharedMemorySize, ICT_TRACK_SMEM_LIMIT);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_track_x8<PN, NP, TPP>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+    cudaError_t e = cudaFuncSetAttribute(k_track_x8<PN, NP, TPP, PK>, cudaFuncAttributeMaxDynamicSharedMemorySize, ICT_TRACK_SMEM_LIMIT);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_track_x8<PN, NP, TPP, PK>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
     if (e != cudaSuccess) return e;
     attr_set = true;
   }
-  k_track_x8<PN, NP, TPP><<<prm.T, (NP + 1) * 32, smem, stream>>>(prm);
+  k_track_x8<PN, NP, TPP, PK><<<prm.T, (NP + 1) * 32, smem, stream>>>(prm);
   count_launch_external();
   return cudaGetLastError();
+}
+
+template <int PK>
+static cudaError_t launch_x8_pk(const TrackParams& prm, bool wide, size_t smem7, size_t smem15, cudaStream_t stream) {
+  if (prm.op.psz == 16)
+    return wide ? launch_x8_t<false, 15, 4, PK>(prm, smem15, stream) : launch_x8_t<false, 7, 4, PK>(prm, smem7, stream);
+  if (wide)
+    return prm.op.dopatchnorm ? launch_x8_t<true, 15, 1, PK>(prm, smem15, stream) : launch_x8_t<false, 15, 1, PK>(prm, smem15, stream);
+  return prm.op.dopatchnorm ? launch_x8_t<true, 7, 1, PK>(prm, smem7, stream) : launch_x8_t<false, 7, 1, PK>(prm, smem7, stream);
 }
 
 cudaError_t launch_track_x8(const TrackParams& prm, int max_pts, cudaStream_t stream) {
@@ -549,10 +598,8 @@ cudaError_t launch_track_x8(const TrackParams& prm, int max_pts, cudaStream_t st
   // 15 producers where they cost no residency: one CTA per SM anyway (more than 113 KB with 7), or a batch that does not
   // fill the SMs twice
   const bool wide = ok15 && (!ok7 || 2 * (smem7 + 1024) > 228 * 1024 || prm.T <= sms);
-  if (prm.op.psz == 16)
-    return wide ? launch_x8_t<false, 15, 4>(prm, smem15, stream) : launch_x8_t<false, 7, 4>(prm, smem7, stream);
-  if (wide) return prm.op.dopatchnorm ? launch_x8_t<true, 15, 1>(prm, smem15, stream) : launch_x8_t<false, 15, 1>(prm, smem15, stream);
-  return prm.op.dopatchnorm ? launch_x8_t<true, 7, 1>(prm, smem7, stream) : launch_x8_t<false, 7, 1>(prm, smem7, stream);
+  return prm.eigen_packet == 8 ? launch_x8_pk<8>(prm, wide, smem7, smem15, stream)
+                               : launch_x8_pk<4>(prm, wide, smem7, smem15, stream);
 }
 
 }  // namespace ict

@@ -64,6 +64,8 @@ struct TrackParams {
   int r_pcap;                      // K2r: points per track the shared-memory layout is sized for (set by its launcher)
   int sum_mode;                    // 0: fixed-order tree reductions (fast); 1: Eigen-3.3 packet order (bit-exact
                                    //    with the oracle's default model of the reference, ~3x slower)
+  int eigen_packet;                // sum_mode 1 only: float packet width of that order, 4 (SSE, eight chains per sum) or
+                                   //    8 (AVX, sixteen chains); read only by code whose chain count depends on it
 };
 
 #define ICT_TRACK_SMEM_LIMIT (227 * 1024 - 8192)
@@ -97,8 +99,8 @@ size_t v8_smem_bytes(const ict_optparam& op, int max_pts);
 cudaError_t launch_track_v8(const TrackParams& prm, int max_pts, cudaStream_t stream);
 
 // K2x (ict_kernel_x.cu): reference-order (Eigen packet) sums for psz 32 without dopatchnorm — bit-identical to the
-// oracle like k_track<32,2>, with producer warps and one chain warp; launch_track routes sum_mode 1 to it unless
-// ICT_EXACT_V1 is set.
+// oracle like k_track<32,2>, with producer warps and one chain warp; launch_track routes sum_mode 1 with 4-float
+// packets to it unless ICT_EXACT_V1 is set (K2x and K2r run eight chains only).
 size_t kx_smem_bytes(const ict_optparam& op, int max_pts);
 cudaError_t launch_track_x(const TrackParams& prm, int max_pts, cudaStream_t stream);
 
@@ -109,7 +111,7 @@ size_t kr_smem_bytes(const ict_optparam& op, int max_pts);
 cudaError_t launch_track_r(const TrackParams& prm, int max_pts, cudaStream_t stream);
 
 // K2x8 (ict_kernel_x8.cu): reference-order sums for 8x8 patches (up to 224 points per track), with or without
-// dopatchnorm — bit-identical to the oracle like k_track<8,2|3>.
+// dopatchnorm — bit-identical to the oracle like k_track<8,2|3> (4-float packets) and k_track<8,6|7> (8-float packets).
 bool kx8_supported(const ict_optparam& op, int max_pts);
 size_t kx8_smem_bytes(const ict_optparam& op, int max_pts);
 cudaError_t launch_track_x8(const TrackParams& prm, int max_pts, cudaStream_t stream);
@@ -119,7 +121,7 @@ cudaError_t launch_reproject(const TrackParams& prm, cudaStream_t stream);
 
 // multi-CTA path for one big track (dense alignment: psz=1, millions of points)
 struct BigTrackWork;
-size_t bigtrack_work_bytes(const ict_optparam& op, int64_t npts);
+size_t bigtrack_work_bytes(const ict_optparam& op, int64_t npts, int eigen_packet);
 cudaError_t launch_track_big(const TrackParams& prm, int t, int64_t npts, void* work, cudaStream_t stream);
 
 // NCC hypothesis scoring, run_track_nposes.cpp:271-355
