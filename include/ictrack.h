@@ -235,7 +235,8 @@ int ict_track_sequence(ict_tracker* tr, const ict_frames* fs, int first, int nst
 int ict_tracker_reproject(ict_tracker* tr, const double* p_in, float* pt2d_out);
 
 /* Reference 2-D points of the LAST SetPose at level lv_l (OdometerClass::Get2DPoints, odometer.h:30):
- * out float[2*n_t] per track at 2*pt_off[t]: x block then y block. Host buffer. */
+ * out float[2*n_t] per track at 2*pt_off[t]: x block then y block; 0 for the points beyond maxpttrack, which the
+ * reference does not project. Host buffer. */
 int ict_tracker_get_2dpoints(ict_tracker* tr, float* out);
 
 /* ---- stream-ordered host-buffer variants ------------------------------------------------------------------------

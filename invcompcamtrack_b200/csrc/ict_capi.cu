@@ -569,11 +569,13 @@ int ict_tracker_set_sum_order(ict_tracker* tr, int mode) {
   return ICT_OK;
 }
 
-static int tracker_reserve(ict_tracker* tr, int T, int64_t total) {
+static int tracker_reserve(ict_tracker* tr, int T, int64_t total, cudaStream_t st) {
   CU(tr->pt_off.reserve(sizeof(int64_t) * (size_t)(T + 1)));
   CU(tr->pt3d.reserve(sizeof(float) * 3 * (size_t)(total ? total : 1)));
   CU(tr->norm.reserve(sizeof(double) * 4 * (size_t)T));
   CU(tr->pt2d.reserve(sizeof(float) * 2 * (size_t)(total ? total : 1)));
+  // no kernel writes the 2-D points of a track's points beyond maxpttrack: they read 0, not a reused buffer's contents
+  CU(cudaMemsetAsync(tr->pt2d.p, 0, sizeof(float) * 2 * (size_t)total, st));
   return ICT_OK;
 }
 
@@ -586,7 +588,7 @@ int ict_tracker_set_points(ict_tracker* tr, int T, const int64_t* pt_off, double
     if (n < 0 || n > 0x7fffffff) return fail(ICT_ERR_BAD_ARG, "pt_off must be non-decreasing");
     if (n > max_pts) max_pts = (int)n;
   }
-  if (tracker_reserve(tr, T, total)) return ICT_ERR_CUDA;
+  if (tracker_reserve(tr, T, total, 0)) return ICT_ERR_CUDA;
   CU(tr->pts.reserve(sizeof(double) * 3 * (size_t)(total ? total : 1)));
   CU(cudaMemcpyAsync(tr->pt_off.p, pt_off, sizeof(int64_t) * (size_t)(T + 1), cudaMemcpyHostToDevice, 0));
   CU(cudaMemcpyAsync(tr->pts.p, pts, sizeof(double) * 3 * (size_t)total, cudaMemcpyHostToDevice, 0));
@@ -613,7 +615,7 @@ int ict_tracker_set_points_stream(ict_tracker* tr, int T, const int64_t* pt_off,
     if (n < 0 || n > 0x7fffffff) return fail(ICT_ERR_BAD_ARG, "pt_off must be non-decreasing");
     if (n > max_pts) max_pts = (int)n;
   }
-  if (tracker_reserve(tr, T, total)) return ICT_ERR_CUDA;
+  if (tracker_reserve(tr, T, total, st)) return ICT_ERR_CUDA;
   CU(tr->pts.reserve(sizeof(double) * 3 * (size_t)(total ? total : 1)));
   CU(tr->lane.begin());
   CU(cudaMemcpyAsync(tr->pt_off.p, pt_off, sizeof(int64_t) * (size_t)(T + 1), cudaMemcpyHostToDevice, tr->lane.s));
@@ -636,7 +638,7 @@ int ict_tracker_set_points_dev(ict_tracker* tr, int T, const int64_t* pt_off_dev
   if (!tr || T <= 0 || !pt_off_dev || !pts_dev || max_pts <= 0)
     return fail(ICT_ERR_BAD_ARG, "ict_tracker_set_points_dev: bad argument");
   cudaStream_t st = (cudaStream_t)stream;
-  if (tracker_reserve(tr, T, total_pts)) return ICT_ERR_CUDA;
+  if (tracker_reserve(tr, T, total_pts, st)) return ICT_ERR_CUDA;
   CU(cudaMemcpyAsync(tr->pt_off.p, pt_off_dev, sizeof(int64_t) * (size_t)(T + 1), cudaMemcpyDeviceToDevice, st));
   CU(launch_set_points(T, tr->pt_off.as<int64_t>(), pts_dev, nullptr, tr->pt3d.as<float>(), tr->norm.as<double>(),
                        tr->op.donorm, tr->op.maxpttrack, max_pts, st));
@@ -647,6 +649,11 @@ int ict_tracker_set_points_dev(ict_tracker* tr, int T, const int64_t* pt_off_dev
   tr->have_2d = false;
   tr->state_valid = false;
   return ICT_OK;
+}
+
+static TrackKernel tracker_kernel(const ict_tracker* tr, const ict_frames* fs) {
+  return select_track_kernel(tr->op, tr->max_pts, tr->sum_mode, tr->eigen_packet, tr->force_general, tr->knob_no_k2r,
+                             fs->tma_ok);
 }
 
 // SetPose + TrackPose for all tracks; every pointer is device memory.
@@ -690,12 +697,13 @@ static int run_tracks(ict_tracker* tr, const ict_frames* fs, const int* rf_dev, 
   prm.knob_no_k2r = tr->knob_no_k2r;
   prm.knob_seq_launches = tr->knob_seq_launches;
   prm.robust = tr->robust;
-  if (tr->robust && !(tr->sum_mode == 0 && !tr->force_general && v8_supported(tr->op, tr->max_pts)))
+  const TrackKernel kern = tracker_kernel(tr, fs);
+  if (tr->robust && kern != TrackKernel::V8)
     return fail(ICT_ERR_UNSUPPORTED, "robustness modes need the fast mode (sum order 0), psz 8 and at most 240 points per track");
   if (tr->keep_state) {
     // carried template state: implemented by the reference-order kernel for 8x8 patches (the drivers' configuration),
     // with either packet width (the carried template does not depend on the order of the sums)
-    if (!(tr->sum_mode == 1 && !tr->force_general && tr->op.psz == 8 && kx8_supported(tr->op, tr->max_pts)))
+    if (kern != TrackKernel::X8 || tr->op.psz != 8)
       return fail(ICT_ERR_UNSUPPORTED, "keep_state needs the reference summation order, psz 8 and at most 224 points per track");
     const int P = tr->max_pts < tr->op.maxpttrack ? tr->max_pts : tr->op.maxpttrack;
     prm.state_stride = (int64_t)(3 * 64 + 12) * P;
@@ -705,11 +713,7 @@ static int run_tracks(ict_tracker* tr, const ict_frames* fs, const int* rf_dev, 
     prm.state = tr->state.as<float>();
     prm.state_load = tr->state_valid ? 1 : 0;
   }
-  // profiling builds only (ict_knobs.h): these change what the kernels compute or where their serial sections run
-  prm.dbg_skip_serial = ict_knob("ICT_DBG_SKIP_SERIAL") ? atoi(ict_knob("ICT_DBG_SKIP_SERIAL")) : 0;
-  prm.serial_warp_last = ict_knob("ICT_SERIAL_WARP_LAST") ? 1 : 0;
-  prm.v2_lu_setup = ict_knob("ICT_V2_LU") ? 1 : 0;
-  if (track_fits_one_cta(tr->op, tr->max_pts, tr->sum_mode, tr->force_general)) {
+  if (kern != TrackKernel::MultiCta) {
     CU(launch_track(prm, tr->max_pts, st));
   } else {
     // tracks too large for one CTA's shared memory: multi-CTA path, one track at a time
@@ -783,7 +787,7 @@ int ict_track_batch(ict_tracker* tr, const ict_frames* fs, const int* ref_frame,
   CU(cudaMemcpyAsync(tr->rf.p, ref_frame, sizeof(int) * (size_t)T, cudaMemcpyHostToDevice, 0));
   CU(cudaMemcpyAsync(tr->nf.p, new_frame, sizeof(int) * (size_t)T, cudaMemcpyHostToDevice, 0));
   CU(cudaMemcpyAsync(tr->p_in.p, p_in, sizeof(double) * 6 * (size_t)T, cudaMemcpyHostToDevice, 0));
-  const bool big = !track_fits_one_cta(tr->op, tr->max_pts, tr->sum_mode, tr->force_general);
+  const bool big = tracker_kernel(tr, fs) == TrackKernel::MultiCta;
   int rc;
   if (big) {
     // multi-CTA path: the tracks run one after the other on the stream, each with its own frame pair
@@ -815,7 +819,7 @@ int ict_track_batch_stream(ict_tracker* tr, const ict_frames* fs, const int* ref
   cudaStream_t st = (cudaStream_t)stream;
   const int T = tr->T;
   if (T <= 0) return fail(ICT_ERR_BAD_ARG, "no points set");
-  if (!track_fits_one_cta(tr->op, tr->max_pts, tr->sum_mode, tr->force_general))
+  if (tracker_kernel(tr, fs) == TrackKernel::MultiCta)
     return fail(ICT_ERR_UNSUPPORTED, "stream variant handles tracks that fit one CTA");
   for (int t = 0; t < T; ++t)
     if (ref_frame[t] < 0 || ref_frame[t] >= fs->nframes || new_frame[t] < 0 || new_frame[t] >= fs->nframes)
@@ -859,7 +863,7 @@ int ict_track_sequence(ict_tracker* tr, const ict_frames* fs, int first, int nst
   CU(tr->npix.reserve(sizeof(long long) * (size_t)T * (nsteps ? nsteps : 1)));
   double* chain = tr->p_out.as<double>();
   CU(cudaMemcpyAsync(chain, p_in, sizeof(double) * 6 * (size_t)T, cudaMemcpyHostToDevice, 0));
-  if (nsteps > 1 && track_chain_in_one_launch(tr->op, tr->max_pts, tr->sum_mode, tr->force_general, tr->knob_seq_launches)) {
+  if (nsteps > 1 && tracker_kernel(tr, fs) == TrackKernel::V8 && !tr->knob_seq_launches) {
     // K2v8 loops over the frames inside the kernel: one launch for the whole chain
     tr->seq_n = nsteps;
     tr->seq_step = step;

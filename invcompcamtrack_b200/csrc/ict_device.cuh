@@ -301,56 +301,11 @@ struct Lu6 {
   int qc[6];      // x[j] = c[qc[j]] (inverse of qd), for the lane-parallel solve
 };
 
-static __device__ __noinline__ void lu6_factor(const float* H, Lu6& f) {
-#define LU(i, j) f.lu[(i) + 6 * (j)]
-  for (int k = 0; k < 36; ++k) f.lu[k] = H[k];
-  int nonzero = 6;
-  float maxpivot = 0.0f;
-  for (int k = 0; k < 6; ++k) {
-    int pr = k, pc = k;
-    float biggest = -1.0f;
-    for (int j = k; j < 6; ++j)
-      for (int i = k; i < 6; ++i) {
-        float v = fabsf(LU(i, j));
-        if (v > biggest) { biggest = v; pr = i; pc = j; }
-      }
-    if (biggest == 0.0f) {
-      nonzero = k;
-      for (int i = k; i < 6; ++i) { f.rowtr[i] = i; f.coltr[i] = i; }
-      break;
-    }
-    if (biggest > maxpivot) maxpivot = biggest;
-    f.rowtr[k] = pr;
-    f.coltr[k] = pc;
-    if (k != pr) for (int j = 0; j < 6; ++j) { float t = LU(k, j); LU(k, j) = LU(pr, j); LU(pr, j) = t; }
-    if (k != pc) for (int i = 0; i < 6; ++i) { float t = LU(i, k); LU(i, k) = LU(i, pc); LU(i, pc) = t; }
-    if (k < 5) {
-      for (int i = k + 1; i < 6; ++i) LU(i, k) = LU(i, k) / LU(k, k);
-      for (int j = k + 1; j < 6; ++j)
-        for (int i = k + 1; i < 6; ++i) LU(i, j) = LU(i, j) - LU(i, k) * LU(k, j);
-    }
-  }
-  const float premult = fabsf(maxpivot) * (1.1920929e-07f * 6.0f);
-  int rank = 0;
-  for (int i = 0; i < nonzero; ++i) rank += (fabsf(LU(i, i)) > premult);
-  f.rank = rank;
-  int qc[6];   // x[j] = c[qc[j]]
-  for (int k = 0; k < 6; ++k) { f.pr[k] = k; qc[k] = k; }
-  for (int k = 0; k < 6; ++k)
-    if (f.rowtr[k] != k) { const int t = f.pr[k]; f.pr[k] = f.pr[f.rowtr[k]]; f.pr[f.rowtr[k]] = t; }
-  for (int k = 5; k >= 0; --k)
-    if (f.coltr[k] != k) { const int t = qc[k]; qc[k] = qc[f.coltr[k]]; qc[f.coltr[k]] = t; }
-  for (int j = 0; j < 6; ++j) { f.qd[qc[j]] = j; f.qc[j] = qc[j]; }
-  for (int j = 0; j < 6; ++j) f.rdiag[j] = 1.0f / LU(j, j);
-#undef LU
-}
-
-// Warp-cooperative form of lu6_factor: the SAME full-pivoting elimination (same pivot choice — first maximum in
-// column-major order —, same divisions, same rank-1 updates, hence the same bits), with lane j < 6 holding column j
-// of the matrix in six registers.  The pivot search is a per-lane scan plus a three-step butterfly, the row swap is
+// Eigen's full-pivoting elimination (pivot = first maximum in column-major order, the same divisions and rank-1
+// updates, hence the same bits) by one warp, with lane j < 6 holding column j of the matrix in six registers.  The pivot search is a per-lane scan plus a three-step butterfly, the row swap is
 // register renaming under predicates, the column swap and the broadcast of the scaled pivot column are shuffles.
 // Called by all 32 lanes of one warp; Hs = the 21 unique sums in the order of ComputeHessian (odometer.cpp:430-455).
-// The single-thread version costs ~26 000 SM cycles per level on a busy SM (dynamic indexing -> local memory,
+// A single-thread version cost ~26 000 SM cycles per level on a busy SM (dynamic indexing -> local memory,
 // one long dependent chain) while every other warp of the CTA waits; this one ~2 000.
 __device__ __forceinline__ void lu6_factor_warp(const float* Hs, Lu6& f) {
   const int lane = threadIdx.x & 31;
@@ -447,32 +402,6 @@ __device__ __forceinline__ void lu6_factor_warp(const float* Hs, Lu6& f) {
   }
   if (lane == 0) f.rank = __popc(ok);
   __syncwarp();
-}
-
-// The same solve as lu6_solve for a full-rank factorisation, as straight-line code: identical operations in
-// identical order (column-oriented unit-lower forward substitution, then upper backward substitution), no loops
-// over run-time bounds and no dynamically indexed locals.  f, b and x live in shared memory.
-__device__ __forceinline__ void lu6_solve_full(const Lu6& f, const float* b, float* x) {
-#define LU(i, j) f.lu[(i) + 6 * (j)]
-  float c0 = b[f.pr[0]], c1 = b[f.pr[1]], c2 = b[f.pr[2]], c3 = b[f.pr[3]], c4 = b[f.pr[4]], c5 = b[f.pr[5]];
-  c1 = c1 - c0 * LU(1, 0); c2 = c2 - c0 * LU(2, 0); c3 = c3 - c0 * LU(3, 0); c4 = c4 - c0 * LU(4, 0); c5 = c5 - c0 * LU(5, 0);
-  c2 = c2 - c1 * LU(2, 1); c3 = c3 - c1 * LU(3, 1); c4 = c4 - c1 * LU(4, 1); c5 = c5 - c1 * LU(5, 1);
-  c3 = c3 - c2 * LU(3, 2); c4 = c4 - c2 * LU(4, 2); c5 = c5 - c2 * LU(5, 2);
-  c4 = c4 - c3 * LU(4, 3); c5 = c5 - c3 * LU(5, 3);
-  c5 = c5 - c4 * LU(5, 4);
-  c5 = c5 / LU(5, 5);
-  c0 = c0 - c5 * LU(0, 5); c1 = c1 - c5 * LU(1, 5); c2 = c2 - c5 * LU(2, 5); c3 = c3 - c5 * LU(3, 5); c4 = c4 - c5 * LU(4, 5);
-  c4 = c4 / LU(4, 4);
-  c0 = c0 - c4 * LU(0, 4); c1 = c1 - c4 * LU(1, 4); c2 = c2 - c4 * LU(2, 4); c3 = c3 - c4 * LU(3, 4);
-  c3 = c3 / LU(3, 3);
-  c0 = c0 - c3 * LU(0, 3); c1 = c1 - c3 * LU(1, 3); c2 = c2 - c3 * LU(2, 3);
-  c2 = c2 / LU(2, 2);
-  c0 = c0 - c2 * LU(0, 2); c1 = c1 - c2 * LU(1, 2);
-  c1 = c1 / LU(1, 1);
-  c0 = c0 - c1 * LU(0, 1);
-  c0 = c0 / LU(0, 0);
-  x[f.qd[0]] = c0; x[f.qd[1]] = c1; x[f.qd[2]] = c2; x[f.qd[3]] = c3; x[f.qd[4]] = c4; x[f.qd[5]] = c5;
-#undef LU
 }
 
 static __device__ __noinline__ void lu6_solve(const Lu6& f, const float* b, float* x) {
@@ -577,37 +506,12 @@ __device__ __forceinline__ void lu6_solve_regs(const float* lu, int rank, const 
 #undef LU
 }
 
-// Production-kernel variant of lu6_solve_full: the six divisions by the pivots become multiplications by their
-// (correctly rounded, once per level) reciprocals.  Differs from the reference's x / u by at most one ulp per
-// division — far below what the fp32 right-hand side carries — and removes six ~10-deep dependent chains from
-// the code the whole CTA waits for.
-__device__ __forceinline__ void lu6_solve_full_rcp(const Lu6& f, const float* b, float* x) {
-#define LU(i, j) f.lu[(i) + 6 * (j)]
-  float c0 = b[f.pr[0]], c1 = b[f.pr[1]], c2 = b[f.pr[2]], c3 = b[f.pr[3]], c4 = b[f.pr[4]], c5 = b[f.pr[5]];
-  c1 = c1 - c0 * LU(1, 0); c2 = c2 - c0 * LU(2, 0); c3 = c3 - c0 * LU(3, 0); c4 = c4 - c0 * LU(4, 0); c5 = c5 - c0 * LU(5, 0);
-  c2 = c2 - c1 * LU(2, 1); c3 = c3 - c1 * LU(3, 1); c4 = c4 - c1 * LU(4, 1); c5 = c5 - c1 * LU(5, 1);
-  c3 = c3 - c2 * LU(3, 2); c4 = c4 - c2 * LU(4, 2); c5 = c5 - c2 * LU(5, 2);
-  c4 = c4 - c3 * LU(4, 3); c5 = c5 - c3 * LU(5, 3);
-  c5 = c5 - c4 * LU(5, 4);
-  c5 = c5 * f.rdiag[5];
-  c0 = c0 - c5 * LU(0, 5); c1 = c1 - c5 * LU(1, 5); c2 = c2 - c5 * LU(2, 5); c3 = c3 - c5 * LU(3, 5); c4 = c4 - c5 * LU(4, 5);
-  c4 = c4 * f.rdiag[4];
-  c0 = c0 - c4 * LU(0, 4); c1 = c1 - c4 * LU(1, 4); c2 = c2 - c4 * LU(2, 4); c3 = c3 - c4 * LU(3, 4);
-  c3 = c3 * f.rdiag[3];
-  c0 = c0 - c3 * LU(0, 3); c1 = c1 - c3 * LU(1, 3); c2 = c2 - c3 * LU(2, 3);
-  c2 = c2 * f.rdiag[2];
-  c0 = c0 - c2 * LU(0, 2); c1 = c1 - c2 * LU(1, 2);
-  c1 = c1 * f.rdiag[1];
-  c0 = c0 - c1 * LU(0, 1);
-  c0 = c0 * f.rdiag[0];
-  x[f.qd[0]] = c0; x[f.qd[1]] = c1; x[f.qd[2]] = c2; x[f.qd[3]] = c3; x[f.qd[4]] = c4; x[f.qd[5]] = c5;
-#undef LU
-}
-
-// lu6_solve_full_rcp spread over six lanes (called by a full warp, rank 6): lane r carries c_r; one shuffle per
-// elimination step broadcasts the pivot row's value.  Same operations per unknown, in the same order, as the
-// straight-line version — about 50 issued instructions instead of 130 on the warp every other warp waits for.
-// Returns x_lane (valid in lanes 0..5).
+// The full-rank solve of the fast-mode kernels, spread over six lanes (called by a full warp, rank 6): lane r carries
+// c_r; one shuffle per elimination step broadcasts the pivot row's value.  Forward and backward substitution in
+// lu6_solve's order, but the six divisions by the pivots are multiplications by their (correctly rounded, once per
+// level) reciprocals: at most one ulp per division from the reference's x / u — far below what the fp32 right-hand
+// side carries — and no ~10-deep dependent division chains in the code the whole CTA waits for.  About 50 issued
+// instructions instead of 130 for the straight-line single-lane form.  Returns x_lane (valid in lanes 0..5).
 __device__ __forceinline__ float lu6_solve_warp_rcp(const Lu6& f, const float* b) {
   const unsigned FULL = 0xffffffffu;
   const int lane = threadIdx.x & 31, r = lane < 6 ? lane : 0;

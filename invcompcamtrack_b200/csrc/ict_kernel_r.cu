@@ -706,7 +706,6 @@ static cudaError_t launch_track_r_t(const TrackParams& prm, size_t smem, cudaStr
 
 cudaError_t launch_track_r(const TrackParams& prm_in, int max_pts, cudaStream_t stream) {
   if (prm_in.T <= 0) return cudaSuccess;
-  if (!kr_supported(prm_in.op, max_pts, prm_in.tma_ok)) return cudaErrorInvalidConfiguration;
   TrackParams prm = prm_in;
   prm.r_pcap = kr_pcap(prm.op, max_pts);
   const size_t smem = kr_smem_bytes(prm.op, max_pts);

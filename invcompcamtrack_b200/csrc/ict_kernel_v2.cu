@@ -32,8 +32,6 @@
 #include "ict_device.cuh"
 #include "ict_kernel_v2.cuh"
 
-#include <cstdlib>
-
 namespace ict {
 
 void count_launch_external();
@@ -76,7 +74,6 @@ __global__ void __launch_bounds__(NT, MINB) k_track_v2(const TrackParams prm) {
   const int nf = prm.new_frame ? prm.new_frame[t] : prm.fixed_new;
   const FrameDesc* fr_ref = prm.frames + rf;
   const FrameDesc* fr_new = prm.frames + nf;
-  const int swarp = prm.serial_warp_last ? nw - 1 : 0;
 
   // ---- ResetOdometer (odometer.cpp:580-609) + points -----------------------------------------------------------------
   {
@@ -111,12 +108,12 @@ __global__ void __launch_bounds__(NT, MINB) k_track_v2(const TrackParams prm) {
 
   float* trace = TRACE && prm.trace ? prm.trace + (int64_t)t * prm.trace_cap * ICT_TRACE_FLOATS : nullptr;
   int trace_n = 0;
-  // state of the serial warp, identical in all its lanes unless noted
+  // state of the serial warp (warp 0), identical in all its lanes unless noted
   float pk = 0.0f;              // lane (k + 8j) carries pose coefficient k (0 for k = 6, 7)
   float normdp_init = 1e-10f;
   int nv = 0;                   // points visible in the new frame at the placements of the coming iteration
   int nvsum = 0;                // sum of nv over all iterations done: pixel-residuals = nvsum * 1024
-  if (warp == swarp) pk = (lane & 7) < 6 ? S.p[lane & 7] : 0.0f;
+  if (warp == 0) pk = (lane & 7) < 6 ? S.p[lane & 7] : 0.0f;
 
   for (int sl = op.lv_f; sl >= op.lv_l; --sl) {
     const float fx = prm.cam.fx[sl], fy = prm.cam.fy[sl], cx = prm.cam.cx[sl], cy = prm.cam.cy[sl];
@@ -182,7 +179,7 @@ __global__ void __launch_bounds__(NT, MINB) k_track_v2(const TrackParams prm) {
     __syncthreads();
 
     // ---- 6b. Hessian from the per-point sums, the level's solve matrix, first placement -----------------------------------
-    if (warp == swarp) {
+    if (warp == 0) {
       const long long t_lv0 = TRACE ? clock64() : 0;
       if (TRACE && lane == 0) S.gather_cycles = (float)(t_lv0 - t_g0);
       if (lane < 21) {
@@ -210,12 +207,7 @@ __global__ void __launch_bounds__(NT, MINB) k_track_v2(const TrackParams prm) {
       S.Hinv[lane] = 0.0f;
       S.Hinv[32 + lane] = 0.0f;
       __syncwarp();
-      if (prm.v2_lu_setup) {             // A/B knob (ICT_V2_LU): Eigen's elimination itself, then M column by column
-        lu6_factor_warp(S.Hsum, S.f);
-        if (lane < 6) lu6_solve_matrix_column(S.f, lane, S.Hinv + lane);
-      } else {
-        sweep6_solve_matrix(lane < 21 ? S.Hsum[lane] : 0.0f, S.Hinv);
-      }
+      sweep6_solve_matrix(lane < 21 ? S.Hsum[lane] : 0.0f, S.Hinv);
       float Gr[12];
 #pragma unroll
       for (int k = 0; k < 12; ++k) Gr[k] = S.G[k];
@@ -283,7 +275,7 @@ __global__ void __launch_bounds__(NT, MINB) k_track_v2(const TrackParams prm) {
       __syncthreads();
 
       // ---- serial section: one warp, every lane active, ~250 instructions --------------------------------------------
-      if (warp == swarp) {
+      if (warp == 0) {
         const long long t_ser0 = TRACE ? clock64() : 0;
         const unsigned FULL = 0xffffffffu;
         const int k = lane & 7, k6 = k < 6 ? k : 0, j4 = lane >> 3;
@@ -398,7 +390,7 @@ __global__ void __launch_bounds__(NT, MINB) k_track_v2(const TrackParams prm) {
     if (tid == 0 && prm.iters) prm.iters[(int64_t)t * (op.lv_f - op.lv_l + 1) + (op.lv_f - sl)] = S.it;
   }
 
-  if (warp == swarp && lane == 0) {
+  if (warp == 0 && lane == 0) {
     getpose_se3(S.p, S.G, donorm, prm.norm + 4 * (int64_t)t, prm.norm[4 * (int64_t)t + 3],
                 prm.p_out + 6 * (int64_t)t);
     if (prm.npixres) prm.npixres[t] = (long long)nvsum * N;
@@ -425,10 +417,8 @@ static cudaError_t launch_v2_t(const TrackParams& prm, size_t smem, cudaStream_t
   if (!attr_set) {
     cudaError_t e = cudaFuncSetAttribute(k_track_v2<KT, MINB, TRACE, NT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          ICT_TRACK_SMEM_LIMIT);
-    const char* co = ict_knob("ICT_V2_CARVEOUT");      // profiling knob: shared-memory carve-out in percent
     if (e == cudaSuccess)
-      e = cudaFuncSetAttribute(k_track_v2<KT, MINB, TRACE, NT>, cudaFuncAttributePreferredSharedMemoryCarveout,
-                               co ? atoi(co) : 100);
+      e = cudaFuncSetAttribute(k_track_v2<KT, MINB, TRACE, NT>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
     if (e != cudaSuccess) return e;
     attr_set = true;
   }
@@ -440,25 +430,15 @@ static cudaError_t launch_v2_t(const TrackParams& prm, size_t smem, cudaStream_t
 cudaError_t launch_track_v2(const TrackParams& prm, int max_pts, cudaStream_t stream) {
   if (prm.T <= 0) return cudaSuccess;
   const size_t smem = v2_smem_bytes(prm.op, max_pts);
-  if (smem > (size_t)ICT_TRACK_SMEM_LIMIT) return cudaErrorInvalidConfiguration;
-  static int variant = -1;
-  if (variant < 0) {
-    const char* e = ict_knob("ICT_V2_VARIANT");       // tuning knob for profiling runs only
-    variant = e ? atoi(e) : 0;
-  }
   // More points per track = more template per CTA = fewer CTAs per SM: keep ~32 warps per SM by giving the track more
   // warps (a warp still owns 16 rows of one point at a time; per-group sums make the result independent of it).
   const int P = max_pts < prm.op.maxpttrack ? max_pts : prm.op.maxpttrack;
-  if (P > 8 && !ict_knob("ICT_V2_256"))
+  if (P > 8)
     return prm.trace ? launch_v2_t<16, 1, true, 1024>(prm, smem, stream) : launch_v2_t<16, 1, false, 1024>(prm, smem, stream);
-  if (P > 4 && !ict_knob("ICT_V2_256"))
+  if (P > 4)
     return prm.trace ? launch_v2_t<16, 2, true, 512>(prm, smem, stream) : launch_v2_t<16, 2, false, 512>(prm, smem, stream);
   if (prm.trace) return launch_v2_t<16, 4, true>(prm, smem, stream);   // same arithmetic + per-iteration records
-  switch (variant) {
-    case 1: return launch_v2_t<8, 4, false>(prm, smem, stream);
-    case 3: return launch_v2_t<16, 3, false>(prm, smem, stream);
-    default: return launch_v2_t<16, 4, false>(prm, smem, stream);
-  }
+  return launch_v2_t<16, 4, false>(prm, smem, stream);
 }
 
 }  // namespace ict

@@ -26,7 +26,6 @@
 #include "ict_kernel_v2.cuh"
 #include "ict_kernel_v8.cuh"
 
-#include <cstdlib>
 
 namespace ict {
 
@@ -478,11 +477,8 @@ cudaError_t launch_track_v8(const TrackParams& prm, int max_pts, cudaStream_t st
   if (prm.T <= 0) return cudaSuccess;
   const size_t smem = v8_smem_bytes(prm.op, max_pts);
   const int P = max_pts < prm.op.maxpttrack ? max_pts : prm.op.maxpttrack;
-  // sixteen warps for more than 128 points (one CTA per SM then anyway), or on request: ICT_V8_WARPS=16 lowers the
-  // latency of a single chain by 15 % at equal throughput
-  static int want16 = -1;
-  if (want16 < 0) want16 = ict_knob("ICT_V8_WARPS") && atoi(ict_knob("ICT_V8_WARPS")) == 16;
-  return (P > 8 * V8_MP || want16) ? launch_v8_nw<16>(prm, smem, stream) : launch_v8_nw<8>(prm, smem, stream);
+  // sixteen warps for more than 128 points (one CTA per SM then anyway)
+  return P > 8 * V8_MP ? launch_v8_nw<16>(prm, smem, stream) : launch_v8_nw<8>(prm, smem, stream);
 }
 
 }  // namespace ict

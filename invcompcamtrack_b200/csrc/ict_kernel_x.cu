@@ -416,7 +416,6 @@ size_t kx_smem_bytes(const ict_optparam& op, int max_pts) {
 cudaError_t launch_track_x(const TrackParams& prm, int max_pts, cudaStream_t stream) {
   if (prm.T <= 0) return cudaSuccess;
   const size_t smem = kx_smem_bytes(prm.op, max_pts);
-  if (smem > (size_t)ICT_TRACK_SMEM_LIMIT) return cudaErrorInvalidConfiguration;
   static bool attr_dev[64] = {};            // function attributes are per device
   int dev_ = 0;
   cudaGetDevice(&dev_);

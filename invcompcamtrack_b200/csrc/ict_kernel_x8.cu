@@ -586,7 +586,6 @@ static cudaError_t launch_x8_pk(const TrackParams& prm, bool wide, size_t smem7,
 
 cudaError_t launch_track_x8(const TrackParams& prm, int max_pts, cudaStream_t stream) {
   if (prm.T <= 0) return cudaSuccess;
-  if (!kx8_supported(prm.op, max_pts)) return cudaErrorInvalidConfiguration;
   const size_t smem7 = kx8_smem_np(prm.op, max_pts, 7), smem15 = kx8_smem_np(prm.op, max_pts, 15);
   const bool ok7 = x8_form_ok(prm.op, max_pts, 7), ok15 = x8_form_ok(prm.op, max_pts, 15);
   int sms = 148;

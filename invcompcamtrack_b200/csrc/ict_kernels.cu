@@ -10,7 +10,6 @@
 #include "ict_device.cuh"
 
 #include <atomic>
-#include <cstdlib>
 
 namespace ict {
 
@@ -865,9 +864,6 @@ __global__ void __launch_bounds__(256, MINB) k_track_fast(const TrackParams prm)
   const FrameDesc* fr_ref = prm.frames + rf;
   const FrameDesc* fr_new = prm.frames + nf;
 
-  // the warp that runs the serial sections (Hessian sums + LU, solve + update); env knob for profiling
-  const int swarp = prm.serial_warp_last ? nw - 1 : 0;
-
   // this warp's run of groups
   const int G_all = P * GPP;
   const int gpw = (G_all + nw - 1) / nw;
@@ -994,7 +990,7 @@ __global__ void __launch_bounds__(256, MINB) k_track_fast(const TrackParams prm)
       warp_sum_store<21>(acc, &S.part[warp * 24]);
     }
     __syncthreads();
-    if (warp == swarp) {
+    if (warp == 0) {                                // the serial sections: Hessian sums + LU, solve + update
       const long long t_lv0 = trace ? clock64() : 0;
       if (lane < 21) {
         float v[8];
@@ -1083,7 +1079,7 @@ __global__ void __launch_bounds__(256, MINB) k_track_fast(const TrackParams prm)
       if (lane == 0) S.part[warp * 24 + 6] = (float)nvis;
       const long long t_par = trace ? clock64() : 0;
       __syncthreads();
-      if (warp == swarp) {
+      if (warp == 0) {
         const long long t_ser0 = trace ? clock64() : 0;
         if (lane < 7) {   // 9a. cross-warp sums, fixed order, seven lanes in parallel (loads issued together)
           float v[8];
@@ -1101,10 +1097,7 @@ __global__ void __launch_bounds__(256, MINB) k_track_fast(const TrackParams prm)
           if (lane < 6) S.dp[lane] = x;
           __syncwarp();
         }
-        if (lane == 0 && prm.dbg_skip_serial) {     // profiling experiment only: how much does the serial section cost?
-          S.it += 1;
-          S.cont = S.it < op.maxiter;
-        } else if (lane == 0) {
+        if (lane == 0) {
           if (!fullrank) lu6_solve(S.lu, S.sum, S.dp);
           float dp[6], pr[6], Gr[12];                // registers: shared-memory operands would be re-read after every store
 #pragma unroll
@@ -1158,8 +1151,12 @@ static size_t fast_smem_bytes(const ict_optparam& op, int max_pts) {
   return sizeof(float) * (3 * P * op.novals + 16 * P);
 }
 
+// Rows per group (KTMAX) x CTAs per SM (MINB) for psz 32, measured on one B200 (8 sequences), in pixel-residuals/s:
+//   KT 4/4 CTAs 2.61e11   KT 4/3 CTAs 2.51e11   KT 8/4 2.75e11   KT 8/3 2.66e11   KT 16/4 2.80e11   KT 16/3 2.66e11
+// More rows per group put more independent gathers in flight per warp, and four resident CTAs beat three even though
+// 64 registers spill ~230 B in the per-level precompute.
 template <int PSZ, int KTMAX, int MINB>
-static cudaError_t launch_track_fast_v(const TrackParams& prm, size_t smem, int nt, cudaStream_t stream) {
+static cudaError_t launch_track_fast_t(const TrackParams& prm, size_t smem, int nt, cudaStream_t stream) {
   static bool attr_dev[64] = {};            // function attributes are per device
   int dev_ = 0;
   cudaGetDevice(&dev_);
@@ -1175,30 +1172,6 @@ static cudaError_t launch_track_fast_v(const TrackParams& prm, size_t smem, int 
   k_track_fast<PSZ, KTMAX, MINB><<<prm.T, nt, smem, stream>>>(prm);
   COUNT_LAUNCH();
   return cudaGetLastError();
-}
-
-template <int PSZ>
-static cudaError_t launch_track_fast_t(const TrackParams& prm, size_t smem, int nt, cudaStream_t stream) {
-  // Rows per group x CTAs per SM, measured on one B200 with profiles/tools/variant_sweep.sh (psz 32, 8 sequences):
-  //   KT 4/4 CTAs 2.61e11   KT 4/3 CTAs 2.51e11   KT 8/4 2.75e11   KT 8/3 2.66e11   KT 16/4 2.80e11   KT 16/3 2.66e11
-  // pixel-residuals/s: more rows per group put more independent gathers in flight per warp, and four resident CTAs
-  // beat three even though 64 registers spill ~230 B in the per-level precompute.
-  static int variant = -1;
-  if (variant < 0) {
-    const char* e = ict_knob("ICT_FAST_VARIANT");   // tuning knob for profiling runs only
-    variant = e ? atoi(e) : 4;
-  }
-  if (PSZ == 32) {
-    switch (variant) {
-      case 0: return launch_track_fast_v<PSZ, 4, 4>(prm, smem, nt, stream);
-      case 1: return launch_track_fast_v<PSZ, 4, 3>(prm, smem, nt, stream);
-      case 2: return launch_track_fast_v<PSZ, 8, 4>(prm, smem, nt, stream);
-      case 3: return launch_track_fast_v<PSZ, 8, 3>(prm, smem, nt, stream);
-      case 5: return launch_track_fast_v<PSZ, 16, 3>(prm, smem, nt, stream);
-      default: return launch_track_fast_v<PSZ, 16, 4>(prm, smem, nt, stream);
-    }
-  }
-  return launch_track_fast_v<PSZ, 4, 4>(prm, smem, nt, stream);
 }
 
 size_t track_smem_bytes(const ict_optparam& op, int max_pts, int sum_mode) {
@@ -1238,62 +1211,63 @@ static cudaError_t launch_track_p(const TrackParams& prm, size_t smem, int nt, i
   }
 }
 
-// True when one CTA can hold a whole track: the general kernel's layout fits, or one of the patch-size-8 kernels
-// (denser layouts: no fourth plane for dopatchnorm) takes the configuration.  Otherwise the multi-CTA path runs.
-bool track_fits_one_cta(const ict_optparam& op, int max_pts, int sum_mode, int force_general) {
-  if (track_smem_bytes(op, max_pts, sum_mode) <= (size_t)ICT_TRACK_SMEM_LIMIT) return true;
-  if (force_general) return false;
-  if (sum_mode) return !ict_knob("ICT_EXACT_V1") && kx8_supported(op, max_pts);
-  return !ict_knob("ICT_FAST_V1") && v8_supported(op, max_pts);
-}
-
-// True when launch_track runs K2v8 for this configuration: the kernel that can take a whole chain of frame steps
-// (TrackParams.seq_n) in one launch.
-bool track_chain_in_one_launch(const ict_optparam& op, int max_pts, int sum_mode, int force_general, int per_frame_launches) {
-  return sum_mode == 0 && !force_general && !per_frame_launches && !ict_knob("ICT_FAST_V1") &&
-         v8_supported(op, max_pts);
+TrackKernel select_track_kernel(const ict_optparam& op, int max_pts, int sum_mode, int eigen_packet, int force_general,
+                                int no_k2r, int tma_ok) {
+  const bool general_fits = track_smem_bytes(op, max_pts, sum_mode) <= (size_t)ICT_TRACK_SMEM_LIMIT;
+  if (!force_general && sum_mode == 0) {
+    if (v8_supported(op, max_pts)) return TrackKernel::V8;           // 8x8 patches, with or without dopatchnorm
+    if (general_fits && !op.dopatchnorm) {
+      if (op.psz == 32 && v2_smem_bytes(op, max_pts) <= (size_t)ICT_TRACK_SMEM_LIMIT) return TrackKernel::V2;
+      if (op.psz == 8 || op.psz == 16 || op.psz == 32) return TrackKernel::Fast;
+    }
+  }
+  if (!force_general && sum_mode != 0) {
+    if (kx8_supported(op, max_pts)) return TrackKernel::X8;          // 8x8 (+/- dopatchnorm) and 16x16 patches
+    // K2r and K2x run the eight chains of 4-float packets only: with 8-float packets psz 32 takes the general kernel
+    if (general_fits && !op.dopatchnorm && eigen_packet == 4) {
+      if (!no_k2r && kr_supported(op, max_pts, tma_ok)) return TrackKernel::R;
+      if (op.psz == 32 && kx_smem_bytes(op, max_pts) <= (size_t)ICT_TRACK_SMEM_LIMIT) return TrackKernel::X;
+    }
+  }
+  return general_fits ? TrackKernel::General : TrackKernel::MultiCta;
 }
 
 cudaError_t launch_track(const TrackParams& prm, int max_pts, cudaStream_t stream) {
   if (prm.T <= 0) return cudaSuccess;
-  if (prm.seq_n > 1 && !track_chain_in_one_launch(prm.op, max_pts, prm.sum_mode, prm.force_general, prm.knob_seq_launches))
+  const TrackKernel k = select_track_kernel(prm.op, max_pts, prm.sum_mode, prm.eigen_packet, prm.force_general,
+                                            prm.knob_no_k2r, prm.tma_ok);
+  if (prm.seq_n > 1 && (k != TrackKernel::V8 || prm.knob_seq_launches))
     return cudaErrorInvalidConfiguration;   // only K2v8 loops over frames
-  const size_t smem = track_smem_bytes(prm.op, max_pts, prm.sum_mode);
-  if (!track_fits_one_cta(prm.op, max_pts, prm.sum_mode, prm.force_general)) return cudaErrorInvalidConfiguration;
   const int P = max_pts < prm.op.maxpttrack ? max_pts : prm.op.maxpttrack;
   const long long E = (long long)P * prm.op.novals;
-  int nt = E >= 2048 ? 256 : (E >= 512 ? 128 : 64);
-  const int mode = (prm.op.dopatchnorm ? 1 : 0) | (prm.sum_mode ? 2 : 0) | (prm.sum_mode && prm.eigen_packet == 8 ? 4 : 0);
-  if (const char* e = ict_knob("ICT_NT")) nt = atoi(e);   // profiling knob
-  if ((mode & 2) == 0 && !prm.force_general && !ict_knob("ICT_FAST_V1") && v8_supported(prm.op, max_pts))
-    return launch_track_v8(prm, max_pts, stream);      // K2v8: 8x8 patches, with or without dopatchnorm
-  if (mode == 0 && !prm.force_general && prm.op.psz == 32 && !ict_knob("ICT_FAST_V1") &&
-      v2_smem_bytes(prm.op, max_pts) <= (size_t)ICT_TRACK_SMEM_LIMIT)
-    return launch_track_v2(prm, max_pts, stream);
-  if (mode == 0 && !prm.force_general && (prm.op.psz == 8 || prm.op.psz == 16 || prm.op.psz == 32)) {
-    const size_t fsm = fast_smem_bytes(prm.op, max_pts);
-    switch (prm.op.psz) {
-      case 8: return launch_track_fast_t<8>(prm, fsm, nt, stream);
-      case 16: return launch_track_fast_t<16>(prm, fsm, nt, stream);
-      default: return launch_track_fast_t<32>(prm, fsm, nt, stream);
+  const int nt = E >= 2048 ? 256 : (E >= 512 ? 128 : 64);
+  switch (k) {
+    case TrackKernel::V8: return launch_track_v8(prm, max_pts, stream);
+    case TrackKernel::V2: return launch_track_v2(prm, max_pts, stream);
+    case TrackKernel::Fast: {
+      const size_t smem = fast_smem_bytes(prm.op, max_pts);
+      switch (prm.op.psz) {
+        case 8: return launch_track_fast_t<8, 4, 4>(prm, smem, nt, stream);
+        case 16: return launch_track_fast_t<16, 4, 4>(prm, smem, nt, stream);
+        default: return launch_track_fast_t<32, 16, 4>(prm, smem, nt, stream);
+      }
     }
-  }
-  if ((mode & 2) && !prm.force_general && !ict_knob("ICT_EXACT_V1") && kx8_supported(prm.op, max_pts))
-    return launch_track_x8(prm, max_pts, stream);      // K2x8: reference-order sums, 8x8 patches, +/- dopatchnorm
-  // K2r and K2x run the eight chains of 4-float packets only: with 8-float packets psz 32 takes the general kernel
-  if (mode == 2 && !prm.force_general && !prm.knob_no_k2r && !ict_knob("ICT_EXACT_V1") &&
-      kr_supported(prm.op, max_pts, prm.tma_ok))
-    return launch_track_r(prm, max_pts, stream);       // K2r: reference-order sums, resident sd images, TMA windows
-  if (mode == 2 && !prm.force_general && prm.op.psz == 32 && !ict_knob("ICT_EXACT_V1") &&
-      kx_smem_bytes(prm.op, max_pts) <= (size_t)ICT_TRACK_SMEM_LIMIT)
-    return launch_track_x(prm, max_pts, stream);       // K2x: reference-order sums, producer/chain warps
-  const int ntx = (mode & 2) && nt < 192 ? 192 : nt;   // the reference-order J^T r needs 6*16 = 96 threads, the Hessian
-                                                       // 21*8 = 168 (it loops over the 21*16 chains of 8-float packets)
-  switch (prm.op.psz) {
-    case 8: return launch_track_p<8>(prm, smem, ntx, mode, stream);
-    case 16: return launch_track_p<16>(prm, smem, ntx, mode, stream);
-    case 32: return launch_track_p<32>(prm, smem, ntx, mode, stream);
-    default: return launch_track_p<0>(prm, smem, ntx, mode, stream);
+    case TrackKernel::X8: return launch_track_x8(prm, max_pts, stream);
+    case TrackKernel::R: return launch_track_r(prm, max_pts, stream);
+    case TrackKernel::X: return launch_track_x(prm, max_pts, stream);
+    case TrackKernel::General: {
+      const size_t smem = track_smem_bytes(prm.op, max_pts, prm.sum_mode);
+      const int mode = (prm.op.dopatchnorm ? 1 : 0) | (prm.sum_mode ? 2 : 0) | (prm.sum_mode && prm.eigen_packet == 8 ? 4 : 0);
+      const int ntx = (mode & 2) && nt < 192 ? 192 : nt;   // the reference-order J^T r needs 6*16 = 96 threads, the Hessian
+                                                           // 21*8 = 168 (it loops over the 21*16 chains of 8-float packets)
+      switch (prm.op.psz) {
+        case 8: return launch_track_p<8>(prm, smem, ntx, mode, stream);
+        case 16: return launch_track_p<16>(prm, smem, ntx, mode, stream);
+        case 32: return launch_track_p<32>(prm, smem, ntx, mode, stream);
+        default: return launch_track_p<0>(prm, smem, ntx, mode, stream);
+      }
+    }
+    default: return cudaErrorInvalidConfiguration;   // MultiCta: launch_track_big, one track at a time
   }
 }
 

@@ -3,7 +3,6 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include "../../include/ictrack.h"
-#include "ict_knobs.h"
 
 namespace ict {
 
@@ -47,9 +46,6 @@ struct TrackParams {
   float* pt2d_out;                 // [2*total] or null: reference 2-D points at lv_l (Get2DPoints)
   int T;                           // tracks in this launch
   int t0;                          // first track of this launch (index into the per-track arrays)
-  int serial_warp_last;            // profiling knob: run the serial sections on the CTA's last warp instead of warp 0
-  int dbg_skip_serial;             // profiling experiment: skip solve/update (results meaningless)
-  int v2_lu_setup;                 // K2v2 A/B knob: per-level solve matrix from the warp LU instead of the sweeps
   int force_general;               // 1: always use the general kernel k_track (tests compare the two)
   int seq_n, seq_step;             // K2v8 only: seq_n > 1 runs a whole chain in one launch — step k tracks frame
                                    //    fixed_ref + k*seq_step -> + seq_step from pose p_in + 6*T*k to p_out + 6*T*k
@@ -80,27 +76,38 @@ cudaError_t launch_pyramid(const float* src_f32, const unsigned char* src_u8, in
 cudaError_t launch_set_points(int T, const int64_t* pt_off, const double* pts, double* pts_mut, float* pt3d,
                               double* norm, int donorm, int maxpttrack, int max_pts, cudaStream_t stream);
 
-// a6..a18: SetPose + TrackPose, one CTA per track, template + gradients resident in shared memory.
-// Returns cudaErrorInvalidConfiguration when a track does not fit (caller then uses the multi-CTA path).
+// a6..a18: SetPose + TrackPose.  Every kernel below but the multi-CTA path runs one CTA per track, template +
+// gradients resident in shared memory.
+//   V8        k_track_v8   fast mode, psz 8 (+/- dopatchnorm); the only kernel that runs a chain of frame steps
+//   V2        k_track_v2   fast mode, psz 32 without dopatchnorm
+//   Fast      k_track_fast fast mode, psz 8 / 16 / 32 without dopatchnorm, where V8 and V2 do not fit
+//   X8        k_track_x8   reference order, psz 8 (+/- dopatchnorm) and psz 16 without dopatchnorm
+//   R         k_track_r    reference order with 4-float packets, psz 32 without dopatchnorm, needs tensor maps
+//   X         k_track_x    reference order with 4-float packets, psz 32 without dopatchnorm
+//   General   k_track      any psz, dopatchnorm and sum order, where its own layout fits (sum order 2: always)
+//   MultiCta  launch_track_big, one track at a time
+enum class TrackKernel { V8, V2, Fast, X8, R, X, General, MultiCta };
+// The kernel family that runs a track set whose largest track has max_pts points.  The only place that decides it:
+// a pure host function, no CUDA calls.  no_k2r and tma_ok matter only where K2r would otherwise run.
+TrackKernel select_track_kernel(const ict_optparam& op, int max_pts, int sum_mode, int eigen_packet, int force_general,
+                                int no_k2r, int tma_ok);
 size_t track_smem_bytes(const ict_optparam& op, int max_pts, int sum_mode);
-bool track_fits_one_cta(const ict_optparam& op, int max_pts, int sum_mode, int force_general);
-bool track_chain_in_one_launch(const ict_optparam& op, int max_pts, int sum_mode, int force_general, int per_frame_launches);
+// Launches the selected kernel; cudaErrorInvalidConfiguration for MultiCta (the caller runs launch_track_big).
 cudaError_t launch_track(const TrackParams& prm, int max_pts, cudaStream_t stream);
 
-// K2v2 (ict_kernel_v2.cu): the production kernel for psz 32 without dopatchnorm, tree sums; launch_track routes
-// to it unless ICT_FAST_V1 is set (then k_track_fast, the previous production kernel, runs — for A/B measurements).
+// Each kernel's own constraints: *_supported / *_smem_bytes.  The launchers assume select_track_kernel chose them.
+// K2v2 (ict_kernel_v2.cu): the production kernel for psz 32 without dopatchnorm, tree sums.
 size_t v2_smem_bytes(const ict_optparam& op, int max_pts);
 cudaError_t launch_track_v2(const TrackParams& prm, int max_pts, cudaStream_t stream);
 
-// K2v8 (ict_kernel_v8.cu): the K2v2 scheme for 8x8 patches (the reference's own configuration), up to 240 points per
+// K2v8 (ict_kernel_v8.cu): the K2v2 scheme for 8x8 patches (the reference's own configuration), up to 241 points per
 // track, with or without dopatchnorm, tree sums; honours TrackParams.seq_n (a chain of frame steps in one launch).
 bool v8_supported(const ict_optparam& op, int max_pts);
 size_t v8_smem_bytes(const ict_optparam& op, int max_pts);
 cudaError_t launch_track_v8(const TrackParams& prm, int max_pts, cudaStream_t stream);
 
 // K2x (ict_kernel_x.cu): reference-order (Eigen packet) sums for psz 32 without dopatchnorm — bit-identical to the
-// oracle like k_track<32,2>, with producer warps and one chain warp; launch_track routes sum_mode 1 with 4-float
-// packets to it unless ICT_EXACT_V1 is set (K2x and K2r run eight chains only).
+// oracle like k_track<32,2>, with producer warps and one chain warp; 4-float packets only (eight chains).
 size_t kx_smem_bytes(const ict_optparam& op, int max_pts);
 cudaError_t launch_track_x(const TrackParams& prm, int max_pts, cudaStream_t stream);
 
@@ -110,7 +117,7 @@ bool kr_supported(const ict_optparam& op, int max_pts, int tma_ok);
 size_t kr_smem_bytes(const ict_optparam& op, int max_pts);
 cudaError_t launch_track_r(const TrackParams& prm, int max_pts, cudaStream_t stream);
 
-// K2x8 (ict_kernel_x8.cu): reference-order sums for 8x8 patches (up to 224 points per track), with or without
+// K2x8 (ict_kernel_x8.cu): reference-order sums for 8x8 patches (up to 222 points per track), with or without
 // dopatchnorm — bit-identical to the oracle like k_track<8,2|3> (4-float packets) and k_track<8,6|7> (8-float packets).
 bool kx8_supported(const ict_optparam& op, int max_pts);
 size_t kx8_smem_bytes(const ict_optparam& op, int max_pts);

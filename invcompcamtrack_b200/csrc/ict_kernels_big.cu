@@ -11,7 +11,6 @@
 #include "ict_kernels.cuh"
 #include "ict_device.cuh"
 
-#include <cstdlib>
 
 namespace ict {
 
@@ -923,8 +922,7 @@ __global__ void __launch_bounds__(256, 4) k_dense_iter_tma(const BigArgs a, int 
   const long long P = a.P;
   const float* sdp = a.w.coef;
   const int ntile = (int)((P + 255) / 256);
-  int nmine = ntile > (int)blockIdx.x ? (ntile - 1 - (int)blockIdx.x) / (int)gridDim.x + 1 : 0;
-  if (a.prm.dbg_skip_serial == 4) nmine = 0;                                   // DBG: launch + finish only
+  const int nmine = ntile > (int)blockIdx.x ? (ntile - 1 - (int)blockIdx.x) / (int)gridDim.x + 1 : 0;
   auto issue = [&](int n) {               // thread 0: the n-th tile of this CTA into stage n % NST
     const long long i0 = ((long long)blockIdx.x + (long long)n * gridDim.x) * 256;
     const unsigned bytes = (unsigned)((P - i0 < 256 ? P - i0 : 256) * 4);
@@ -962,12 +960,10 @@ __global__ void __launch_bounds__(256, 4) k_dense_iter_tma(const BigArgs a, int 
 #pragma unroll
   for (int k = 0; k < 6; ++k) acc[k] = 0.0f;
   int cnt = 0;
-  const int dbg = a.prm.dbg_skip_serial;
   // one point of a staged tile: projection, placement, the four-texel gather (returns the sample, sets vis).
   // (Tried: placing tile n+1 and issuing its gather before folding tile n — 23.1 instead of 21.3 us per iteration.)
   auto sample = [&](int st, bool& vis) -> float {
     const float X = s_buf[st][0][tid], Y = s_buf[st][1][tid], Z = s_buf[st][2][tid];
-    if (dbg == 2) { vis = true; return X + Y + Z; }                            // DBG: streams only
     const float tx = G[0] * X + G[1] * Y + G[2] * Z + G[3];                    // project_pt, pose.cpp:307-397
     const float ty = G[4] * X + G[5] * Y + G[6] * Z + G[7];
     const float tz = G[8] * X + G[9] * Y + G[10] * Z + G[11];
@@ -1031,7 +1027,7 @@ cudaError_t launch_track_big(const TrackParams& prm, int t, int64_t npts, void* 
   const bool pn = op.dopatchnorm != 0;
   const bool ex = prm.sum_mode != 0;   // reference-order sums
   const bool pk8 = ex && prm.eigen_packet == 8;   // ... with 8-float packets: sixteen chains per sum
-  const bool fused = !pn && !ex && !prm.force_general && op.novals == 1 && !ict_knob("ICT_DENSE_V1");
+  const bool fused = !pn && !ex && !prm.force_general && op.novals == 1;
   int nl = 0;
   const size_t chain_smem = pk8 ? sizeof(float) * BIG_STAGES * 16 * (big_chunk(16) + 4)    // 128.5 KB
                                 : sizeof(float) * BIG_STAGES * 8 * BIG_CHUNK;                  // 128 KB
@@ -1050,24 +1046,13 @@ cudaError_t launch_track_big(const TrackParams& prm, int t, int64_t npts, void* 
   k_big_project_ref<<<pcta, 256, 0, st>>>(a); ++nl;
   for (int sl = op.lv_f; sl >= op.lv_l && fused; --sl) {   // dense path: one launch per level + one per iteration
     // bulk-copy staging needs 16-byte aligned streams: point counts and the track's offset multiples of four
-    const bool tma = t == 0 && (a.P % 4 == 0) && (a.n_in % 4 == 0) && !ict_knob("ICT_DENSE_LDG");   // t == 0: offset 0
-    const int nst = ict_knob("ICT_DENSE_NST") ? atoi(ict_knob("ICT_DENSE_NST")) : 3;     // A/B knobs (profiling builds)
-    const int pdl = ict_knob("ICT_DENSE_NOPDL") ? 0 : 1;
-    static bool attr_dev[64] = {};            // function attributes are per device
-    int dev_ = 0;
-    cudaGetDevice(&dev_);
-    if (!attr_dev[dev_ & 63]) {
-      cudaError_t e = cudaFuncSetAttribute(k_dense_iter_tma<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, 5 * 10240);
-      if (e == cudaSuccess) e = cudaFuncSetAttribute(k_dense_iter_tma<5>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
-      if (e != cudaSuccess) return e;
-      attr_dev[dev_ & 63] = true;
-    }
+    const bool tma = t == 0 && (a.P % 4 == 0) && (a.n_in % 4 == 0);   // t == 0: offset 0
     // programmatic dependent launch: iteration k+1 becomes resident while the last CTA of iteration k still runs the
     // solve, and its first tiles are in flight by the time the pose is published
     cudaLaunchConfig_t cfg = {};
     cudaLaunchAttribute lattr[1];
     lattr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    lattr[0].val.programmaticStreamSerializationAllowed = pdl;
+    lattr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.gridDim = dim3(ncta);
     cfg.blockDim = dim3(256);
     cfg.stream = st;
@@ -1078,8 +1063,7 @@ cudaError_t launch_track_big(const TrackParams& prm, int t, int64_t npts, void* 
     cudaLaunchKernelEx(&cfg, k_big_level_finish, a, sl); ++nl;
     cfg.gridDim = dim3(ncta);
     for (int it = 0; it < op.maxiter; ++it) {
-      if (tma && nst == 3) { cfg.dynamicSmemBytes = 3 * 10240; cudaLaunchKernelEx(&cfg, k_dense_iter_tma<3>, a, sl); }
-      else if (tma) { cfg.dynamicSmemBytes = 5 * 10240; cudaLaunchKernelEx(&cfg, k_dense_iter_tma<5>, a, sl); }
+      if (tma) { cfg.dynamicSmemBytes = 3 * 10240; cudaLaunchKernelEx(&cfg, k_dense_iter_tma<3>, a, sl); }
       else k_dense_iter<<<ncta, 256, 0, st>>>(a, sl);
       ++nl;
     }

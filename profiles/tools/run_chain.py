@@ -15,6 +15,8 @@ op = ict.OptParam.from_buffer_copy(bytes(op_c))
 fr = ict.Frames(NF, 640, 480, 3, 8); fr.upload(0, np.stack(frames))
 tr = ict.Tracker(op, sc.fc, sc.cc, sc.wh)
 tr.set_sum_order(int(os.environ.get('SUM_ORDER', 0)))
+if os.environ.get('SEQ_LAUNCHES') == '1':
+    tr.set_knob("seq_launches", 1)   # one launch per frame step instead of the whole chain in one K2v8 launch
 pts = np.concatenate([sc.points(100 + s, NP, 8, 3) for s in range(S)])
 tr.set_points(np.arange(S + 1, dtype=np.int64) * NP, pts)
 for rep in range(3):
