@@ -105,7 +105,11 @@ int ict_frames_download(ict_frames* fs, int frame, float* out_I, float* out_dx, 
 typedef struct ict_tracker ict_tracker;
 ict_tracker* ict_tracker_create(const ict_optparam* op, const float fc[2], const float cc[2], const int wh[2]);
 void ict_tracker_destroy(ict_tracker* tr);
-/* later changes of the caller's optparam (run_track_nposes.cpp:281 flips dopatchnorm mid-run) */
+/* later changes of the caller's optparam (run_track_nposes.cpp:281 flips dopatchnorm mid-run).  psz and lv_f are fixed
+ * at creation; lv_l, maxiter, normdp_ratio, dopatchnorm and verbosity may change between any two calls.  maxpttrack and
+ * donorm shape the points that ict_tracker_set_points* stores (how many per track, and their normalisation): after a
+ * change of either, the calls that read the points (tracking, reproject, get_2dpoints, ncc_score) return
+ * ICT_ERR_BAD_ARG until ict_tracker_set_points* runs again.  Set both before the points, as OdometerClass does. */
 int ict_tracker_set_optparam(ict_tracker* tr, const ict_optparam* op);
 
 /* Order of the fp32 reductions (Hessian, J^T r, patch means):
@@ -200,7 +204,13 @@ int ict_tracker_set_teacher(ict_tracker* tr, const float* poses, int trace_cap);
 /* Set3Dpoints for T tracks (odometer.cpp:171-239).  Track t has points pt_off[t]..pt_off[t+1]-1; its points are
  * stored as the reference expects them: X block, Y block, Z block, each of length n_t, at pts + 3*pt_off[t].
  * HOST pointers.  With donorm the reference centres the CALLER's array in place (odometer.cpp:207-212); pass
- * mutate_caller=1 to get the same side effect (pts is then written). */
+ * mutate_caller=1 to get the same side effect (pts is then written).
+ * Tracks of one batch may differ in size, and a track may be empty (n_t == 0): it runs one iteration per level on no
+ * pixel, its J^T r and delta_p are 0 and its pose is p_in rounded to fp32.  With donorm, a track of one point or of
+ * equal points has a variance of 0 and an empty one a mean of 0/0: the reference leaves these undefined (it samples
+ * the image at NaN coordinates).  Here the normalised points are NaN, and a NaN placement counts as outside the
+ * image, so such a track runs one iteration per level on no pixel and returns a NaN translation and a zero rotation;
+ * the CPU oracle does the same. */
 int ict_tracker_set_points(ict_tracker* tr, int T, const int64_t* pt_off, double* pts, int mutate_caller);
 /* Same with device pointers (pt_off_dev: int64[T+1], pts_dev: double[3*total]); nothing is written back.
  * max_pts = the largest n_t (the host needs it to size the launch). */

@@ -458,6 +458,7 @@ struct ict_tracker {
   int T = 0;
   int64_t total = 0;
   int max_pts = 0;
+  int pts_maxpttrack = 0, pts_donorm = 0;   // the optparam fields ict_tracker_set_points* stored the points with
   std::vector<int64_t> h_off;
   bool have_2d = false;
   int sum_mode = 1;            // the reference's summation order is the default (ictrack.h, ict_tracker_set_sum_order)
@@ -599,6 +600,8 @@ int ict_tracker_set_points(ict_tracker* tr, int T, const int64_t* pt_off, double
   tr->T = T;
   tr->total = total;
   tr->max_pts = max_pts;
+  tr->pts_maxpttrack = tr->op.maxpttrack;
+  tr->pts_donorm = tr->op.donorm;
   tr->h_off.assign(pt_off, pt_off + T + 1);
   tr->have_2d = false;
   tr->state_valid = false;     // Set3Dpoints resets the odometer (odometer.cpp:173)
@@ -627,6 +630,8 @@ int ict_tracker_set_points_stream(ict_tracker* tr, int T, const int64_t* pt_off,
   tr->T = T;
   tr->total = total;
   tr->max_pts = max_pts;
+  tr->pts_maxpttrack = tr->op.maxpttrack;
+  tr->pts_donorm = tr->op.donorm;
   tr->h_off.assign(pt_off, pt_off + T + 1);
   tr->have_2d = false;
   tr->state_valid = false;     // Set3Dpoints resets the odometer (odometer.cpp:173)
@@ -645,9 +650,22 @@ int ict_tracker_set_points_dev(ict_tracker* tr, int T, const int64_t* pt_off_dev
   tr->T = T;
   tr->total = total_pts;
   tr->max_pts = max_pts;
+  tr->pts_maxpttrack = tr->op.maxpttrack;
+  tr->pts_donorm = tr->op.donorm;
   tr->h_off.clear();
   tr->have_2d = false;
   tr->state_valid = false;
+  return ICT_OK;
+}
+
+// k_set_points stores min(n, maxpttrack) points per track, normalised or not by donorm: a later optparam with another
+// maxpttrack or donorm would make the kernels read points that were never stored, or undo a normalisation that does
+// not match them.  Every call that reads the points refuses until ict_tracker_set_points runs again.
+static int points_current(const ict_tracker* tr) {
+  if (tr->T <= 0) return fail(ICT_ERR_BAD_ARG, "no points set: call ict_tracker_set_points first");
+  if (tr->op.maxpttrack != tr->pts_maxpttrack || tr->op.donorm != tr->pts_donorm)
+    return fail(ICT_ERR_BAD_ARG, "maxpttrack or donorm changed since the points were set: call ict_tracker_set_points "
+                                 "again");
   return ICT_OK;
 }
 
@@ -661,7 +679,7 @@ static int run_tracks(ict_tracker* tr, const ict_frames* fs, const int* rf_dev, 
                       int fixed_new, const double* p_in_dev, double* p_out_dev, int* iters_dev, float* trace_dev,
                       int trace_cap, long long* npix_dev, cudaStream_t st) {
   if (!tr || !fs) return fail(ICT_ERR_BAD_ARG, "null tracker / frame store");
-  if (tr->T <= 0) return fail(ICT_ERR_BAD_ARG, "no points set: call ict_tracker_set_points first");
+  if (points_current(tr)) return ICT_ERR_BAD_ARG;
   if (fs->lv_f != tr->op.lv_f || fs->pad != tr->op.psz || fs->w != tr->wh[0] || fs->h != tr->wh[1])
     return fail(ICT_ERR_BAD_ARG, "frame store does not match the tracker (need lv_f, pad == psz, w, h equal)");
   if (!rf_dev && (fixed_ref < 0 || fixed_ref >= fs->nframes || fixed_new < 0 || fixed_new >= fs->nframes))
@@ -772,7 +790,7 @@ int ict_track_batch(ict_tracker* tr, const ict_frames* fs, const int* ref_frame,
                     const double* p_in, double* p_out, int* iters, float* trace, int trace_cap, int64_t* npixres) {
   if (!tr || !fs || !ref_frame || !new_frame || !p_in || !p_out) return fail(ICT_ERR_BAD_ARG, "null argument");
   const int T = tr->T;
-  if (T <= 0) return fail(ICT_ERR_BAD_ARG, "no points set");
+  if (points_current(tr)) return ICT_ERR_BAD_ARG;
   const int L = tr->op.lv_f - tr->op.lv_l + 1;
   for (int t = 0; t < T; ++t)
     if (ref_frame[t] < 0 || ref_frame[t] >= fs->nframes || new_frame[t] < 0 || new_frame[t] >= fs->nframes)
@@ -818,7 +836,7 @@ int ict_track_batch_stream(ict_tracker* tr, const ict_frames* fs, const int* ref
   if (!tr || !fs || !ref_frame || !new_frame || !p_in || !p_out) return fail(ICT_ERR_BAD_ARG, "null argument");
   cudaStream_t st = (cudaStream_t)stream;
   const int T = tr->T;
-  if (T <= 0) return fail(ICT_ERR_BAD_ARG, "no points set");
+  if (points_current(tr)) return ICT_ERR_BAD_ARG;
   if (tracker_kernel(tr, fs) == TrackKernel::MultiCta)
     return fail(ICT_ERR_UNSUPPORTED, "stream variant handles tracks that fit one CTA");
   for (int t = 0; t < T; ++t)
@@ -852,7 +870,7 @@ int ict_track_sequence(ict_tracker* tr, const ict_frames* fs, int first, int nst
   if (!tr || !fs || !p_in || !poses_out || nsteps < 0 || (step != 1 && step != -1))
     return fail(ICT_ERR_BAD_ARG, "ict_track_sequence: bad argument");
   const int T = tr->T;
-  if (T <= 0) return fail(ICT_ERR_BAD_ARG, "no points set");
+  if (points_current(tr)) return ICT_ERR_BAD_ARG;
   const int L = tr->op.lv_f - tr->op.lv_l + 1;
   const int last = first + nsteps * step;
   if (first < 0 || first >= fs->nframes || last < 0 || last >= fs->nframes)
@@ -891,7 +909,7 @@ int ict_track_sequence(ict_tracker* tr, const ict_frames* fs, int first, int nst
 
 int ict_tracker_reproject(ict_tracker* tr, const double* p_in, float* pt2d_out) {
   if (!tr || !p_in) return fail(ICT_ERR_BAD_ARG, "null argument");
-  if (tr->T <= 0) return fail(ICT_ERR_BAD_ARG, "no points set");
+  if (points_current(tr)) return ICT_ERR_BAD_ARG;
   CU(tr->p_in.reserve(sizeof(double) * 6 * (size_t)tr->T));
   CU(cudaMemcpyAsync(tr->p_in.p, p_in, sizeof(double) * 6 * (size_t)tr->T, cudaMemcpyHostToDevice, 0));
   TrackParams prm;
@@ -912,6 +930,7 @@ int ict_tracker_reproject(ict_tracker* tr, const double* p_in, float* pt2d_out) 
 
 int ict_tracker_get_2dpoints(ict_tracker* tr, float* out) {
   if (!tr || !out) return fail(ICT_ERR_BAD_ARG, "null argument");
+  if (points_current(tr)) return ICT_ERR_BAD_ARG;
   if (!tr->have_2d) return fail(ICT_ERR_BAD_ARG, "no SetPose has run yet");
   CU(cudaMemcpy(out, tr->pt2d.p, sizeof(float) * 2 * (size_t)tr->total, cudaMemcpyDeviceToHost));
   return ICT_OK;
@@ -1011,6 +1030,7 @@ int ict_ncc_score(ict_tracker* tr, const ict_frames* fs, int frame_b, int frame_
                   const float* pt2d_back, const float* pt2d_refe, const float* pt2d_forw, float* out_corr) {
   if (!tr || !fs || !pt2d_back || !pt2d_refe || !pt2d_forw || !out_corr) return fail(ICT_ERR_BAD_ARG, "null argument");
   if (tr->T <= 0 || tr->h_off.empty()) return fail(ICT_ERR_BAD_ARG, "no points set");
+  if (points_current(tr)) return ICT_ERR_BAD_ARG;
   if (fs->view || !fs->I) return fail(ICT_ERR_BAD_ARG, "ict_ncc_score: needs a store that owns its pixels (not a view)");
   if (fs->lv_f != tr->op.lv_f || fs->pad != tr->op.psz || fs->w != tr->wh[0] || fs->h != tr->wh[1])
     return fail(ICT_ERR_BAD_ARG, "frame store does not match the tracker (need lv_f, pad == psz, w, h equal)");

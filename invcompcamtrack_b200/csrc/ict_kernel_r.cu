@@ -563,7 +563,8 @@ __global__ void __launch_bounds__((NPROD + 2) * 32, NPROD == 4 ? 2 : 1) k_track_
         long long t_c0 = 0, t_c1 = 0, w0 = 0;   // instrumentation (chain warp A, trace only)
         const unsigned want = gi + 1u;
         if (chainA && trace) t_c0 = clock64();
-        while (ld_acquire_s(&S.pd_flag[0]) != want) {}
+        if (U > 0)   // an empty track has no unit whose producer would ever raise the flag
+          while (ld_acquire_s(&S.pd_flag[0]) != want) {}
         if (chainA && trace) w0 = clock64() - t_c0;
 #pragma unroll 1
         for (int u = 0; u < U; ++u) {

@@ -346,6 +346,8 @@ __global__ void __launch_bounds__(256, 2) k_track_x(const TrackParams prm) {
       if (chainw) {
         // 9a. sumsd[k]: Eigen's redux of the eight chains
         const float rx = kx_finish(sx), ry = kx_finish(sy);
+        // S.nv reaches this warp through the ring's barriers; an empty track has no rounds, and no visible point
+        const int nv = NTILE > 0 ? S.nv : 0;
         if ((lane & 7) == 0) {
           S.sum[lane >> 3] = rx;
           if (lane < 16) S.sum[4 + (lane >> 3)] = ry;
@@ -372,7 +374,7 @@ __global__ void __launch_bounds__(256, 2) k_track_x(const TrackParams prm) {
             rec[1] = (float)it;
             for (int k = 0; k < 6; ++k) { rec[2 + k] = sumsd[k]; rec[8 + k] = dp[k]; }
             rec[14] = normdp;
-            rec[15] = (float)S.nv;
+            rec[15] = (float)nv;
             for (int k = 16; k < ICT_TRACE_FLOATS; ++k) rec[k] = 0.0f;
             rec[22] = (float)(clock64() - t_c1);   // cycles of the serial section (finish, solve, exp)
             rec[23] = (float)(t_c1 - t_c0);        // cycles the chain warp spent consuming the rounds of this sum
@@ -383,7 +385,7 @@ __global__ void __launch_bounds__(256, 2) k_track_x(const TrackParams prm) {
         const float normdp = S.dp[6];
         if (it == 0) normdp_init = normdp;
         const int cont = (it + 1 < op.maxiter) & ((normdp / normdp_init) > op.normdp_ratio);   // odometer.cpp:344-346
-        nvsum += S.nv;
+        nvsum += nv;
         if (lane == 0) {
           S.it = it + 1;
           S.cont = cont;

@@ -474,7 +474,9 @@ __global__ void __launch_bounds__((NP + 1) * 32, NP == 7 ? 2 : 1) k_track_x8(con
         __syncwarp();
         int nv = 0;
         if (lane == 0) {
-          for (int w = 0; w < NP; ++w) nv += s_nv[w];
+          // s_nv reaches this warp through the ring's barriers; an empty track has no rounds, and no visible point
+          if (ROUNDS > 0)
+            for (int w = 0; w < NP; ++w) nv += s_nv[w];
           float sumsd[6], dp[6];
 #pragma unroll
           for (int k = 0; k < 6; ++k) sumsd[k] = S.sum[k];

@@ -663,7 +663,10 @@ void ict_oracle_trackpose(ict_oracle_odom* o, double* p_out) {
     /* 4. reference patches + gradients, odometer.cpp:268-298 */
     for (int i = 0; i < np; ++i) {
       float mid[2] = {o->pt2d[sl][i], o->pt2d[sl][i + M]};
-      if ((mid[0] < 0) | (mid[1] < 0) | (mid[0] > swo) | (mid[1] > sho)) {
+      /* The reference tests (x < 0) | (y < 0) | (x > swo) | (y > sho): the same for finite x, y, but a NaN placement
+       * (donorm on one point or on equal points, include/ictrack.h) would pass it and be sampled.  Negated, as in the
+       * kernels, NaN is outside. */
+      if (!((mid[0] >= 0) & (mid[1] >= 0) & (mid[0] <= swo) & (mid[1] <= sho))) {
         o->ind_ref[i] = 0;
       } else {
         o->ind_ref[i] = 1;
@@ -713,7 +716,7 @@ void ict_oracle_trackpose(ict_oracle_odom* o, double* p_out) {
       double abssum[6] = {0, 0, 0, 0, 0, 0};
       for (int i = 0; i < np; ++i) { /* :363-396 */
         float mid[2] = {o->pt2d_new[i], o->pt2d_new[i + M]};
-        if ((mid[0] < 0) | (mid[1] < 0) | (mid[0] > swo) | (mid[1] > sho)) {
+        if (!((mid[0] >= 0) & (mid[1] >= 0) & (mid[0] <= swo) & (mid[1] <= sho))) { /* NaN: outside (see 4.) */
           o->ind_new[i] = 0;
         } else {
           o->ind_new[i] = 1;

@@ -141,3 +141,37 @@ def test_oracle_modes_spread(orc):
         om = oracle_run(orc, case, sum_mode=mode)
         res = check_parity(om, o0, case, min_same_iters=0.85, min_trans_ok=0.5, jtr_traj_tol=1.0)
         assert res["jtr_first"] < 1e-5
+
+
+def test_degenerate_donorm_tracks(orc):
+    """donorm on a track of one point (or of equal points) divides by a variance of 0 and on an empty track by 0
+    points: the points become NaN.  A NaN placement is not visible (the test reads !(x >= 0 & ... & y <= sho), as the
+    kernels do), so such a track runs one iteration per level on no pixel and returns a NaN translation and a zero
+    rotation; the other tracks of the batch are not affected."""
+    from invcompcamtrack_b200 import synth
+    sc, A, B, _ = synth.make_pair(21, 320, 240)
+    pa = orc.pyramid_build(A.astype(np.float32), 2, 8)
+    pb = orc.pyramid_build(B.astype(np.float32), 2, 8)
+    sizes = [5, 1, 0, 37]
+    pts = [sc.points(90 + t, n, 8, 2) for t, n in enumerate(sizes)]
+    pt_off = np.concatenate([[0], np.cumsum(sizes)]).astype(np.int64)
+    op = O.make_optparam(lv_f=2, psz=8, donorm=1, maxpttrack=40)
+
+    def run(idx):
+        n = [sizes[t] for t in idx]
+        return orc.track_batch(op, sc.fc, sc.cc, sc.wh, [pa[0], pb[0]], [pa[1], pb[1]], [pa[2], pb[2]],
+                               np.concatenate([[0], np.cumsum(n)]).astype(np.int64),
+                               np.concatenate([pts[t] for t in idx]), np.zeros(len(idx), np.int32),
+                               np.ones(len(idx), np.int32), np.zeros((len(idx), 6)), trace_cap=16, want_pt2d=True)
+    o = run(range(4))
+    for t in (1, 2):
+        assert np.isnan(o["p_out"][t, :3]).all() and np.array_equal(o["p_out"][t, 3:], np.zeros(3))
+        assert np.array_equal(o["iters"][t], [1, 1, 1]) and o["npixres"][t] == 0
+        assert (o["trace"][t, :3, 15] == 0).all()
+    assert np.isnan(o["pt2d"][2 * pt_off[1]:2 * pt_off[2]]).all()
+    for t in (0, 3):
+        assert np.isfinite(o["p_out"][t]).all() and (o["iters"][t] >= 2).all()
+        alone = run([t])
+        assert np.array_equal(alone["p_out"][0], o["p_out"][t])
+        assert np.array_equal(alone["trace"][0], o["trace"][t])
+        assert np.array_equal(alone["pt2d"], o["pt2d"][2 * pt_off[t]:2 * pt_off[t + 1]])
