@@ -244,6 +244,38 @@ int ict_track_sequence(ict_tracker* tr, const ict_frames* fs, int first, int nst
  * laid out like ict_tracker_get_2dpoints; may be NULL (then fetch with ict_tracker_get_2dpoints). */
 int ict_tracker_reproject(ict_tracker* tr, const double* p_in, float* pt2d_out);
 
+/* ---- quality of a pose: one Gauss-Newton measurement per track, without iterating ---------------------------------
+ * For the T tracks of the last ict_tracker_set_points* (host or device form), track t:
+ *   SetPose(p_ref[t], frame ref_frame[t] as reference, new_frame[t] as new) exactly as ict_track_batch, donorm's
+ *   normalisation included; the template state TrackPose holds when it reaches `level` from lv_f, starting from zeroed
+ *   arrays: a point outside the reference image at `level` keeps the template and steepest-descent values of the finest
+ *   level in (level, lv_f] at which it was inside, or zeros if it never was (SURVEY.md §9 item 6; these depend on p_ref
+ *   only); then ONE measurement at p_cur[t] (NULL: p_cur = p_ref) set like setpose_se3: projection at `level`, the test
+ *   against the new image, the new patch (mean-subtracted with dopatchnorm), pdiff = template - new patch, 0 for points
+ *   outside the new image (odometer.cpp:360-396).  Host buffers; any output may be NULL:
+ *     out_H      float[T*36]  the level's Hessian sum_s sd_a*sd_b over all maxpttrack*novals slots (ComputeHessian,
+ *                             odometer.cpp:428-472), symmetric
+ *     out_jtr    float[T*6]   J^T r = sum_s sd_k * pdiff (odometer.cpp:399-404)
+ *     out_dp     float[T*6]   the Gauss-Newton step H.fullPivLu().solve(J^T r) (odometer.cpp:407): what the next update
+ *                             of TrackPose at this pose would add
+ *     out_ssr    float[T]     sum_s pdiff^2
+ *     out_nvis   int[T]       points inside the new image (trace field [15])
+ *     out_pt_ssr float[total] each point's sum of pdiff^2 over its novals pixels, laid out like the points; -1 for a
+ *                             point outside the new image or beyond maxpttrack
+ * The reference's gradients are I(x+1) - I(x-1), twice the derivative, so sd is twice the Jacobian: H is 4x the
+ * Gauss-Newton information matrix J^T J and J^T r twice the gradient; with pixel noise sigma a pose covariance is
+ * 4 sigma^2 H^-1.  With p_cur = p_ref and level = lv_f, J^T r, delta_p and nvis are TrackPose's first iteration.
+ * Sums follow ict_tracker_set_sum_order: orders 1 and 3 Eigen's packet order (8 or 16 chains) for every sum, the
+ * per-point ones and the patch means included (bit-identical to a CPU restatement built from the oracle's pieces); orders 0 and 2 a fixed
+ * tree per track, deterministic and independent of the other tracks of the batch.  Tracks of any size, empty tracks,
+ * one-point donorm tracks (NaN points: nothing visible, all sums 0) and the maxpttrack cap behave as for
+ * ict_track_batch.  level outside [lv_l, lv_f], a frame index outside fs, or points set before a change of maxpttrack or
+ * donorm: ICT_ERR_BAD_ARG; robustness flags set: ICT_ERR_UNSUPPORTED.  The call changes nothing a later call reads:
+ * not the 2-D points of ict_tracker_get_2dpoints, not the carried "keep_state" arrays, not the teacher or the knobs. */
+int ict_track_evaluate(ict_tracker* tr, const ict_frames* fs, const int* ref_frame, const int* new_frame,
+                       const double* p_ref, const double* p_cur, int level, float* out_H, float* out_jtr, float* out_dp,
+                       float* out_ssr, int* out_nvis, float* out_pt_ssr);
+
 /* Reference 2-D points of the LAST SetPose at level lv_l (OdometerClass::Get2DPoints, odometer.h:30):
  * out float[2*n_t] per track at 2*pt_off[t]: x block then y block; 0 for the points beyond maxpttrack, which the
  * reference does not project. Host buffer. */

@@ -82,6 +82,8 @@ SIGNATURES = {
                                      C.c_void_p, C.c_void_p]),
     "ict_tracker_reproject": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "ict_tracker_get_2dpoints": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "ict_track_evaluate": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
+                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "ict_track_pair": (C.c_int, [C.POINTER(OptParam), _f, _f, _i, _f, _f, _d, C.c_int, _d, _d, C.c_void_p,
                                  C.c_void_p, C.c_int]),
     "ict_pose_hypotheses": (C.c_int, [_f, _f, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_double,
@@ -326,6 +328,27 @@ class Tracker:
         p_in = np.ascontiguousarray(np.broadcast_to(p_in, (self.T, 6)), np.float64)
         out = np.zeros(2 * self.total, np.float32)
         _check(lib().ict_tracker_reproject(self.h_, _p(p_in), _p(out)))
+        return out
+
+    def evaluate(self, frames, ref_frame, new_frame, p_ref, p_cur=None, level=None, per_point=False):
+        """One Gauss-Newton measurement per track at p_cur (default p_ref) with the template of SetPose(p_ref) at `level`
+        (default lv_l), see ict_track_evaluate: dict H (T,6,6), jtr (T,6), dp (T,6), ssr (T,), nvis (T,) and, with
+        per_point, pt_ssr (total,) laid out like the points (-1 where a point is not measured).  H is 4x J^T J: the
+        reference's gradients are twice the derivative."""
+        T = self.T
+        level = self.op.lv_l if level is None else int(level)
+        ref_frame = np.ascontiguousarray(np.broadcast_to(ref_frame, (T,)), np.int32)
+        new_frame = np.ascontiguousarray(np.broadcast_to(new_frame, (T,)), np.int32)
+        p_ref = np.ascontiguousarray(np.broadcast_to(p_ref, (T, 6)), np.float64)
+        p_cur = None if p_cur is None else np.ascontiguousarray(np.broadcast_to(p_cur, (T, 6)), np.float64)
+        H = np.zeros((T, 6, 6), np.float32); jtr = np.zeros((T, 6), np.float32); dp = np.zeros((T, 6), np.float32)
+        ssr = np.zeros(T, np.float32); nvis = np.zeros(T, np.int32)
+        pt = np.zeros(self.total, np.float32) if per_point else None
+        _check(lib().ict_track_evaluate(self.h_, frames.h_, _p(ref_frame), _p(new_frame), _p(p_ref), _p(p_cur), level,
+                                        _p(H), _p(jtr), _p(dp), _p(ssr), _p(nvis), _p(pt)))
+        out = dict(H=H, jtr=jtr, dp=dp, ssr=ssr, nvis=nvis)
+        if per_point:
+            out["pt_ssr"] = pt
         return out
 
     def get_2dpoints(self):

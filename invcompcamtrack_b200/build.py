@@ -14,7 +14,7 @@ NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 # -fmad=false: the reference is built without FMA (CMakeLists.txt:4), contraction would change its fp32 results
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-fmad=false", "-std=c++17",
               "-Xcompiler", "-fPIC", "-ccbin", "g++"] + os.environ.get("ICT_EXTRA_NVCC", "").split()
-LIB_SOURCES = ["ict_kernels.cu", "ict_kernel_v2.cu", "ict_kernel_v8.cu", "ict_kernel_x.cu", "ict_kernel_x8.cu", "ict_kernel_r.cu", "ict_kernels_big.cu", "ict_hypotheses.cu", "ict_capi.cu"]
+LIB_SOURCES = ["ict_kernels.cu", "ict_kernel_v2.cu", "ict_kernel_v8.cu", "ict_kernel_x.cu", "ict_kernel_x8.cu", "ict_kernel_r.cu", "ict_kernels_big.cu", "ict_hypotheses.cu", "ict_evaluate.cu", "ict_capi.cu"]
 LIB_DEPS = LIB_SOURCES + ["ict_kernels.cuh", "ict_device.cuh", "ict_kernel_v2.cuh", "ict_kernel_v8.cuh", "ict_kernel_x.cuh", os.path.join("..", "..", "include", "ictrack.h")]
 
 

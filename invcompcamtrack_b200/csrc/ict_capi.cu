@@ -471,6 +471,7 @@ struct ict_tracker {
   int seq_n = 0, seq_step = 0;   // set by ict_track_sequence around one run_tracks call (chain in one launch)
   const int *big_rf = nullptr, *big_nf = nullptr;   // set by ict_track_batch around run_tracks: per-track frames (host) of the multi-CTA path
   DevBuf pt_off, pts, pt3d, norm, p_in, p_out, iters, npix, trace, pt2d, rf, nf, big, teacher, state;
+  DevBuf ev, ev_in;              // ict_track_evaluate: scratch + outputs, per-call inputs (its own: no other call's data)
   int teacher_cap = 0;           // ict_tracker_set_teacher: records per track of the staged teacher poses (0: none)
   // several multi-CTA tracks in one call run on up to ICT_BIG_LANES streams side by side (each track is a chain of a few
   // hundred small launches: their latencies overlap); every lane has its own work buffer
@@ -505,7 +506,8 @@ ict_tracker* ict_tracker_create(const ict_optparam* op, const float fc[2], const
 void ict_tracker_destroy(ict_tracker* tr) {
   if (!tr) return;
   DevBuf* b[] = {&tr->pt_off, &tr->pts, &tr->pt3d, &tr->norm, &tr->p_in, &tr->p_out, &tr->iters,
-                 &tr->npix, &tr->trace, &tr->pt2d, &tr->rf, &tr->nf, &tr->big, &tr->teacher, &tr->state};
+                 &tr->npix, &tr->trace, &tr->pt2d, &tr->rf, &tr->nf, &tr->big, &tr->teacher, &tr->state,
+                 &tr->ev, &tr->ev_in};
   for (DevBuf* x : b) x->release();
   for (int k = 0; k < ict_tracker::ICT_BIG_LANES; ++k) {
     tr->big_lane[k].release();
@@ -925,6 +927,79 @@ int ict_tracker_reproject(ict_tracker* tr, const double* p_in, float* pt2d_out) 
   CU(launch_reproject(prm, 0));
   tr->have_2d = true;
   if (pt2d_out) CU(cudaMemcpy(pt2d_out, tr->pt2d.p, sizeof(float) * 2 * (size_t)tr->total, cudaMemcpyDeviceToHost));
+  return ICT_OK;
+}
+
+int ict_track_evaluate(ict_tracker* tr, const ict_frames* fs, const int* ref_frame, const int* new_frame,
+                       const double* p_ref, const double* p_cur, int level, float* out_H, float* out_jtr, float* out_dp,
+                       float* out_ssr, int* out_nvis, float* out_pt_ssr) {
+  if (!tr || !fs || !ref_frame || !new_frame || !p_ref) return fail(ICT_ERR_BAD_ARG, "null argument");
+  if (points_current(tr)) return ICT_ERR_BAD_ARG;
+  if (fs->lv_f != tr->op.lv_f || fs->pad != tr->op.psz || fs->w != tr->wh[0] || fs->h != tr->wh[1])
+    return fail(ICT_ERR_BAD_ARG, "frame store does not match the tracker (need lv_f, pad == psz, w, h equal)");
+  if (level < tr->op.lv_l || level > tr->op.lv_f) return fail(ICT_ERR_BAD_ARG, "ict_track_evaluate: level outside [lv_l, lv_f]");
+  if (tr->robust) return fail(ICT_ERR_UNSUPPORTED, "ict_track_evaluate measures the reference's model: clear the robustness flags");
+  const int T = tr->T;
+  for (int t = 0; t < T; ++t)
+    if (ref_frame[t] < 0 || ref_frame[t] >= fs->nframes || new_frame[t] < 0 || new_frame[t] >= fs->nframes)
+      return fail(ICT_ERR_BAD_ARG, "frame index out of range");
+  std::vector<int64_t> off = tr->h_off;
+  if (off.empty()) {   // points set from device memory
+    off.resize((size_t)T + 1);
+    CU(cudaMemcpy(off.data(), tr->pt_off.p, sizeof(int64_t) * (size_t)(T + 1), cudaMemcpyDeviceToHost));
+  }
+  EvalArgs a;
+  memset(&a, 0, sizeof(a));
+  a.op = tr->op;
+  a.cam = tr->cam;
+  a.frames = fs->desc;
+  a.pt_off = tr->pt_off.as<int64_t>();
+  a.pt3d = tr->pt3d.as<float>();
+  a.norm = tr->norm.as<double>();
+  a.T = T;
+  a.level = level;
+  a.ref_order = tr->sum_mode;
+  a.eigen_packet = tr->eigen_packet;
+  a.total = tr->total;
+  a.S = tr->total * tr->op.novals;
+  // tree order: the chunks of each track (a track's partial sums do not depend on the other tracks)
+  std::vector<int64_t> chunk_off((size_t)T + 1, 0);
+  for (int t = 0; t < T; ++t) {
+    const int64_t n = off[t + 1] - off[t];
+    const int64_t P = n < tr->op.maxpttrack ? n : tr->op.maxpttrack;
+    chunk_off[t + 1] = chunk_off[t] + (a.ref_order ? 0 : evaluate_chunks(P * tr->op.novals));
+  }
+  const int64_t nchunks = chunk_off[T];
+  const size_t in_bytes = sizeof(int64_t) * (T + 1) + sizeof(int) * 2 * (size_t)T + 8 + sizeof(double) * 12 * (size_t)T;
+  CU(tr->ev_in.reserve(in_bytes));
+  char* in = tr->ev_in.as<char>();
+  int64_t* d_chunk = (int64_t*)in;
+  int* d_rf = (int*)(d_chunk + T + 1);
+  int* d_nf = d_rf + T;
+  double* d_pref = (double*)(in + ((sizeof(int64_t) * (T + 1) + sizeof(int) * 2 * (size_t)T + 7) & ~(size_t)7));
+  double* d_pcur = d_pref + 6 * (size_t)T;
+  CU(tr->ev.reserve(evaluate_workspace(a, nchunks, nullptr)));
+  evaluate_workspace(a, nchunks, tr->ev.p);
+  CU(cudaMemcpyAsync(d_chunk, chunk_off.data(), sizeof(int64_t) * (size_t)(T + 1), cudaMemcpyHostToDevice, 0));
+  CU(cudaMemcpyAsync(d_rf, ref_frame, sizeof(int) * (size_t)T, cudaMemcpyHostToDevice, 0));
+  CU(cudaMemcpyAsync(d_nf, new_frame, sizeof(int) * (size_t)T, cudaMemcpyHostToDevice, 0));
+  CU(cudaMemcpyAsync(d_pref, p_ref, sizeof(double) * 6 * (size_t)T, cudaMemcpyHostToDevice, 0));
+  if (p_cur) CU(cudaMemcpyAsync(d_pcur, p_cur, sizeof(double) * 6 * (size_t)T, cudaMemcpyHostToDevice, 0));
+  CU(cudaMemsetAsync(a.nvis, 0, sizeof(int) * (size_t)T, 0));
+  a.chunk_off = d_chunk;
+  a.ref_frame = d_rf;
+  a.new_frame = d_nf;
+  a.p_ref = d_pref;
+  a.p_cur = p_cur ? d_pcur : nullptr;
+  CU(launch_evaluate(a, nchunks, 0));
+  if (out_H) CU(cudaMemcpyAsync(out_H, a.out_H, sizeof(float) * 36 * (size_t)T, cudaMemcpyDeviceToHost, 0));
+  if (out_jtr) CU(cudaMemcpyAsync(out_jtr, a.out_jtr, sizeof(float) * 6 * (size_t)T, cudaMemcpyDeviceToHost, 0));
+  if (out_dp) CU(cudaMemcpyAsync(out_dp, a.out_dp, sizeof(float) * 6 * (size_t)T, cudaMemcpyDeviceToHost, 0));
+  if (out_ssr) CU(cudaMemcpyAsync(out_ssr, a.out_ssr, sizeof(float) * (size_t)T, cudaMemcpyDeviceToHost, 0));
+  if (out_nvis) CU(cudaMemcpyAsync(out_nvis, a.nvis, sizeof(int) * (size_t)T, cudaMemcpyDeviceToHost, 0));
+  if (out_pt_ssr && tr->total)
+    CU(cudaMemcpyAsync(out_pt_ssr, a.pt_ssr, sizeof(float) * (size_t)tr->total, cudaMemcpyDeviceToHost, 0));
+  CU(cudaStreamSynchronize(0));
   return ICT_OK;
 }
 

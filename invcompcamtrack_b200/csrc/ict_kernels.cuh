@@ -131,6 +131,40 @@ struct BigTrackWork;
 size_t bigtrack_work_bytes(const ict_optparam& op, int64_t npts, int eigen_packet);
 cudaError_t launch_track_big(const TrackParams& prm, int t, int64_t npts, void* work, cudaStream_t stream);
 
+// ict_track_evaluate (ict_evaluate.cu): one measurement per track at a chosen pose.  All pointers device memory; the
+// scratch arrays are laid out by evaluate_workspace.
+struct EvalPoint;
+struct EvalArgs {
+  ict_optparam op;
+  CamLevels cam;
+  const FrameDesc* frames;
+  const int* ref_frame;            // [T]
+  const int* new_frame;            // [T]
+  const int64_t* pt_off;           // [T+1]
+  const float* pt3d;               // as TrackParams.pt3d
+  const double* norm;              // as TrackParams.norm
+  const double* p_ref;             // [T*6] SetPose pose
+  const double* p_cur;             // [T*6] measurement pose, or null: p_ref
+  int T, level;
+  int ref_order;                   // 1: Eigen packet order (eigen_packet 4 or 8); 0: fixed tree
+  int eigen_packet;                // packet width of the reference order and of the per-point sums
+  int64_t total, S;                // points, pixel slots (total * novals)
+  const int64_t* chunk_off;        // [T+1] tree order: first chunk of each track
+  // scratch
+  float *G_ref, *G_cur;            // [T*12]
+  EvalPoint* pts;                  // [total]
+  float *sd, *ref, *pd;            // [6*S], [S], [S]
+  float *chains, *partials;        // [T*28*2W] reference order, [chunks*28] tree order
+  int* nvis;                       // [T], zeroed before the launch
+  // outputs
+  float *out_H, *out_jtr, *out_dp, *out_ssr, *pt_ssr;   // [T*36], [T*6], [T*6], [T], [total]
+};
+// Bytes of scratch + outputs for a's sizes (T, total, S, eigen_packet) and nchunks tree chunks; with base != null also
+// points a's scratch and output pointers into it.
+size_t evaluate_workspace(EvalArgs& a, int64_t nchunks, void* base);
+int64_t evaluate_chunks(int64_t pixels);   // tree-order chunks of a track with that many pixel slots
+cudaError_t launch_evaluate(const EvalArgs& a, int64_t nchunks, cudaStream_t stream);
+
 // NCC hypothesis scoring, run_track_nposes.cpp:271-355
 cudaError_t launch_ncc(const ict_optparam& op, const CamLevels& cam, const float* img_b, const float* img_r,
                        const float* img_f, int nback, int nfwd, const int64_t* pt_off, int T, const float* pb,
