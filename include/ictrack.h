@@ -276,6 +276,24 @@ int ict_track_evaluate(ict_tracker* tr, const ict_frames* fs, const int* ref_fra
                        const double* p_ref, const double* p_cur, int level, float* out_H, float* out_jtr, float* out_dp,
                        float* out_ssr, int* out_nvis, float* out_pt_ssr);
 
+/* ---- many candidate poses per track against one template ----------------------------------------------------------
+ * K measurements per track: for every k, the outputs for candidate k are bit for bit those of ict_track_evaluate(tr, fs,
+ * ref_frame, new_frame, p_ref, p_cur = candidate k, level, ...), in every sum order, and out_H is that call's H.  The
+ * template, steepest-descent images, H and its factorisation depend on p_ref only and are built once per track; only the
+ * projection, new patch, J^T r, step and SSR are redone per candidate.  So every rule of ict_track_evaluate holds
+ * unchanged: the template state at `level`, stale slots, the maxpttrack cap, empty and NaN one-point donorm tracks,
+ * points outside the new image.  Host buffers; any output may be NULL:
+ *   p_cand    double[T*K*6]  candidate k of track t at (t*K + k)*6, as p_cur of ict_track_evaluate
+ *   out_H     float[T*36]    once per track
+ *   out_jtr   float[T*K*6]   out_dp float[T*K*6]   out_ssr float[T*K]   out_nvis int[T*K]   (track t, candidate k at
+ *                            t*K + k)
+ * Errors are those of ict_track_evaluate, and ICT_ERR_BAD_ARG for K < 1, a NULL p_cand or T*K beyond INT_MAX;
+ * ICT_ERR_NOMEM when the scratch (it grows with T*K and with the points times K) cannot be allocated.  Like
+ * ict_track_evaluate, the call changes nothing a later call reads. */
+int ict_track_evaluate_poses(ict_tracker* tr, const ict_frames* fs, const int* ref_frame, const int* new_frame,
+                             const double* p_ref, int K, const double* p_cand, int level, float* out_H, float* out_jtr,
+                             float* out_dp, float* out_ssr, int* out_nvis);
+
 /* Reference 2-D points of the LAST SetPose at level lv_l (OdometerClass::Get2DPoints, odometer.h:30):
  * out float[2*n_t] per track at 2*pt_off[t]: x block then y block; 0 for the points beyond maxpttrack, which the
  * reference does not project. Host buffer. */

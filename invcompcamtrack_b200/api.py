@@ -84,6 +84,9 @@ SIGNATURES = {
     "ict_tracker_get_2dpoints": (C.c_int, [C.c_void_p, C.c_void_p]),
     "ict_track_evaluate": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
                                      C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "ict_track_evaluate_poses": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
+                                           C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                           C.c_void_p]),
     "ict_track_pair": (C.c_int, [C.POINTER(OptParam), _f, _f, _i, _f, _f, _d, C.c_int, _d, _d, C.c_void_p,
                                  C.c_void_p, C.c_int]),
     "ict_pose_hypotheses": (C.c_int, [_f, _f, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_double,
@@ -350,6 +353,26 @@ class Tracker:
         if per_point:
             out["pt_ssr"] = pt
         return out
+
+    def evaluate_poses(self, frames, ref_frame, new_frame, p_ref, p_cand, level=None):
+        """evaluate at K candidate poses per track against the template of SetPose(p_ref) at `level` (default lv_l),
+        see ict_track_evaluate_poses: p_cand (T, K, 6), broadcast like evaluate's arguments.  Returns dict H (T,6,6),
+        once per track, and jtr (T,K,6), dp (T,K,6), ssr (T,K), nvis (T,K); [:, k] is evaluate(p_cur=p_cand[:, k])."""
+        T = self.T
+        level = self.op.lv_l if level is None else int(level)
+        p_cand = np.asarray(p_cand, np.float64)
+        if p_cand.ndim < 2 or p_cand.shape[-1] != 6:
+            raise ValueError("p_cand must have shape (T, K, 6) or broadcast to it")
+        K = p_cand.shape[-2]
+        ref_frame = np.ascontiguousarray(np.broadcast_to(ref_frame, (T,)), np.int32)
+        new_frame = np.ascontiguousarray(np.broadcast_to(new_frame, (T,)), np.int32)
+        p_ref = np.ascontiguousarray(np.broadcast_to(p_ref, (T, 6)), np.float64)
+        p_cand = np.ascontiguousarray(np.broadcast_to(p_cand, (T, K, 6)))
+        H = np.zeros((T, 6, 6), np.float32); jtr = np.zeros((T, K, 6), np.float32)
+        dp = np.zeros((T, K, 6), np.float32); ssr = np.zeros((T, K), np.float32); nvis = np.zeros((T, K), np.int32)
+        _check(lib().ict_track_evaluate_poses(self.h_, frames.h_, _p(ref_frame), _p(new_frame), _p(p_ref), K,
+                                              _p(p_cand), level, _p(H), _p(jtr), _p(dp), _p(ssr), _p(nvis)))
+        return dict(H=H, jtr=jtr, dp=dp, ssr=ssr, nvis=nvis)
 
     def get_2dpoints(self):
         out = np.zeros(2 * self.total, np.float32)

@@ -3,6 +3,7 @@
 #include "ict_kernels.cuh"
 
 #include <cuda.h>
+#include <limits.h>
 #include <math.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -930,15 +931,16 @@ int ict_tracker_reproject(ict_tracker* tr, const double* p_in, float* pt2d_out) 
   return ICT_OK;
 }
 
-int ict_track_evaluate(ict_tracker* tr, const ict_frames* fs, const int* ref_frame, const int* new_frame,
-                       const double* p_ref, const double* p_cur, int level, float* out_H, float* out_jtr, float* out_dp,
-                       float* out_ssr, int* out_nvis, float* out_pt_ssr) {
+// the checks and the per-track setup shared by ict_track_evaluate and ict_track_evaluate_poses: EvalArgs without its
+// scratch, the host copy of the tree-order chunk offsets
+static int evaluate_setup(ict_tracker* tr, const ict_frames* fs, const int* ref_frame, const int* new_frame,
+                          const double* p_ref, int level, const char* who, EvalArgs& a, std::vector<int64_t>& chunk_off) {
   if (!tr || !fs || !ref_frame || !new_frame || !p_ref) return fail(ICT_ERR_BAD_ARG, "null argument");
   if (points_current(tr)) return ICT_ERR_BAD_ARG;
   if (fs->lv_f != tr->op.lv_f || fs->pad != tr->op.psz || fs->w != tr->wh[0] || fs->h != tr->wh[1])
     return fail(ICT_ERR_BAD_ARG, "frame store does not match the tracker (need lv_f, pad == psz, w, h equal)");
-  if (level < tr->op.lv_l || level > tr->op.lv_f) return fail(ICT_ERR_BAD_ARG, "ict_track_evaluate: level outside [lv_l, lv_f]");
-  if (tr->robust) return fail(ICT_ERR_UNSUPPORTED, "ict_track_evaluate measures the reference's model: clear the robustness flags");
+  if (level < tr->op.lv_l || level > tr->op.lv_f) return fail(ICT_ERR_BAD_ARG, std::string(who) + ": level outside [lv_l, lv_f]");
+  if (tr->robust) return fail(ICT_ERR_UNSUPPORTED, std::string(who) + " measures the reference's model: clear the robustness flags");
   const int T = tr->T;
   for (int t = 0; t < T; ++t)
     if (ref_frame[t] < 0 || ref_frame[t] >= fs->nframes || new_frame[t] < 0 || new_frame[t] >= fs->nframes)
@@ -948,7 +950,6 @@ int ict_track_evaluate(ict_tracker* tr, const ict_frames* fs, const int* ref_fra
     off.resize((size_t)T + 1);
     CU(cudaMemcpy(off.data(), tr->pt_off.p, sizeof(int64_t) * (size_t)(T + 1), cudaMemcpyDeviceToHost));
   }
-  EvalArgs a;
   memset(&a, 0, sizeof(a));
   a.op = tr->op;
   a.cam = tr->cam;
@@ -963,12 +964,22 @@ int ict_track_evaluate(ict_tracker* tr, const ict_frames* fs, const int* ref_fra
   a.total = tr->total;
   a.S = tr->total * tr->op.novals;
   // tree order: the chunks of each track (a track's partial sums do not depend on the other tracks)
-  std::vector<int64_t> chunk_off((size_t)T + 1, 0);
+  chunk_off.assign((size_t)T + 1, 0);
   for (int t = 0; t < T; ++t) {
     const int64_t n = off[t + 1] - off[t];
     const int64_t P = n < tr->op.maxpttrack ? n : tr->op.maxpttrack;
     chunk_off[t + 1] = chunk_off[t] + (a.ref_order ? 0 : evaluate_chunks(P * tr->op.novals));
   }
+  return ICT_OK;
+}
+
+int ict_track_evaluate(ict_tracker* tr, const ict_frames* fs, const int* ref_frame, const int* new_frame,
+                       const double* p_ref, const double* p_cur, int level, float* out_H, float* out_jtr, float* out_dp,
+                       float* out_ssr, int* out_nvis, float* out_pt_ssr) {
+  EvalArgs a;
+  std::vector<int64_t> chunk_off;
+  if (int rc = evaluate_setup(tr, fs, ref_frame, new_frame, p_ref, level, "ict_track_evaluate", a, chunk_off)) return rc;
+  const int T = tr->T;
   const int64_t nchunks = chunk_off[T];
   const size_t in_bytes = sizeof(int64_t) * (T + 1) + sizeof(int) * 2 * (size_t)T + 8 + sizeof(double) * 12 * (size_t)T;
   CU(tr->ev_in.reserve(in_bytes));
@@ -999,6 +1010,56 @@ int ict_track_evaluate(ict_tracker* tr, const ict_frames* fs, const int* ref_fra
   if (out_nvis) CU(cudaMemcpyAsync(out_nvis, a.nvis, sizeof(int) * (size_t)T, cudaMemcpyDeviceToHost, 0));
   if (out_pt_ssr && tr->total)
     CU(cudaMemcpyAsync(out_pt_ssr, a.pt_ssr, sizeof(float) * (size_t)tr->total, cudaMemcpyDeviceToHost, 0));
+  CU(cudaStreamSynchronize(0));
+  return ICT_OK;
+}
+
+int ict_track_evaluate_poses(ict_tracker* tr, const ict_frames* fs, const int* ref_frame, const int* new_frame,
+                             const double* p_ref, int K, const double* p_cand, int level, float* out_H, float* out_jtr,
+                             float* out_dp, float* out_ssr, int* out_nvis) {
+  EvalArgs a;
+  std::vector<int64_t> chunk_off;
+  if (int rc = evaluate_setup(tr, fs, ref_frame, new_frame, p_ref, level, "ict_track_evaluate_poses", a, chunk_off))
+    return rc;
+  if (K < 1 || !p_cand) return fail(ICT_ERR_BAD_ARG, "ict_track_evaluate_poses: need K >= 1 and p_cand");
+  const int T = tr->T;
+  const int64_t TK = (int64_t)T * K;
+  if (TK > INT_MAX) return fail(ICT_ERR_BAD_ARG, "ict_track_evaluate_poses: T*K beyond INT_MAX");
+  const int64_t nchunks = chunk_off[T];
+  EvalPoses b;
+  memset(&b, 0, sizeof(b));
+  b.K = K;
+  const size_t head = (sizeof(int64_t) * (T + 1) + sizeof(int) * 2 * (size_t)T + 7) & ~(size_t)7;
+  CU(tr->ev_in.reserve(head + sizeof(double) * 6 * ((size_t)T + (size_t)TK)));
+  char* in = tr->ev_in.as<char>();
+  int64_t* d_chunk = (int64_t*)in;
+  int* d_rf = (int*)(d_chunk + T + 1);
+  int* d_nf = d_rf + T;
+  double* d_pref = (double*)(in + head);
+  double* d_pcand = d_pref + 6 * (size_t)T;
+  const size_t ws = evaluate_poses_workspace(a, b, nchunks, nullptr);
+  if (tr->ev.reserve(ws) != cudaSuccess) {
+    cudaGetLastError();
+    return fail(ICT_ERR_NOMEM, "ict_track_evaluate_poses: cannot allocate " + std::to_string(ws) + " bytes of scratch");
+  }
+  evaluate_poses_workspace(a, b, nchunks, tr->ev.p);
+  CU(cudaMemcpyAsync(d_chunk, chunk_off.data(), sizeof(int64_t) * (size_t)(T + 1), cudaMemcpyHostToDevice, 0));
+  CU(cudaMemcpyAsync(d_rf, ref_frame, sizeof(int) * (size_t)T, cudaMemcpyHostToDevice, 0));
+  CU(cudaMemcpyAsync(d_nf, new_frame, sizeof(int) * (size_t)T, cudaMemcpyHostToDevice, 0));
+  CU(cudaMemcpyAsync(d_pref, p_ref, sizeof(double) * 6 * (size_t)T, cudaMemcpyHostToDevice, 0));
+  CU(cudaMemcpyAsync(d_pcand, p_cand, sizeof(double) * 6 * (size_t)TK, cudaMemcpyHostToDevice, 0));
+  CU(cudaMemsetAsync(b.nvis, 0, sizeof(int) * (size_t)TK, 0));
+  a.chunk_off = d_chunk;
+  a.ref_frame = d_rf;
+  a.new_frame = d_nf;
+  a.p_ref = d_pref;
+  b.p_cand = d_pcand;
+  CU(launch_evaluate_poses(a, b, nchunks, 0));
+  if (out_H) CU(cudaMemcpyAsync(out_H, a.out_H, sizeof(float) * 36 * (size_t)T, cudaMemcpyDeviceToHost, 0));
+  if (out_jtr) CU(cudaMemcpyAsync(out_jtr, b.out_jtr, sizeof(float) * 6 * (size_t)TK, cudaMemcpyDeviceToHost, 0));
+  if (out_dp) CU(cudaMemcpyAsync(out_dp, b.out_dp, sizeof(float) * 6 * (size_t)TK, cudaMemcpyDeviceToHost, 0));
+  if (out_ssr) CU(cudaMemcpyAsync(out_ssr, b.out_ssr, sizeof(float) * (size_t)TK, cudaMemcpyDeviceToHost, 0));
+  if (out_nvis) CU(cudaMemcpyAsync(out_nvis, b.nvis, sizeof(int) * (size_t)TK, cudaMemcpyDeviceToHost, 0));
   CU(cudaStreamSynchronize(0));
   return ICT_OK;
 }

@@ -134,6 +134,7 @@ cudaError_t launch_track_big(const TrackParams& prm, int t, int64_t npts, void* 
 // ict_track_evaluate (ict_evaluate.cu): one measurement per track at a chosen pose.  All pointers device memory; the
 // scratch arrays are laid out by evaluate_workspace.
 struct EvalPoint;
+struct Lu6;
 struct EvalArgs {
   ict_optparam op;
   CamLevels cam;
@@ -158,12 +159,29 @@ struct EvalArgs {
   int* nvis;                       // [T], zeroed before the launch
   // outputs
   float *out_H, *out_jtr, *out_dp, *out_ssr, *pt_ssr;   // [T*36], [T*6], [T*6], [T], [total]
+  Lu6* lu;                         // [T] each track's factorisation of H, or null (ict_track_evaluate_poses)
 };
 // Bytes of scratch + outputs for a's sizes (T, total, S, eigen_packet) and nchunks tree chunks; with base != null also
 // points a's scratch and output pointers into it.
 size_t evaluate_workspace(EvalArgs& a, int64_t nchunks, void* base);
 int64_t evaluate_chunks(int64_t pixels);   // tree-order chunks of a track with that many pixel slots
 cudaError_t launch_evaluate(const EvalArgs& a, int64_t nchunks, cudaStream_t stream);
+
+// ict_track_evaluate_poses (ict_evaluate.cu): K measurements per track, one per candidate pose, against the template
+// and the factorised H of SetPose(p_ref) built once per track.  The EvalArgs part carries the per-track template pass
+// (p_cur null, out_jtr / out_dp / out_ssr / pt_ssr null, out_H and lu set); the candidate arrays scale with K.
+struct EvalCand;
+struct EvalPoses {
+  int K;
+  const double* p_cand;            // [T*K*6] candidate k of track t at (t*K + k)*6
+  float* G_cand;                   // [T*K*12]
+  EvalCand* cand;                  // [total*K] point g, candidate k at g*K + k
+  float *chains, *partials;        // [T*K*7*2W] reference order, [chunks*K*7] tree order
+  int* nvis;                       // [T*K], zeroed before the launch
+  float *out_jtr, *out_dp, *out_ssr;   // [T*K*6], [T*K*6], [T*K]
+};
+size_t evaluate_poses_workspace(EvalArgs& a, EvalPoses& b, int64_t nchunks, void* base);
+cudaError_t launch_evaluate_poses(const EvalArgs& a, const EvalPoses& b, int64_t nchunks, cudaStream_t stream);
 
 // NCC hypothesis scoring, run_track_nposes.cpp:271-355
 cudaError_t launch_ncc(const ict_optparam& op, const CamLevels& cam, const float* img_b, const float* img_r,
