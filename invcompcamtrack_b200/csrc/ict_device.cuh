@@ -7,6 +7,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include "ict_kernels.cuh"
 
 #define ICT_LIEALG_SIGTHRESH 1e-4   /* utilities.h:22 */
 #define ICT_LIEALG_EPSILON 1e-10    /* utilities.h:23 */
@@ -288,6 +289,104 @@ static __device__ __noinline__ void getpose_se3(const float* cpos_p, const float
   }
 #pragma unroll
   for (int k = 0; k < 6; ++k) p_out[k] = (double)pu[k];
+}
+
+// ---- the per-track bookkeeping every tracking kernel shares: what a track reads and reports (ictrack.h) -----------
+// G (3 x 4, row-major) applied to a point, pose.cpp:307-397 / 400-488
+template <typename T>
+__device__ __forceinline__ void rigid_apply(const T* G, T X, T Y, T Z, T& x, T& y, T& z) {
+  x = G[0] * X + G[1] * Y + G[2] * Z + G[3];
+  y = G[4] * X + G[5] * Y + G[6] * Z + G[7];
+  z = G[8] * X + G[9] * Y + G[10] * Z + G[11];
+}
+
+// the reference and new frame of track t; a sequence step adds its frame offset (K2v8's chains)
+struct TrackFrames {
+  const FrameDesc* ref;
+  const FrameDesc* nw;
+};
+__device__ __forceinline__ TrackFrames track_frames(const TrackParams& prm, int t, int shift = 0) {
+  const int rf = (prm.ref_frame ? prm.ref_frame[t] : prm.fixed_ref) + shift;
+  const int nf = (prm.new_frame ? prm.new_frame[t] : prm.fixed_new) + shift;
+  return {prm.frames + rf, prm.frames + nf};
+}
+
+// SetPose (pose.cpp:25-76) of track t from its row of p_in and its normalisation (norm: meanshift[3], varval)
+__device__ __forceinline__ void track_setpose(const double* p_in, const double* norm, int t, bool donorm, float* p,
+                                              float* G) {
+  setpose_se3(p_in + 6 * (int64_t)t, donorm, norm + 4 * (int64_t)t, norm[4 * (int64_t)t + 3], p, G);
+}
+
+// project_pt_save_rotated (pose.cpp:400-488) of point i at the SetPose pose G: the camera-frame point into Xc/Yc/Zc
+// (SAVE), and Get2DPoints() (odometer.h:30), the point at level lv_l, into pt2d_out (when set)
+template <bool SAVE = true, typename I>
+__device__ __forceinline__ void save_rotated_point(const TrackParams& prm, const float* G, int64_t off, int n_in, I i,
+                                                   float X, float Y, float Z, float* Xc, float* Yc, float* Zc) {
+  float xc, yc, zc;
+  rigid_apply(G, X, Y, Z, xc, yc, zc);
+  if (SAVE) {
+    Xc[i] = xc;
+    Yc[i] = yc;
+    Zc[i] = zc;
+  }
+  if (prm.pt2d_out) {
+    const int l = prm.op.lv_l;
+    prm.pt2d_out[2 * off + i] = (xc / zc) * prm.cam.fx[l] + prm.cam.cx[l];
+    prm.pt2d_out[2 * off + n_in + i] = (yc / zc) * prm.cam.fy[l] + prm.cam.cy[l];
+  }
+}
+
+// lpNorm<1> of delta_p (odometer.cpp:412) in the reference's association order
+__device__ __forceinline__ float normdp_l1(const float* dp) {
+  return ((fabsf(dp[0]) + fabsf(dp[2])) + (fabsf(dp[1]) + fabsf(dp[3]))) + (fabsf(dp[4]) + fabsf(dp[5]));
+}
+
+// the stop rule (odometer.cpp:341-346) after `done` iterations of a level: go on while done < maxiter and the step
+// norm relative to the level's first is above normdp_ratio.  A level starts at normdp = normdp_init = 1e-10:
+// keep_iterating(op, 0, 1e-10f, 1e-10f).
+__device__ __forceinline__ int keep_iterating(const ict_optparam& op, int done, float normdp, float normdp_init) {
+  return (done < op.maxiter) & ((normdp / normdp_init) > op.normdp_ratio);
+}
+
+// track t's trace records (ICT_TRACE_FLOATS floats each), or null
+__device__ __forceinline__ float* track_trace(const TrackParams& prm, int t) {
+  return prm.trace ? prm.trace + (int64_t)t * prm.trace_cap * ICT_TRACE_FLOATS : nullptr;
+}
+
+// fields 0-15 of an iteration's trace record (level, iteration, J^T r, delta_p, normdp, visible points), 16-23 zeroed:
+// kernels that record cycle counts there write them afterwards
+__device__ __forceinline__ void trace_record(float* rec, int sl, int it, const float* jtr, const float* dp, float normdp,
+                                             int nvis) {
+  rec[0] = (float)sl;
+  rec[1] = (float)it;
+  for (int k = 0; k < 6; ++k) { rec[2 + k] = jtr[k]; rec[8 + k] = dp[k]; }
+  rec[14] = normdp;
+  rec[15] = (float)nvis;
+  for (int k = 16; k < ICT_TRACE_FLOATS; ++k) rec[k] = 0.0f;
+}
+
+// the records from..cap-1 that no iteration filled: (-1, 0, ..., 0)
+__device__ __forceinline__ void pad_trace(float* trace, int from, int cap) {
+  if (!trace) return;
+  for (int k = from; k < cap; ++k) {
+    float* rec = trace + (int64_t)ICT_TRACE_FLOATS * k;
+    for (int j = 0; j < ICT_TRACE_FLOATS; ++j) rec[j] = 0.0f;
+    rec[0] = -1.0f;
+  }
+}
+
+// iterations of level sl of track t, at iters[t][lv_f - sl] (when iters is set)
+__device__ __forceinline__ void store_level_iters(int* iters, const ict_optparam& op, int t, int sl, int n) {
+  if (iters) iters[(int64_t)t * (op.lv_f - op.lv_l + 1) + (op.lv_f - sl)] = n;
+}
+
+// the end of track t (one thread): getPose_se3 into row t of p_out, the pixel-residual count, the trace padding
+__device__ __forceinline__ void finish_track(const TrackParams& prm, int t, bool donorm, const float* p, const float* G,
+                                             double* p_out, long long* npixres, long long npix, float* trace,
+                                             int trace_n) {
+  getpose_se3(p, G, donorm, prm.norm + 4 * (int64_t)t, prm.norm[4 * (int64_t)t + 3], p_out + 6 * (int64_t)t);
+  if (npixres) npixres[t] = npix;
+  pad_trace(trace, trace_n, prm.trace_cap);
 }
 
 // ---- Hes.fullPivLu() (odometer.cpp:514), factor once per level; same elimination order as Eigen 3.3 ----------

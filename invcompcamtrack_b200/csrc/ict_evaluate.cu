@@ -25,7 +25,6 @@
 
 namespace ict {
 
-void count_launch_external();
 
 #define ICT_EVAL_NQ 28          // 21 H + 6 J^T r + 1 SSR
 #define ICT_EVAL_CHUNK 4096     // pixels per CTA of the tree-order partials
@@ -562,10 +561,10 @@ size_t evaluate_poses_workspace(EvalArgs& a, EvalPoses& b, int64_t nchunks, void
 
 // SetPose poses, the points' placements, the template and sd of every pixel slot
 static void launch_eval_template(const EvalArgs& a, cudaStream_t st) {
-  count_launch_external();
+  count_launch();
   k_eval_pose<<<(unsigned)((a.T + 127) / 128), 128, 0, st>>>(a);
   if (a.total > 0) {
-    for (int k = 0; k < 2; ++k) count_launch_external();
+    for (int k = 0; k < 2; ++k) count_launch();
     k_eval_points<<<(unsigned)((a.total + 255) / 256), 256, 0, st>>>(a);
     k_eval_slots<<<(unsigned)((a.S + 255) / 256), 256, 0, st>>>(a);
   }
@@ -575,8 +574,8 @@ static void launch_eval_template(const EvalArgs& a, cudaStream_t st) {
 static void launch_eval_sums(const EvalArgs& a, int64_t nchunks, cudaStream_t st) {
   const int64_t T = a.T;
   const unsigned solve_blocks = (unsigned)((T + 3) / 4);
-  count_launch_external();                                 // the sums
-  if (a.ref_order || nchunks > 0) count_launch_external();  // the solve
+  count_launch();                                 // the sums
+  if (a.ref_order || nchunks > 0) count_launch();  // the solve
   if (a.ref_order) {
     const int64_t nthr = T * ICT_EVAL_NQ * 2 * a.eigen_packet;
     if (a.eigen_packet == 8) {
@@ -596,7 +595,7 @@ cudaError_t launch_evaluate(const EvalArgs& a, int64_t nchunks, cudaStream_t st)
   if (a.T <= 0) return cudaSuccess;
   launch_eval_template(a, st);
   if (a.total > 0) {
-    count_launch_external();
+    count_launch();
     if (a.eigen_packet == 8)
       k_eval_patch<8><<<(unsigned)((a.total + 127) / 128), 128, 0, st>>>(a);
     else
@@ -615,26 +614,26 @@ static cudaError_t launch_poses_w(const EvalArgs& a, const EvalPoses& b, int64_t
   // the J^T r, SSR and visible count of that pass are neither kept nor read)
   launch_eval_template(a, st);
   if (a.total > 0) {
-    count_launch_external();
+    count_launch();
     k_evp_template<W><<<(unsigned)((a.total + 127) / 128), 128, 0, st>>>(a);
   }
   launch_eval_sums(a, nchunks, st);
   // per candidate
-  count_launch_external();
+  count_launch();
   k_evp_pose<<<(unsigned)((TK + 127) / 128), 128, 0, st>>>(a, b);
   if (a.total > 0) {
-    count_launch_external();
+    count_launch();
     const dim3 grid((unsigned)((a.total + 255) / 256), (unsigned)(b.K < 65535 ? b.K : 65535));
     k_evp_points<W><<<grid, 256, 0, st>>>(a, b);
   }
   if (a.ref_order) {
-    count_launch_external();
+    count_launch();
     k_evp_chains<W><<<(unsigned)((a.T * ng * 2 * W + 255) / 256), 256, 0, st>>>(a, b);
   } else if (nchunks > 0) {
-    count_launch_external();
+    count_launch();
     k_evp_partials<<<(unsigned)(nchunks * ng), 256, 0, st>>>(a, b);
   }
-  count_launch_external();
+  count_launch();
   if (a.ref_order)
     k_evp_solve<W, true><<<(unsigned)((TK + 127) / 128), 128, 0, st>>>(a, b);
   else

@@ -14,7 +14,6 @@
 
 namespace ict {
 
-void count_launch_external();
 
 struct HypArgs {
   double fx, fy, cx, cy;
@@ -61,8 +60,8 @@ __device__ double hyp_cost(const HypArgs& a, const double* G, const int* id, dou
   for (int m = 0; m < 4; ++m) {
     const int i = id[m];
     const double X = a.pt3d[i], Y = a.pt3d[a.npts + i], Z = a.pt3d[2 * a.npts + i];
-    const double xc = G[0] * X + G[1] * Y + G[2] * Z + G[3], yc = G[4] * X + G[5] * Y + G[6] * Z + G[7];
-    const double zc = G[8] * X + G[9] * Y + G[10] * Z + G[11];
+    double xc, yc, zc;
+    rigid_apply(G, X, Y, Z, xc, yc, zc);
     Xc[3 * m] = xc; Xc[3 * m + 1] = yc; Xc[3 * m + 2] = zc;
     if (!(zc > 1e-12)) return -1.0;
     r[2 * m] = xc / zc * a.fx + a.cx - a.pt2d[i];
@@ -197,9 +196,9 @@ cudaError_t launch_hypotheses(const double fc[2], const double cc[2], int npts, 
   for (int k = 0; k < 6; ++k) a.p_init[k] = p_init[k];
   a.pose = pose; a.status = status; a.ninl = ninl; a.mask = mask;
   k_hyp_solve<<<(nsamples + 127) / 128, 128, 0, stream>>>(a);
-  count_launch_external();
+  count_launch();
   k_hyp_inliers<<<nsamples, 256, 0, stream>>>(a);
-  count_launch_external();
+  count_launch();
   return cudaGetLastError();
 }
 

@@ -13,9 +13,8 @@ __device__ __forceinline__ float4 ld4s(const float* p) { return *reinterpret_cas
 __device__ __forceinline__ int place_point(const float* G, float X, float Y, float Z, float fx, float fy, float cx,
                                            float cy, float swo, float sho, int width, float4* dst, int pszd2 = 16,
                                            bool consistent = false) {
-  const float tx = G[0] * X + G[1] * Y + G[2] * Z + G[3];
-  const float ty = G[4] * X + G[5] * Y + G[6] * Z + G[7];
-  const float tz = G[8] * X + G[9] * Y + G[10] * Z + G[11];
+  float tx, ty, tz;
+  rigid_apply(G, X, Y, Z, tx, ty, tz);
   const float mx = (tx / tz) * fx + cx, my = (ty / tz) * fy + cy;
   const int vis = (mx >= 0) & (my >= 0) & (mx <= swo) & (my <= sho);   // odometer.cpp:369-371 (NaN -> outside)
   PatchPlace pl = {0, 0.f, 0.f, 0.f, 0.f};

@@ -66,6 +66,39 @@ struct TrackParams {
 
 #define ICT_TRACK_SMEM_LIMIT (227 * 1024 - 8192)
 
+// points per track a kernel's shared-memory layout holds for a track set whose largest track has max_pts points
+inline int track_pcap(const ict_optparam& op, int max_pts) { return max_pts < op.maxpttrack ? max_pts : op.maxpttrack; }
+
+int64_t launch_count(int reset);
+void count_launch();               // adds one kernel launch to launch_count
+
+// Sets kernel K's dynamic shared-memory limit and, with carveout >= 0, its preferred shared-memory carve-out (percent)
+// once per device (function attributes are per device).  Templated on the kernel itself: the instances of a kernel
+// template share one function-pointer type, and each needs its own attributes.
+template <auto K>
+cudaError_t set_kernel_attrs(int smem_limit, int carveout) {
+  static bool attr_dev[64] = {};
+  int dev = 0;
+  cudaGetDevice(&dev);
+  if (attr_dev[dev & 63]) return cudaSuccess;
+  cudaError_t e = cudaFuncSetAttribute(K, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_limit);
+  if (e == cudaSuccess && carveout >= 0) e = cudaFuncSetAttribute(K, cudaFuncAttributePreferredSharedMemoryCarveout, carveout);
+  if (e == cudaSuccess) attr_dev[dev & 63] = true;
+  return e;
+}
+
+// One counted launch of the CTA-per-track kernel K, allowed up to ICT_TRACK_SMEM_LIMIT of dynamic shared memory
+// (carveout as set_kernel_attrs).
+template <auto K, typename... Args>
+cudaError_t launch_cta_kernel(dim3 grid, int threads, size_t smem, int carveout, cudaStream_t stream,
+                              const Args&... args) {
+  const cudaError_t e = set_kernel_attrs<K>(ICT_TRACK_SMEM_LIMIT, carveout);
+  if (e != cudaSuccess) return e;
+  K<<<grid, threads, smem, stream>>>(args...);
+  count_launch();
+  return cudaGetLastError();
+}
+
 // ---- launches (all asynchronous on `stream`) -------------------------------------------------------------------
 // K0: util_constructpyramide for `count` frames.  src is float (src_u8 == nullptr) or uint8.
 cudaError_t launch_pyramid(const float* src_f32, const unsigned char* src_u8, int count, int w, int h, int lv_f,
@@ -197,7 +230,5 @@ cudaError_t launch_get_patches(const float* I, const float* dx, const float* dy,
 cudaError_t launch_hypotheses(const double fc[2], const double cc[2], int npts, const double* pt2d, const double* pt3d,
                               int nsamples, const int* sample, const double p_init[6], double inlthresh, int maxiter,
                               double* pose, int* status, int* ninl, unsigned char* mask, cudaStream_t stream);
-
-int64_t launch_count(int reset);
 
 }  // namespace ict
