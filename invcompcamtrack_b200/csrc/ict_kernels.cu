@@ -1115,12 +1115,9 @@ TrackKernel select_track_kernel(const ict_optparam& op, int max_pts, int sum_mod
   return general_fits ? TrackKernel::General : TrackKernel::MultiCta;
 }
 
-cudaError_t launch_track(const TrackParams& prm, int max_pts, cudaStream_t stream) {
+cudaError_t launch_track(const TrackParams& prm, TrackKernel k, int max_pts, cudaStream_t stream) {
   if (prm.T <= 0) return cudaSuccess;
-  const TrackKernel k = select_track_kernel(prm.op, max_pts, prm.sum_mode, prm.eigen_packet, prm.force_general,
-                                            prm.knob_no_k2r, prm.tma_ok);
-  if (prm.seq_n > 1 && (k != TrackKernel::V8 || prm.knob_seq_launches))
-    return cudaErrorInvalidConfiguration;   // only K2v8 loops over frames
+  if (prm.seq_n > 1 && k != TrackKernel::V8) return cudaErrorInvalidConfiguration;   // only K2v8 loops over frames
   const int P = track_pcap(prm.op, max_pts);
   const long long E = (long long)P * prm.op.novals;
   const int nt = E >= 2048 ? 256 : (E >= 512 ? 128 : 64);

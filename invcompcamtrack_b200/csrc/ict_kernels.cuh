@@ -46,7 +46,7 @@ struct TrackParams {
   float* pt2d_out;                 // [2*total] or null: reference 2-D points at lv_l (Get2DPoints)
   int T;                           // tracks in this launch
   int t0;                          // first track of this launch (index into the per-track arrays)
-  int force_general;               // 1: always use the general kernel k_track (tests compare the two)
+  int force_general;               // sum order 2: the multi-CTA path runs without its fused sums (tests compare the two)
   int seq_n, seq_step;             // K2v8 only: seq_n > 1 runs a whole chain in one launch — step k tracks frame
                                    //    fixed_ref + k*seq_step -> + seq_step from pose p_in + 6*T*k to p_out + 6*T*k
                                    //    (iters + T*L*k, npixres + T*k); 0/1: a single step
@@ -54,9 +54,6 @@ struct TrackParams {
   int64_t state_stride;            //    (floats per track: 3*64 + 12 per point of the largest track), null: reset every call
   int state_load;                  //    0: the first call after Set3Dpoints (arrays start zeroed, odometer.cpp:173)
   unsigned robust;                 // ICT_ROBUST_* flags (ictrack.h): opt-in deviations from the reference, fast mode / psz 8 (K2v8)
-  int knob_no_k2r;                 // tracker knob "no_k2r": reference-order psz 32 runs K2x even where K2r applies (A/B, tests)
-  int knob_seq_launches;           // tracker knob "seq_launches": a chain is one launch per frame step even where K2v8 could loop
-  int tma_ok;                      // every frame of the store carries tensor maps (FrameDesc.tmap)
   int r_pcap;                      // K2r: points per track the shared-memory layout is sized for (set by its launcher)
   int sum_mode;                    // 0: fixed-order tree reductions (fast); 1: Eigen-3.3 packet order (bit-exact
                                    //    with the oracle's default model of the reference, ~3x slower)
@@ -125,8 +122,9 @@ enum class TrackKernel { V8, V2, Fast, X8, R, X, General, MultiCta };
 TrackKernel select_track_kernel(const ict_optparam& op, int max_pts, int sum_mode, int eigen_packet, int force_general,
                                 int no_k2r, int tma_ok);
 size_t track_smem_bytes(const ict_optparam& op, int max_pts, int sum_mode);
-// Launches the selected kernel; cudaErrorInvalidConfiguration for MultiCta (the caller runs launch_track_big).
-cudaError_t launch_track(const TrackParams& prm, int max_pts, cudaStream_t stream);
+// Launches kernel k, which select_track_kernel chose for max_pts; cudaErrorInvalidConfiguration for MultiCta (the
+// caller runs launch_track_big) and for a chain (seq_n > 1) on any kernel but V8.
+cudaError_t launch_track(const TrackParams& prm, TrackKernel k, int max_pts, cudaStream_t stream);
 
 // Each kernel's own constraints: *_supported / *_smem_bytes.  The launchers assume select_track_kernel chose them.
 // K2v2 (ict_kernel_v2.cu): the production kernel for psz 32 without dopatchnorm, tree sums.
@@ -145,7 +143,7 @@ size_t kx_smem_bytes(const ict_optparam& op, int max_pts);
 cudaError_t launch_track_x(const TrackParams& prm, int max_pts, cudaStream_t stream);
 
 // K2r (ict_kernel_r.cu): reference-order sums for psz 32 without dopatchnorm, up to 8 points per track, with the
-// steepest-descent images resident in shared memory and the windows staged by 2-D TMA; needs prm.tma_ok.
+// steepest-descent images resident in shared memory and the windows staged by 2-D TMA; needs the tensor maps (tma_ok).
 bool kr_supported(const ict_optparam& op, int max_pts, int tma_ok);
 size_t kr_smem_bytes(const ict_optparam& op, int max_pts);
 cudaError_t launch_track_r(const TrackParams& prm, int max_pts, cudaStream_t stream);
