@@ -157,9 +157,11 @@ cudaError_t launch_track_x8(const TrackParams& prm, int max_pts, cudaStream_t st
 // SetPose only: setpose_se3 + reprojection at lv_l into prm.pt2d_out (one CTA per track)
 cudaError_t launch_reproject(const TrackParams& prm, cudaStream_t stream);
 
-// multi-CTA path for one big track (dense alignment: psz=1, millions of points)
-struct BigTrackWork;
-size_t bigtrack_work_bytes(const ict_optparam& op, int64_t npts, int eigen_packet);
+// multi-CTA path for one big track (dense alignment: psz=1, millions of points).  bigtrack_work_bytes: bytes of the
+// track's work buffer; with base != null also points *out into it.
+struct BigWork;
+size_t bigtrack_work_bytes(const ict_optparam& op, int64_t npts, int eigen_packet, void* base = nullptr,
+                           BigWork* out = nullptr);
 cudaError_t launch_track_big(const TrackParams& prm, int t, int64_t npts, void* work, cudaStream_t stream);
 
 // ict_track_evaluate (ict_evaluate.cu): one measurement per track at a chosen pose.  All pointers device memory; the

@@ -1,6 +1,5 @@
-// ict_kernels_big.cu — (1) the multi-CTA form of SetPose + TrackPose for ONE track that is too large for a CTA's
-// shared memory (dense full-frame alignment: psz = 1, one point per pixel, BASELINE config 4), and (2) the NCC
-// hypothesis scoring kernel.
+// ict_kernels_big.cu — the multi-CTA form of SetPose + TrackPose for ONE track that is too large for a CTA's shared
+// memory (dense full-frame alignment: psz = 1, one point per pixel, BASELINE config 4; more than 240 8x8 patches).
 //
 // Same arithmetic as k_track (ict_kernels.cu), including the optional reference-order sums (sum_mode 1: Hessian and
 // J^T r by one CTA running Eigen's eight sequential chains, sixteen with 8-float packets); the template (pat_ref, pat_dx, pat_dy) and the per-point state
@@ -11,10 +10,9 @@
 #include "ict_kernels.cuh"
 #include "ict_device.cuh"
 
+#include <type_traits>
 
 namespace ict {
-
-int64_t launch_count(int reset);
 
 struct BigState {
   float G[12];
@@ -39,8 +37,6 @@ struct BigWork {
   int ncta;
 };
 
-static inline size_t al(size_t x) { return (x + 255) & ~(size_t)255; }
-
 #define BIG_CHUNK 2048         /* chain elements per staged chunk (8 KB per chain, 64 KB per stage) of the reference-order
                                   chain kernel: every chunk costs ~150 cycles of hand-over on the critical path, so few and
                                   large ones (512 x 4 stages: 0.66 ms per pass of 247 k additions; 2048 x 2: 0.585 ms) */
@@ -48,6 +44,8 @@ static inline size_t al(size_t x) { return (x + 255) & ~(size_t)255; }
 // A stage holds 8 * BIG_CHUNK floats whatever the chain count: sixteen chains (8-float packets) take chunks of half the
 // length, and their chains are half as long, so the hand-overs per chain pass stay the same.
 __host__ __device__ constexpr int big_chunk(int nch) { return 8 * BIG_CHUNK / nch; }
+// row stride of a chain-kernel stage in shared memory: sixteen chains' rows get a 16-byte skew (see k_big_chains)
+__host__ __device__ constexpr int big_row_stride(int nch) { return nch == 8 ? big_chunk(nch) : big_chunk(nch) + 4; }
 // position of element j of chain c of product row q: chunk-major — the NCH chains' pieces of one chunk are contiguous
 // (64 KB), so that a stage of the chain kernel is one stretch of memory
 template <int NCH>
@@ -69,42 +67,37 @@ static int big_ncta(int64_t E) {
   return (int)c;
 }
 
-size_t bigtrack_work_bytes(const ict_optparam& op, int64_t npts, int eigen_packet) {
+size_t bigtrack_work_bytes(const ict_optparam& op, int64_t npts, int eigen_packet, void* base, BigWork* out) {
   const int64_t P = npts < op.maxpttrack ? npts : op.maxpttrack;
   const int64_t E = P * op.novals;
-  size_t b = al(sizeof(BigState));
-  b += 4 * al(sizeof(float) * E);
-  b += al(sizeof(float) * 10 * P) + al(sizeof(float) * 4 * P) + 4 * al(sizeof(float) * P);
-  b += 2 * al(sizeof(int) * P);
-  b += al(sizeof(float) * 21 * big_ncta(E));
   const int nch = eigen_packet == 8 ? 16 : 8;
-  b += al(sizeof(float) * nch * 24 * (size_t)big_cstride((int64_t)op.maxpttrack * op.novals, nch));   // 24 product rows: the 21 Hessian sums at once
-  return b;
-}
-
-static BigWork carve(const ict_optparam& op, int64_t npts, int eigen_packet, void* work) {
-  const int64_t P = npts < op.maxpttrack ? npts : op.maxpttrack;
-  const int64_t E = P * op.novals;
-  char* c = (char*)work;
-  BigWork w;
-  w.st = (BigState*)c; c += al(sizeof(BigState));
-  w.ref = (float*)c; c += al(sizeof(float) * E);
-  w.gx = (float*)c; c += al(sizeof(float) * E);
-  w.gy = (float*)c; c += al(sizeof(float) * E);
-  w.pnew = (float*)c; c += al(sizeof(float) * E);
-  w.coef = (float*)c; c += al(sizeof(float) * 10 * P);
-  w.w = (float*)c; c += al(sizeof(float) * 4 * P);
-  w.mean = (float*)c; c += al(sizeof(float) * P);
-  w.Xc = (float*)c; c += al(sizeof(float) * P);
-  w.Yc = (float*)c; c += al(sizeof(float) * P);
-  w.Zc = (float*)c; c += al(sizeof(float) * P);
-  w.base = (int*)c; c += al(sizeof(int) * P);
-  w.vis = (int*)c; c += al(sizeof(int) * P);
-  w.part = (float*)c; c += al(sizeof(float) * 21 * big_ncta(E));
-  w.prod = (float*)c;
-  w.cstride = big_cstride((int64_t)op.maxpttrack * op.novals, eigen_packet == 8 ? 16 : 8);
+  BigWork w = {};
   w.ncta = big_ncta(E);
-  return w;
+  w.cstride = big_cstride((int64_t)op.maxpttrack * op.novals, nch);
+  size_t off = 0;
+  auto take = [&](auto*& p, int64_t count) {   // 256-byte aligned regions, in this order
+    using T = std::remove_reference_t<decltype(*p)>;
+    off = (off + 255) & ~(size_t)255;
+    if (base) p = reinterpret_cast<T*>(static_cast<char*>(base) + off);
+    off += sizeof(T) * (size_t)count;
+  };
+  take(w.st, 1);
+  take(w.ref, E);
+  take(w.gx, E);
+  take(w.gy, E);
+  take(w.pnew, E);
+  take(w.coef, 10 * P);
+  take(w.w, 4 * P);
+  take(w.mean, P);
+  take(w.Xc, P);
+  take(w.Yc, P);
+  take(w.Zc, P);
+  take(w.base, P);
+  take(w.vis, P);
+  take(w.part, 21 * w.ncta);
+  take(w.prod, nch * 24 * w.cstride);   // 24 product rows: the 21 Hessian sums at once
+  if (out) *out = w;
+  return (off + 255) & ~(size_t)255;
 }
 
 struct BigArgs {
@@ -167,6 +160,103 @@ __device__ __forceinline__ void finish_partials(const float* part, int ncta, flo
   __syncthreads();
 }
 
+// ---- per-element work shared by the kernels below --------------------------------------------------------------------
+// a pyramid level's intrinsics and image bounds
+struct LevelCam {
+  float fx, fy, cx, cy, swo, sho;
+  int width;
+};
+__device__ __forceinline__ LevelCam level_cam(const CamLevels& cam, int sl) {
+  return {cam.fx[sl], cam.fy[sl], cam.cx[sl], cam.cy[sl], cam.swo[sl], cam.sho[sl], cam.width[sl]};
+}
+
+// camera-frame point (x, y, z) projected at level lc: false outside [0, swo] x [0, sho] (odometer.cpp:273-275,
+// 369-371), else true with q = the placement of its patch
+__device__ __forceinline__ bool project_place(const LevelCam& lc, int pszd2, float x, float y, float z, PatchPlace& q) {
+  const float mx = (x / z) * lc.fx + lc.cx;
+  const float my = (y / z) * lc.fy + lc.cy;
+  if (!((mx >= 0) & (my >= 0) & (mx <= lc.swo) & (my <= lc.sho))) return false;
+  q = patch_place(mx, my, pszd2, lc.width);
+  return true;
+}
+
+__device__ __forceinline__ float sample(const float* __restrict__ img, const PatchPlace& q, int width) {
+  return bilin4(img, q.base, width, q.w0, q.w1, q.w2, q.w3);
+}
+
+// point i's placement into the per-point arrays (base, w), and back moved to pixel slot e = (i, row r, column c)
+__device__ __forceinline__ void store_place(const BigArgs& a, long long i, const PatchPlace& q) {
+  a.w.base[i] = q.base;
+  a.w.w[i] = q.w0; a.w.w[a.P + i] = q.w1; a.w.w[2LL * a.P + i] = q.w2; a.w.w[3LL * a.P + i] = q.w3;
+}
+__device__ __forceinline__ PatchPlace slot_place(const BigArgs& a, long long e, long long i, int width) {
+  const int n = a.prm.op.novals, psz = a.prm.op.psz;
+  const int rem = (int)(e - i * n), r = rem / psz, c = rem - r * psz;
+  return {a.w.base[i] + r * width + c, a.w.w[i], a.w.w[a.P + i], a.w.w[2LL * a.P + i], a.w.w[3LL * a.P + i]};
+}
+
+// the six steepest-descent values of a slot of point i with gradient (gx, gy), from the point's coefficient rows
+// (sd_values' arithmetic)
+__device__ __forceinline__ void slot_sd(const BigArgs& a, long long i, float gx, float gy, float* sd) {
+  const float* cf = a.w.coef;
+  sd[0] = gx * cf[0 * (long long)a.P + i];
+  sd[1] = gy * cf[1 * (long long)a.P + i];
+  sd[2] = gx * cf[2 * (long long)a.P + i] + gy * cf[3 * (long long)a.P + i];
+  sd[3] = gx * cf[4 * (long long)a.P + i] + gy * cf[5 * (long long)a.P + i];
+  sd[4] = gx * cf[6 * (long long)a.P + i] + gy * cf[7 * (long long)a.P + i];
+  sd[5] = gx * cf[8 * (long long)a.P + i] + gy * cf[9 * (long long)a.P + i];
+}
+
+// acc[k] += sd_p * sd_q for the 21 pairs p <= q in ComputeHessian's order
+__device__ __forceinline__ void add_hessian(float* acc, const float* sd) {
+  int k = 0;
+#pragma unroll
+  for (int p = 0; p < 6; ++p)
+#pragma unroll
+    for (int q = p; q < 6; ++q) { acc[k] = acc[k] + sd[p] * sd[q]; ++k; }
+}
+
+// ---- the start of a level and the serial tail of a non-fused iteration -----------------------------------------------
+// Called by one warp once the level's 21 Hessian sums are in s_H: factors H, resets the level's state and records 0
+// iterations for it (a level the stop rule does not enter keeps that count).
+__device__ __forceinline__ void big_level_start(const BigArgs& a, int sl, const float* s_H) {
+  BigState* S = a.w.st;
+  lu6_factor_warp(s_H, S->lu);
+  if (threadIdx.x == 0) {
+    const ict_optparam& op = a.prm.op;
+    S->normdp_init = 1e-10f;
+    S->normdp = 1e-10f;
+    S->it = 0;
+    S->nvis = 0;
+    S->cont = keep_iterating(op, 0, 1e-10f, 1e-10f);
+    store_level_iters(a.prm.iters, op, a.t, sl, 0);
+  }
+}
+
+// Solve, pose update, trace record, pixel-residual count, the level's iteration count and the stop rule of one
+// iteration of the non-fused paths (one thread); sum6 = the six sums of J^T r.  The same steps as the fused dense
+// path's tail in dense_iter_finish, which keeps its own copy: there the state comes from a shared-memory snapshot and
+// teacher forcing applies.
+__device__ __forceinline__ void big_iter_finish_serial(const BigArgs& a, int sl, const float* sum6) {
+  BigState* S = a.w.st;
+  const ict_optparam& op = a.prm.op;
+  float sumsd[6], dp[6];
+  for (int k = 0; k < 6; ++k) sumsd[k] = sum6[k];
+  lu6_solve_exact(S->lu, sumsd, dp);   // == lu6_solve, straight-line
+  for (int k = 0; k < 6; ++k) S->p[k] += dp[k];
+  se3_exp<float>(S->G, S->p);
+  const float normdp = normdp_l1(dp);
+  if (S->it == 0) S->normdp_init = normdp;
+  S->normdp = normdp;
+  if (a.prm.trace && S->trace_n < a.prm.trace_cap)
+    trace_record(track_trace(a.prm, a.t) + (int64_t)ICT_TRACE_FLOATS * S->trace_n++, sl, S->it, sumsd, dp, normdp, S->nvis);
+  S->npix += (long long)S->nvis * op.novals;
+  S->nvis = 0;
+  S->it += 1;
+  store_level_iters(a.prm.iters, op, a.t, sl, S->it);
+  S->cont = keep_iterating(op, S->it, S->normdp, S->normdp_init);
+}
+
 __global__ void k_big_init(const BigArgs a, int fused) {
   // ResetOdometer for the element/point state + setpose_se3.  The fused dense path keeps (ref, sd1..6) only.
   const long long gid = blockIdx.x * (long long)blockDim.x + threadIdx.x, gsz = (long long)gridDim.x * blockDim.x;
@@ -202,43 +292,35 @@ __global__ void k_big_project_ref(const BigArgs a) {
 }
 
 __global__ void k_big_level_points(const BigArgs a, int sl) {
-  const CamLevels& cam = a.prm.cam;
-  const float fx = cam.fx[sl], fy = cam.fy[sl], cx = cam.cx[sl], cy = cam.cy[sl], swo = cam.swo[sl], sho = cam.sho[sl];
-  const int width = cam.width[sl];
+  const LevelCam lc = level_cam(a.prm.cam, sl);
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < a.P; i += (long long)gridDim.x * blockDim.x) {
     const float xc = a.w.Xc[i], yc = a.w.Yc[i], zc = a.w.Zc[i];
-    const float mx = (xc / zc) * fx + cx;
-    const float my = (yc / zc) * fy + cy;
-    const bool out = !((mx >= 0) & (my >= 0) & (mx <= swo) & (my <= sho));
-    if (out) {
+    PatchPlace q;
+    if (!project_place(lc, a.prm.op.pszd2, xc, yc, zc, q)) {
       a.w.vis[i] = 0;
     } else {
       a.w.vis[i] = 1;
-      const PatchPlace q = patch_place(mx, my, a.prm.op.pszd2, width);
-      a.w.base[i] = q.base;
-      a.w.w[i] = q.w0; a.w.w[a.P + i] = q.w1; a.w.w[2LL * a.P + i] = q.w2; a.w.w[3LL * a.P + i] = q.w3;
+      store_place(a, i, q);
       float c[10];
-      sd_coefs(xc, yc, zc, fx, fy, c);
+      sd_coefs(xc, yc, zc, lc.fx, lc.fy, c);
       for (int k = 0; k < 10; ++k) a.w.coef[(long long)k * a.P + i] = c[k];
     }
   }
 }
 
 __global__ void __launch_bounds__(256) k_big_level_gather(const BigArgs a, int sl) {
-  const int n = a.prm.op.novals, psz = a.prm.op.psz, width = a.prm.cam.width[sl];
+  const int n = a.prm.op.novals, width = a.prm.cam.width[sl];
   const int rf = a.prm.fixed_ref;
   const float* __restrict__ Iref = a.prm.frames[rf].I[sl];
   const float* __restrict__ Dxr = a.prm.frames[rf].dx[sl];
   const float* __restrict__ Dyr = a.prm.frames[rf].dy[sl];
   for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < a.E; e += (long long)gridDim.x * blockDim.x) {
     const long long i = e / n;
-    const int rem = (int)(e - i * n), r = rem / psz, c = rem - r * psz;
     if (a.w.vis[i] & 1) {
-      const int addr = a.w.base[i] + r * width + c;
-      const float w0 = a.w.w[i], w1 = a.w.w[a.P + i], w2 = a.w.w[2LL * a.P + i], w3 = a.w.w[3LL * a.P + i];
-      a.w.ref[e] = bilin4(Iref, addr, width, w0, w1, w2, w3);
-      a.w.gx[e] = bilin4(Dxr, addr, width, w0, w1, w2, w3);
-      a.w.gy[e] = bilin4(Dyr, addr, width, w0, w1, w2, w3);
+      const PatchPlace q = slot_place(a, e, i, width);
+      a.w.ref[e] = sample(Iref, q, width);
+      a.w.gx[e] = sample(Dxr, q, width);
+      a.w.gy[e] = sample(Dyr, q, width);
     }
   }
 }
@@ -275,16 +357,9 @@ __global__ void __launch_bounds__(256) k_big_level_hessian(const BigArgs a) {
 #pragma unroll
   for (int k = 0; k < 21; ++k) acc[k] = 0.0f;
   for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < a.E; e += (long long)gridDim.x * blockDim.x) {
-    const long long i = e / n;
-    float cf[10], sd[6];
-#pragma unroll
-    for (int k = 0; k < 10; ++k) cf[k] = a.w.coef[(long long)k * a.P + i];
-    sd_values(a.w.gx[e], a.w.gy[e], cf, sd);
-    int k = 0;
-#pragma unroll
-    for (int p = 0; p < 6; ++p)
-#pragma unroll
-      for (int q = p; q < 6; ++q) { acc[k] = acc[k] + sd[p] * sd[q]; ++k; }
+    float sd[6];
+    slot_sd(a, e / n, a.w.gx[e], a.w.gy[e], sd);
+    add_hessian(acc, sd);
   }
   cta_partials<21>(acc, a.w.part);
 }
@@ -296,41 +371,25 @@ __global__ void __launch_bounds__(256) k_big_level_finish(const BigArgs a, int s
   asm volatile("griddepcontrol.wait;" ::: "memory");
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
   finish_partials<21>(a.w.part, a.w.ncta, s_H);
-  if (threadIdx.x < 32) lu6_factor_warp(s_H, a.w.st->lu);
-  if (threadIdx.x == 0) {
-    BigState* S = a.w.st;
-    const ict_optparam& op = a.prm.op;
-    S->normdp_init = 1e-10f;
-    S->normdp = 1e-10f;
-    S->it = 0;
-    S->nvis = 0;
-    S->cont = keep_iterating(op, 0, 1e-10f, 1e-10f);
-    store_level_iters(a.prm.iters, op, a.t, sl, 0);
-  }
+  if (threadIdx.x < 32) big_level_start(a, sl, s_H);
 }
 
 __global__ void k_big_iter_points(const BigArgs a, int sl) {
   BigState* S = a.w.st;
   if (!S->cont) return;
-  const CamLevels& cam = a.prm.cam;
-  const float fx = cam.fx[sl], fy = cam.fy[sl], cx = cam.cx[sl], cy = cam.cy[sl], swo = cam.swo[sl], sho = cam.sho[sl];
-  const int width = cam.width[sl];
+  const LevelCam lc = level_cam(a.prm.cam, sl);
   const int64_t off = a.prm.pt_off[a.t];
   const float* q = a.prm.pt3d + 3 * off;
   int cnt = 0;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < a.P; i += (long long)gridDim.x * blockDim.x) {
     float tx, ty, tz;
     rigid_apply<float>(S->G, q[i], q[a.n_in + i], q[2 * (int64_t)a.n_in + i], tx, ty, tz);
-    const float mx = (tx / tz) * fx + cx;
-    const float my = (ty / tz) * fy + cy;
-    const bool out = !((mx >= 0) & (my >= 0) & (mx <= swo) & (my <= sho));
-    if (out) {
+    PatchPlace pp;
+    if (!project_place(lc, a.prm.op.pszd2, tx, ty, tz, pp)) {
       a.w.vis[i] &= ~2;
     } else {
       a.w.vis[i] |= 2;
-      const PatchPlace pp = patch_place(mx, my, a.prm.op.pszd2, width);
-      a.w.base[i] = pp.base;
-      a.w.w[i] = pp.w0; a.w.w[a.P + i] = pp.w1; a.w.w[2LL * a.P + i] = pp.w2; a.w.w[3LL * a.P + i] = pp.w3;
+      store_place(a, i, pp);
       ++cnt;
     }
   }
@@ -341,21 +400,18 @@ __global__ void k_big_iter_points(const BigArgs a, int sl) {
 
 __global__ void __launch_bounds__(256) k_big_iter_sample(const BigArgs a, int sl) {
   if (!a.w.st->cont) return;
-  const int n = a.prm.op.novals, psz = a.prm.op.psz, width = a.prm.cam.width[sl];
+  const int n = a.prm.op.novals, width = a.prm.cam.width[sl];
   const float* __restrict__ Inew = a.prm.frames[a.prm.fixed_new].I[sl];
   for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < a.E; e += (long long)gridDim.x * blockDim.x) {
     const long long i = e / n;
-    const int rem = (int)(e - i * n), r = rem / psz, c = rem - r * psz;
-    if (a.w.vis[i] & 2)
-      a.w.pnew[e] = bilin4(Inew, a.w.base[i] + r * width + c, width, a.w.w[i], a.w.w[a.P + i], a.w.w[2LL * a.P + i],
-                           a.w.w[3LL * a.P + i]);
+    if (a.w.vis[i] & 2) a.w.pnew[e] = sample(Inew, slot_place(a, e, i, width), width);
   }
 }
 
 template <bool PN>
 __global__ void __launch_bounds__(256) k_big_iter_elems(const BigArgs a, int sl) {
   if (!a.w.st->cont) return;
-  const int n = a.prm.op.novals, psz = a.prm.op.psz, width = a.prm.cam.width[sl];
+  const int n = a.prm.op.novals, width = a.prm.cam.width[sl];
   const float* __restrict__ Inew = a.prm.frames[a.prm.fixed_new].I[sl];
   float acc[6];
 #pragma unroll
@@ -364,13 +420,8 @@ __global__ void __launch_bounds__(256) k_big_iter_elems(const BigArgs a, int sl)
     const long long i = e / n;
     if (a.w.vis[i] & 2) {
       float pn;
-      if (PN) {
-        pn = a.w.pnew[e];   // mean already subtracted by k_big_patch_means
-      } else {
-        const int rem = (int)(e - i * n), r = rem / psz, c = rem - r * psz;
-        pn = bilin4(Inew, a.w.base[i] + r * width + c, width, a.w.w[i], a.w.w[a.P + i], a.w.w[2LL * a.P + i],
-                    a.w.w[3LL * a.P + i]);
-      }
+      if (PN) pn = a.w.pnew[e];   // mean already subtracted by k_big_patch_means
+      else pn = sample(Inew, slot_place(a, e, i, width), width);
       const float pd = a.w.ref[e] - pn;
       float cf[10], sd[6];
 #pragma unroll
@@ -381,26 +432,6 @@ __global__ void __launch_bounds__(256) k_big_iter_elems(const BigArgs a, int sl)
     }
   }
   cta_partials<6>(acc, a.w.part);
-}
-
-// solve, pose update, stop rule and trace record of one iteration (one thread); sum6 = the six sums of J^T r
-__device__ __forceinline__ void big_iter_finish_serial(const BigArgs& a, int sl, const float* sum6) {
-  BigState* S = a.w.st;
-  const ict_optparam& op = a.prm.op;
-  float sumsd[6], dp[6];
-  for (int k = 0; k < 6; ++k) sumsd[k] = sum6[k];
-  lu6_solve(S->lu, sumsd, dp);
-  for (int k = 0; k < 6; ++k) S->p[k] += dp[k];
-  se3_exp<float>(S->G, S->p);
-  const float normdp = normdp_l1(dp);
-  if (S->it == 0) S->normdp_init = normdp;
-  S->normdp = normdp;
-  if (a.prm.trace && S->trace_n < a.prm.trace_cap)
-    trace_record(track_trace(a.prm, a.t) + (int64_t)ICT_TRACE_FLOATS * S->trace_n++, sl, S->it, sumsd, dp, normdp, S->nvis);
-  S->npix += (long long)S->nvis * op.novals;
-  S->nvis = 0;
-  S->it += 1;
-  S->cont = keep_iterating(op, S->it, S->normdp, S->normdp_init);
 }
 
 __global__ void __launch_bounds__(256) k_big_iter_finish(const BigArgs a, int sl, int ncta) {
@@ -437,22 +468,14 @@ __global__ void __launch_bounds__(256) k_big_products(const BigArgs a, int pass)
   const int n = a.prm.op.novals;
   const long long lim = a.E;                       // elements beyond E are zeros the reference adds nothing for
   const long long nj = (lim + NCH - 1) / NCH;
-  const float* cf = a.w.coef;
   for (long long j = blockIdx.x * (long long)blockDim.x + threadIdx.x; j < nj; j += (long long)gridDim.x * blockDim.x) {
 #pragma unroll
     for (int c = 0; c < NCH; ++c) {
       const long long e = NCH * j + c;
       float v[6];
       if (e < lim) {
-        const long long i = n == 1 ? e : e / n;
-        const float gx = a.w.gx[e], gy = a.w.gy[e];
         float sd[6];
-        sd[0] = gx * cf[0 * (long long)a.P + i];
-        sd[1] = gy * cf[1 * (long long)a.P + i];
-        sd[2] = gx * cf[2 * (long long)a.P + i] + gy * cf[3 * (long long)a.P + i];
-        sd[3] = gx * cf[4 * (long long)a.P + i] + gy * cf[5 * (long long)a.P + i];
-        sd[4] = gx * cf[6 * (long long)a.P + i] + gy * cf[7 * (long long)a.P + i];
-        sd[5] = gx * cf[8 * (long long)a.P + i] + gy * cf[9 * (long long)a.P + i];
+        slot_sd(a, n == 1 ? e : e / n, a.w.gx[e], a.w.gy[e], sd);
         if (MODE == 0) {
           const float pd = a.w.pnew[e];
 #pragma unroll
@@ -486,9 +509,8 @@ template <int NCH>
 __global__ void __launch_bounds__(256) k_big_iter_fused_exact(const BigArgs a, int sl) {
   BigState* S = a.w.st;
   if (!S->cont) return;
-  const CamLevels& cam = a.prm.cam;
-  const float fx = cam.fx[sl], fy = cam.fy[sl], cx = cam.cx[sl], cy = cam.cy[sl], swo = cam.swo[sl], sho = cam.sho[sl];
-  const int width = cam.width[sl], n = a.prm.op.novals, psz = a.prm.op.psz, pszd2 = a.prm.op.pszd2;
+  const LevelCam lc = level_cam(a.prm.cam, sl);
+  const int width = lc.width, n = a.prm.op.novals, psz = a.prm.op.psz, pszd2 = a.prm.op.pszd2;
   const float* __restrict__ Inew = a.prm.frames[a.prm.fixed_new].I[sl];
   const float* q3 = a.prm.pt3d + 3 * a.prm.pt_off[a.t];
   const long long lim = a.E;
@@ -508,14 +530,10 @@ __global__ void __launch_bounds__(256) k_big_iter_fused_exact(const BigArgs a, i
         const float X = q3[i], Y = q3[a.n_in + i], Z = q3[2 * (int64_t)a.n_in + i];
         float tx, ty, tz;
         rigid_apply(G, X, Y, Z, tx, ty, tz);
-        const float mx = (tx / tz) * fx + cx;
-        const float my = (ty / tz) * fy + cy;
-        const bool vis = (mx >= 0) & (my >= 0) & (mx <= swo) & (my <= sho);
+        PatchPlace pp;
         float pd = 0.0f;
-        if (vis) {
-          const PatchPlace pp = patch_place(mx, my, pszd2, width);
-          const float pn = bilin4(Inew, pp.base + r * width + cc, width, pp.w0, pp.w1, pp.w2, pp.w3);
-          pd = a.w.ref[e] - pn;
+        if (project_place(lc, pszd2, tx, ty, tz, pp)) {
+          pd = a.w.ref[e] - bilin4(Inew, pp.base + r * width + cc, width, pp.w0, pp.w1, pp.w2, pp.w3);
           if (rem == 0) ++cnt;
         }
         const float gx = a.w.gx[e], gy = a.w.gy[e];
@@ -544,7 +562,7 @@ template <int NCH>
 __global__ void __launch_bounds__(64) k_big_chains(const BigArgs a, int nq, float* out, int iteration) {
   if (iteration && !a.w.st->cont) return;
   constexpr int CH = big_chunk(NCH);                     // chain elements per stage
-  constexpr int RS = NCH == 8 ? CH : CH + 4;             // row stride of a stage in shared memory
+  constexpr int RS = big_row_stride(NCH);                // row stride of a stage in shared memory
   extern __shared__ __align__(128) float s_ring[];     // [BIG_STAGES][NCH][RS]
   __shared__ unsigned long long s_full[BIG_STAGES], s_free[BIG_STAGES];
   __shared__ float s_ch[NCH];
@@ -621,44 +639,24 @@ __global__ void __launch_bounds__(64) k_big_chains(const BigArgs a, int nq, floa
   }
 }
 
-// factorisation + state of a level after the 21 reference-order Hessian sums (part[0..20]) are in
-__global__ void __launch_bounds__(32) k_big_hessian_exact_finish(const BigArgs a) {
+// the level start after the 21 reference-order Hessian sums (part[0..20]) are in
+__global__ void __launch_bounds__(32) k_big_hessian_exact_finish(const BigArgs a, int sl) {
   __shared__ float s_H[21];
-  const int tid = threadIdx.x;
-  if (tid < 21) s_H[tid] = a.w.part[tid];
+  if (threadIdx.x < 21) s_H[threadIdx.x] = a.w.part[threadIdx.x];
   __syncwarp();
-  lu6_factor_warp(s_H, a.w.st->lu);
-  if (tid == 0) {
-    BigState* S = a.w.st;
-    const ict_optparam& op = a.prm.op;
-    S->normdp_init = 1e-10f;
-    S->normdp = 1e-10f;
-    S->it = 0;
-    S->nvis = 0;
-    S->cont = keep_iterating(op, 0, 1e-10f, 1e-10f);
-  }
+  big_level_start(a, sl, s_H);
 }
 
 // pdiff of every slot into w.pnew (0 where the point is not visible in the new frame)
 template <bool PN>
 __global__ void __launch_bounds__(256) k_big_iter_pdiff(const BigArgs a, int sl) {
   if (!a.w.st->cont) return;
-  const int n = a.prm.op.novals, psz = a.prm.op.psz, width = a.prm.cam.width[sl];
+  const int n = a.prm.op.novals, width = a.prm.cam.width[sl];
   const float* __restrict__ Inew = a.prm.frames[a.prm.fixed_new].I[sl];
   for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < a.E; e += (long long)gridDim.x * blockDim.x) {
     const long long i = e / n;
     float pd = 0.0f;
-    if (a.w.vis[i] & 2) {
-      float pn;
-      if (PN) {
-        pn = a.w.pnew[e];
-      } else {
-        const int rem = (int)(e - i * n), r = rem / psz, c = rem - r * psz;
-        pn = bilin4(Inew, a.w.base[i] + r * width + c, width, a.w.w[i], a.w.w[a.P + i], a.w.w[2LL * a.P + i],
-                    a.w.w[3LL * a.P + i]);
-      }
-      pd = a.w.ref[e] - pn;
-    }
+    if (a.w.vis[i] & 2) pd = a.w.ref[e] - (PN ? a.w.pnew[e] : sample(Inew, slot_place(a, e, i, width), width));
     a.w.pnew[e] = pd;
   }
 }
@@ -675,9 +673,7 @@ __global__ void __launch_bounds__(256) k_big_iter_pdiff(const BigArgs a, int sl)
 // as k_big_iter_points/elems/finish: results are bit-identical to that path (tests/test_gpu_parity.py).
 // ==================================================================================================
 __global__ void __launch_bounds__(256, 4) k_dense_level(const BigArgs a, int sl) {   // 592 CTAs = one resident wave
-  const CamLevels& cam = a.prm.cam;
-  const float fx = cam.fx[sl], fy = cam.fy[sl], cx = cam.cx[sl], cy = cam.cy[sl], swo = cam.swo[sl], sho = cam.sho[sl];
-  const int width = cam.width[sl];
+  const LevelCam lc = level_cam(a.prm.cam, sl);
   const int rf = a.prm.fixed_ref;
   const float* __restrict__ Iref = a.prm.frames[rf].I[sl];
   const float* __restrict__ Dxr = a.prm.frames[rf].dx[sl];
@@ -691,17 +687,14 @@ __global__ void __launch_bounds__(256, 4) k_dense_level(const BigArgs a, int sl)
   for (int k = 0; k < 21; ++k) acc[k] = 0.0f;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < P; i += (long long)gridDim.x * blockDim.x) {
     const float xc = a.w.Xc[i], yc = a.w.Yc[i], zc = a.w.Zc[i];
-    const float mx = (xc / zc) * fx + cx;
-    const float my = (yc / zc) * fy + cy;
-    const bool out = !((mx >= 0) & (my >= 0) & (mx <= swo) & (my <= sho));   // odometer.cpp:273-275
     float sd[6];
-    if (!out) {
-      const PatchPlace q = patch_place(mx, my, a.prm.op.pszd2, width);      // util_getPatch_grad, one pixel
-      a.w.ref[i] = bilin4(Iref, q.base, width, q.w0, q.w1, q.w2, q.w3);
-      const float gx = bilin4(Dxr, q.base, width, q.w0, q.w1, q.w2, q.w3);
-      const float gy = bilin4(Dyr, q.base, width, q.w0, q.w1, q.w2, q.w3);
+    PatchPlace q;
+    if (project_place(lc, a.prm.op.pszd2, xc, yc, zc, q)) {               // util_getPatch_grad, one pixel
+      a.w.ref[i] = sample(Iref, q, lc.width);
+      const float gx = sample(Dxr, q, lc.width);
+      const float gy = sample(Dyr, q, lc.width);
       float c[10];
-      sd_coefs(xc, yc, zc, fx, fy, c);
+      sd_coefs(xc, yc, zc, lc.fx, lc.fy, c);
       sd_values(gx, gy, c, sd);                                              // odometer.cpp:317-326
 #pragma unroll
       for (int k = 0; k < 6; ++k) sdp[k * P + i] = sd[k];
@@ -709,13 +702,19 @@ __global__ void __launch_bounds__(256, 4) k_dense_level(const BigArgs a, int sl)
 #pragma unroll
       for (int k = 0; k < 6; ++k) sd[k] = sdp[k * P + i];
     }
-    int k = 0;
-#pragma unroll
-    for (int p = 0; p < 6; ++p)
-#pragma unroll
-      for (int q = p; q < 6; ++q) { acc[k] = acc[k] + sd[p] * sd[q]; ++k; }
+    add_hessian(acc, sd);
   }
   cta_partials<21>(acc, a.w.part);
+}
+
+// the new image at the projection of reference point (X, Y, Z) under pose G, one pixel; vis: inside the level
+__device__ __forceinline__ float dense_sample(const LevelCam& lc, int pszd2, const float* G, const float* __restrict__ Inew,
+                                              float X, float Y, float Z, bool& vis) {
+  float tx, ty, tz;
+  rigid_apply(G, X, Y, Z, tx, ty, tz);                                         // project_pt, pose.cpp:307-397
+  PatchPlace pp;
+  vis = project_place(lc, pszd2, tx, ty, tz, pp);
+  return vis ? sample(Inew, pp, lc.width) : 0.0f;
 }
 
 // Shared tail of the dense iteration kernels: CTA partial sums, visible-point count, ticket; the CTA that arrives last
@@ -820,9 +819,7 @@ __global__ void __launch_bounds__(256, 4) k_dense_iter(const BigArgs a, int sl) 
   float G[12];
 #pragma unroll
   for (int k = 0; k < 12; ++k) G[k] = s_G[k];
-  const CamLevels& cam = a.prm.cam;
-  const float fx = cam.fx[sl], fy = cam.fy[sl], cx = cam.cx[sl], cy = cam.cy[sl], swo = cam.swo[sl], sho = cam.sho[sl];
-  const int width = cam.width[sl];
+  const LevelCam lc = level_cam(a.prm.cam, sl);
   const float* __restrict__ Inew = a.prm.frames[a.prm.fixed_new].I[sl];
   const int64_t off = a.prm.pt_off[a.t];
   const float* __restrict__ q = a.prm.pt3d + 3 * off;
@@ -835,16 +832,6 @@ __global__ void __launch_bounds__(256, 4) k_dense_iter(const BigArgs a, int sl) 
   // Two points per trip: both points' streams (X, Y, Z, ref, sd1..6) and then both gathers are in flight together;
   // the additions stay in point order, so the sums are those of the one-point loop.
   const long long stride = (long long)gridDim.x * blockDim.x;
-  auto sample = [&](long long i, float X, float Y, float Z, bool& vis) -> float {
-    float tx, ty, tz;
-    rigid_apply(G, X, Y, Z, tx, ty, tz);                                         // project_pt, pose.cpp:307-397
-    const float mx = (tx / tz) * fx + cx;
-    const float my = (ty / tz) * fy + cy;
-    vis = (mx >= 0) & (my >= 0) & (mx <= swo) & (my <= sho);                   // odometer.cpp:369-371
-    if (!vis) return 0.0f;
-    const PatchPlace pp = patch_place(mx, my, a.prm.op.pszd2, width);
-    return bilin4(Inew, pp.base, width, pp.w0, pp.w1, pp.w2, pp.w3);
-  };
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < P; i += 2 * stride) {
     const long long j = i + stride;
     const bool hj = j < P;
@@ -855,8 +842,8 @@ __global__ void __launch_bounds__(256, 4) k_dense_iter(const BigArgs a, int sl) 
 #pragma unroll
     for (int k = 0; k < 6; ++k) { s0[k] = sdp[k * P + i]; s1[k] = hj ? sdp[k * P + j] : 0.0f; }
     bool v0, v1 = false;
-    const float pn0 = sample(i, X0, Y0, Z0, v0);
-    const float pn1 = hj ? sample(j, X1, Y1, Z1, v1) : 0.0f;
+    const float pn0 = dense_sample(lc, a.prm.op.pszd2, G, Inew, X0, Y0, Z0, v0);
+    const float pn1 = hj ? dense_sample(lc, a.prm.op.pszd2, G, Inew, X1, Y1, Z1, v1) : 0.0f;
     if (v0) {
       const float pd = r0 - pn0;                                               // pdiff, odometer.cpp:381
 #pragma unroll
@@ -924,34 +911,20 @@ __global__ void __launch_bounds__(256, 4) k_dense_iter_tma(const BigArgs a, int 
   float G[12];
 #pragma unroll
   for (int k = 0; k < 12; ++k) G[k] = s_S.G[k];
-  const CamLevels& cam = a.prm.cam;
-  const float fx = cam.fx[sl], fy = cam.fy[sl], cx = cam.cx[sl], cy = cam.cy[sl], swo = cam.swo[sl], sho = cam.sho[sl];
-  const int width = cam.width[sl];
+  const LevelCam lc = level_cam(a.prm.cam, sl);
   const float* __restrict__ Inew = a.prm.frames[a.prm.fixed_new].I[sl];
   float acc[6];
 #pragma unroll
   for (int k = 0; k < 6; ++k) acc[k] = 0.0f;
   int cnt = 0;
-  // one point of a staged tile: projection, placement, the four-texel gather (returns the sample, sets vis).
   // (Tried: placing tile n+1 and issuing its gather before folding tile n — 23.1 instead of 21.3 us per iteration.)
-  auto sample = [&](int st, bool& vis) -> float {
-    const float X = s_buf[st][0][tid], Y = s_buf[st][1][tid], Z = s_buf[st][2][tid];
-    float tx, ty, tz;
-    rigid_apply(G, X, Y, Z, tx, ty, tz);                                         // project_pt, pose.cpp:307-397
-    const float mx = (tx / tz) * fx + cx;
-    const float my = (ty / tz) * fy + cy;
-    vis = (mx >= 0) & (my >= 0) & (mx <= swo) & (my <= sho);                   // odometer.cpp:369-371
-    if (!vis) return 0.0f;
-    const PatchPlace pp = patch_place(mx, my, a.prm.op.pszd2, width);
-    return bilin4(Inew, pp.base, width, pp.w0, pp.w1, pp.w2, pp.w3);
-  };
   for (int n = 0; n < nmine; ++n) {
     const int st = n % NST;
     const long long i = ((long long)blockIdx.x + (long long)n * gridDim.x) * 256 + tid;
     mbar_wait(&s_full[st], (n / NST) & 1);
     bool vis = false;
     float pn = 0.0f;
-    if (i < P) pn = sample(st, vis);
+    if (i < P) pn = dense_sample(lc, a.prm.op.pszd2, G, Inew, s_buf[st][0][tid], s_buf[st][1][tid], s_buf[st][2][tid], vis);
     if (vis) {
       const float pd = s_buf[st][3][tid] - pn;                                 // pdiff, odometer.cpp:381
 #pragma unroll
@@ -964,277 +937,117 @@ __global__ void __launch_bounds__(256, 4) k_dense_iter_tma(const BigArgs a, int 
   dense_iter_finish(a, sl, acc, cnt, &s_S);
 }
 
-__global__ void k_big_level_end(const BigArgs a, int sl) {
-  store_level_iters(a.prm.iters, a.prm.op, a.t, sl, a.w.st->it);
-}
-
 __global__ void k_big_final(const BigArgs a) {
   const BigState* S = a.w.st;
   finish_track(a.prm, a.t, a.prm.op.donorm != 0, S->p, S->G, a.prm.p_out, a.prm.npixres, S->npix,
                track_trace(a.prm, a.t), S->trace_n);
 }
 
-cudaError_t launch_track_big(const TrackParams& prm, int t, int64_t npts, void* work, cudaStream_t st) {
-  BigArgs a;
-  a.prm = prm;
-  a.w = carve(prm.op, npts, prm.eigen_packet, work);
-  a.t = t;
-  a.n_in = (int)npts;
-  a.P = (int)(npts < prm.op.maxpttrack ? npts : prm.op.maxpttrack);
-  a.E = (long long)a.P * prm.op.novals;
+// One counted launch of a kernel of this file.  pdl: programmatic stream serialization — the kernel may become resident
+// while its predecessor drains, so it has to start with griddepcontrol.wait.
+template <typename... KArgs, typename... Args>
+static void big_launch(void (*k)(KArgs...), int grid, int threads, size_t smem, bool pdl, cudaStream_t st,
+                       Args&&... args) {
+  cudaLaunchAttribute attr;
+  attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr.val.programmaticStreamSerializationAllowed = 1;
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(grid);
+  cfg.blockDim = dim3(threads);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = st;
+  cfg.attrs = &attr;
+  cfg.numAttrs = pdl ? 1 : 0;
+  cudaLaunchKernelEx(&cfg, k, std::forward<Args>(args)...);
+  count_launch();
+}
+
+// NCH: chains per reference-order sum (8 for 4-float packets, 16 for 8-float packets)
+template <int NCH>
+static cudaError_t track_big(const BigArgs& a, cudaStream_t st) {
+  const TrackParams& prm = a.prm;
   const ict_optparam& op = prm.op;
   const int ncta = a.w.ncta;
   const int pcta_ = (int)((a.P + 255) / 256 < 148 * 8 ? (a.P + 255) / 256 : 148 * 8);
   const int pcta = pcta_ > 0 ? pcta_ : 1;   // an empty track still runs the launch chain (its sums are empty, its pose unchanged)
   const bool pn = op.dopatchnorm != 0;
   const bool ex = prm.sum_mode != 0;   // reference-order sums
-  const bool pk8 = ex && prm.eigen_packet == 8;   // ... with 8-float packets: sixteen chains per sum
   const bool fused = !pn && !ex && !prm.force_general && op.novals == 1;
-  int nl = 0;
-  const size_t chain_smem = pk8 ? sizeof(float) * BIG_STAGES * 16 * (big_chunk(16) + 4)    // 128.5 KB
-                                : sizeof(float) * BIG_STAGES * 8 * BIG_CHUNK;                  // 128 KB
+  const int mean_order = ex ? prm.eigen_packet : 0;
+  constexpr size_t chain_smem = sizeof(float) * BIG_STAGES * NCH * big_row_stride(NCH);   // 128 KB; 128.5 KB for NCH 16
   if (ex) {
-    const cudaError_t e = pk8 ? set_kernel_attrs<k_big_chains<16>>((int)chain_smem, -1)
-                              : set_kernel_attrs<k_big_chains<8>>((int)chain_smem, -1);
+    const cudaError_t e = set_kernel_attrs<k_big_chains<NCH>>((int)chain_smem, -1);
     if (e != cudaSuccess) return e;
   }
-  k_big_init<<<ncta, 256, 0, st>>>(a, fused ? 1 : 0); ++nl;
-  k_big_project_ref<<<pcta, 256, 0, st>>>(a); ++nl;
-  for (int sl = op.lv_f; sl >= op.lv_l && fused; --sl) {   // dense path: one launch per level + one per iteration
-    // bulk-copy staging needs 16-byte aligned streams: point counts and the track's offset multiples of four
-    const bool tma = t == 0 && (a.P % 4 == 0) && (a.n_in % 4 == 0);   // t == 0: offset 0
-    // programmatic dependent launch: iteration k+1 becomes resident while the last CTA of iteration k still runs the
-    // solve, and its first tiles are in flight by the time the pose is published
-    cudaLaunchConfig_t cfg = {};
-    cudaLaunchAttribute lattr[1];
-    lattr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    lattr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.gridDim = dim3(ncta);
-    cfg.blockDim = dim3(256);
-    cfg.stream = st;
-    cfg.attrs = lattr;
-    cfg.numAttrs = 1;
-    cudaLaunchKernelEx(&cfg, k_dense_level, a, sl); ++nl;
-    cfg.gridDim = dim3(1);
-    cudaLaunchKernelEx(&cfg, k_big_level_finish, a, sl); ++nl;
-    cfg.gridDim = dim3(ncta);
-    for (int it = 0; it < op.maxiter; ++it) {
-      if (tma) { cfg.dynamicSmemBytes = 3 * 10240; cudaLaunchKernelEx(&cfg, k_dense_iter_tma<3>, a, sl); }
-      else k_dense_iter<<<ncta, 256, 0, st>>>(a, sl);
-      ++nl;
-    }
-    // (no k_big_level_end: the iteration's serial tail records the level's iteration count)
-  }
-  for (int sl = op.lv_f; sl >= op.lv_l && !fused; --sl) {
-    k_big_level_points<<<pcta, 256, 0, st>>>(a, sl); ++nl;
-    k_big_level_gather<<<ncta, 256, 0, st>>>(a, sl); ++nl;
-    if (pn) { k_big_patch_means<<<pcta, 256, 0, st>>>(a, a.w.ref, 1, 1, ex ? prm.eigen_packet : 0); ++nl; }
-    if (ex) {
-      // the products of all 21 sums (four passes of six rows), then their 21 x 8 chains side by side: one chain pass
-      // (E / 8 dependent additions) per level instead of four
-      for (int pass = 0; pass < 4; ++pass) {
-        if (pk8) k_big_products<1, 16><<<ncta, 256, 0, st>>>(a, pass); else k_big_products<1, 8><<<ncta, 256, 0, st>>>(a, pass);
-        ++nl;
-      }
-      if (pk8) k_big_chains<16><<<21, 64, chain_smem, st>>>(a, 21, a.w.part, 0); else k_big_chains<8><<<21, 64, chain_smem, st>>>(a, 21, a.w.part, 0);
-      ++nl;
-      k_big_hessian_exact_finish<<<1, 32, 0, st>>>(a); ++nl;
+  // bulk-copy staging needs 16-byte aligned streams: point counts and the track's offset multiples of four
+  const bool tma = a.t == 0 && (a.P % 4 == 0) && (a.n_in % 4 == 0);   // t == 0: offset 0
+  big_launch(k_big_init, ncta, 256, 0, false, st, a, fused ? 1 : 0);
+  big_launch(k_big_project_ref, pcta, 256, 0, false, st, a);
+  for (int sl = op.lv_f; sl >= op.lv_l; --sl) {
+    // the level's template and Hessian, then its start (factorisation, state)
+    if (fused) {   // programmatic dependent launches: each kernel becomes resident while its predecessor drains
+      big_launch(k_dense_level, ncta, 256, 0, true, st, a, sl);
+      big_launch(k_big_level_finish, 1, 256, 0, true, st, a, sl);
     } else {
-      k_big_level_hessian<<<ncta, 256, 0, st>>>(a); ++nl;
-      k_big_level_finish<<<1, 256, 0, st>>>(a, sl); ++nl;
+      big_launch(k_big_level_points, pcta, 256, 0, false, st, a, sl);
+      big_launch(k_big_level_gather, ncta, 256, 0, false, st, a, sl);
+      if (pn) big_launch(k_big_patch_means, pcta, 256, 0, false, st, a, a.w.ref, 1, 1, mean_order);
+      if (ex) {
+        // the products of all 21 sums (four passes of six rows), then their 21 x NCH chains side by side: one chain
+        // pass (E / NCH dependent additions) per level instead of four
+        for (int pass = 0; pass < 4; ++pass) big_launch(k_big_products<1, NCH>, ncta, 256, 0, false, st, a, pass);
+        big_launch(k_big_chains<NCH>, 21, 64, chain_smem, false, st, a, 21, a.w.part, 0);
+        big_launch(k_big_hessian_exact_finish, 1, 32, 0, false, st, a, sl);
+      } else {
+        big_launch(k_big_level_hessian, ncta, 256, 0, false, st, a);
+        big_launch(k_big_level_finish, 1, 256, 0, false, st, a, sl);
+      }
     }
     for (int it = 0; it < op.maxiter; ++it) {
-      if (ex && !pn && a.E <= (1 << 18)) {
+      if (fused) {
+        // one launch per iteration; with programmatic dependent launch, iteration k+1 becomes resident while the last
+        // CTA of iteration k still runs the solve, and its first tiles are in flight by the time the pose is published.
+        // k_dense_iter has no griddepcontrol.wait, so it is launched in stream order.
+        if (tma) big_launch(k_dense_iter_tma<3>, ncta, 256, 3 * 10240, true, st, a, sl);
+        else big_launch(k_dense_iter, ncta, 256, 0, false, st, a, sl);
+      } else if (ex && !pn && a.E <= (1 << 18)) {
         // three launches per iteration instead of five: products of all elements, the chains, the serial tail.  For
         // tracks whose launches are latency-bound; beyond ~256 k elements the three streaming kernels below are faster
         // than the fused one.  (The serial tail inside the chain kernel's last CTA was measured: passing the argument
         // block on costs the chain kernel a local copy of it, 26 -> 32 ms per dense TrackPose.)
-        if (pk8) {
-          k_big_iter_fused_exact<16><<<ncta, 256, 0, st>>>(a, sl);
-          k_big_chains<16><<<6, 64, chain_smem, st>>>(a, 6, a.w.part, 1);
-        } else {
-          k_big_iter_fused_exact<8><<<ncta, 256, 0, st>>>(a, sl);
-          k_big_chains<8><<<6, 64, chain_smem, st>>>(a, 6, a.w.part, 1);
-        }
-        nl += 2;
-        k_big_iter_finish<<<1, 256, 0, st>>>(a, sl, 1); ++nl;
-        continue;
-      }
-      k_big_iter_points<<<pcta, 256, 0, st>>>(a, sl); ++nl;
-      if (pn) {
-        k_big_iter_sample<<<ncta, 256, 0, st>>>(a, sl); ++nl;
-        k_big_patch_means<<<pcta, 256, 0, st>>>(a, a.w.pnew, 2, 1, ex ? prm.eigen_packet : 0); ++nl;
-      }
-      if (ex) {
-        if (pn) k_big_iter_pdiff<true><<<ncta, 256, 0, st>>>(a, sl); else k_big_iter_pdiff<false><<<ncta, 256, 0, st>>>(a, sl);
-        ++nl;
-        if (pk8) {
-          k_big_products<0, 16><<<ncta, 256, 0, st>>>(a, 0);
-          k_big_chains<16><<<6, 64, chain_smem, st>>>(a, 6, a.w.part, 1);
-        } else {
-          k_big_products<0, 8><<<ncta, 256, 0, st>>>(a, 0);
-          k_big_chains<8><<<6, 64, chain_smem, st>>>(a, 6, a.w.part, 1);
-        }
-        nl += 2;
+        big_launch(k_big_iter_fused_exact<NCH>, ncta, 256, 0, false, st, a, sl);
+        big_launch(k_big_chains<NCH>, 6, 64, chain_smem, false, st, a, 6, a.w.part, 1);
+        big_launch(k_big_iter_finish, 1, 256, 0, false, st, a, sl, 1);
       } else {
-        if (pn) k_big_iter_elems<true><<<ncta, 256, 0, st>>>(a, sl); else k_big_iter_elems<false><<<ncta, 256, 0, st>>>(a, sl);
-        ++nl;
+        big_launch(k_big_iter_points, pcta, 256, 0, false, st, a, sl);
+        if (pn) {
+          big_launch(k_big_iter_sample, ncta, 256, 0, false, st, a, sl);
+          big_launch(k_big_patch_means, pcta, 256, 0, false, st, a, a.w.pnew, 2, 1, mean_order);
+        }
+        if (ex) {
+          big_launch(pn ? k_big_iter_pdiff<true> : k_big_iter_pdiff<false>, ncta, 256, 0, false, st, a, sl);
+          big_launch(k_big_products<0, NCH>, ncta, 256, 0, false, st, a, 0);
+          big_launch(k_big_chains<NCH>, 6, 64, chain_smem, false, st, a, 6, a.w.part, 1);
+        } else {
+          big_launch(pn ? k_big_iter_elems<true> : k_big_iter_elems<false>, ncta, 256, 0, false, st, a, sl);
+        }
+        big_launch(k_big_iter_finish, 1, 256, 0, false, st, a, sl, ex ? 1 : ncta);
       }
-      k_big_iter_finish<<<1, 256, 0, st>>>(a, sl, ex ? 1 : ncta); ++nl;
     }
-    k_big_level_end<<<1, 1, 0, st>>>(a, sl); ++nl;
   }
-  k_big_final<<<1, 1, 0, st>>>(a); ++nl;
-  for (int k = 0; k < nl; ++k) count_launch();
+  big_launch(k_big_final, 1, 1, 0, false, st, a);
   return cudaGetLastError();
 }
 
-// ==================================================================================================
-// util_getPatch / util_getPatch_grad (utilities.cpp:55-113, 115-189) for a list of patch centres: one CTA per centre,
-// bilinear samples with the reference's placement (ceil(x + 1e-5f) quirk included) and association order, optional
-// mean subtraction of the INTENSITY patch with Eigen's packet sum (utilities.cpp:111-112, 187-188).
-// planes: bit 0 intensity, bit 1 dx, bit 2 dy.  out_* : [npatch][psz*psz].
-// ==================================================================================================
-__global__ void __launch_bounds__(128) k_get_patches(const float* __restrict__ I, const float* __restrict__ dx,
-                                                     const float* __restrict__ dy, int width, int psz, int pszd2,
-                                                     int patchnorm, const float* __restrict__ mids, float* out_I,
-                                                     float* out_dx, float* out_dy) {
-  const int n = psz * psz;
-  const long long g = blockIdx.x;
-  const float mx = mids[2 * g], my = mids[2 * g + 1];
-  const PatchPlace q = patch_place(mx, my, pszd2, width);
-  for (int e = threadIdx.x; e < n; e += blockDim.x) {
-    const int r = e / psz, c = e - r * psz, ad = q.base + r * width + c;
-    if (out_I) out_I[g * n + e] = bilin4(I, ad, width, q.w0, q.w1, q.w2, q.w3);
-    if (out_dx) out_dx[g * n + e] = bilin4(dx, ad, width, q.w0, q.w1, q.w2, q.w3);
-    if (out_dy) out_dy[g * n + e] = bilin4(dy, ad, width, q.w0, q.w1, q.w2, q.w3);
-  }
-  if (patchnorm && out_I) {
-    __shared__ float s_mean;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      float* p = out_I + g * n;
-      s_mean = eigen_sum_serial<4>([&](int e) { return p[e]; }, n) / n;   // tmp_in_e.sum() / novals
-    }
-    __syncthreads();
-    for (int e = threadIdx.x; e < n; e += blockDim.x) out_I[g * n + e] = out_I[g * n + e] - s_mean;
-  }
-}
-
-cudaError_t launch_get_patches(const float* I, const float* dx, const float* dy, int width, int psz, int pszd2,
-                               int patchnorm, int npatch, const float* mids, float* out_I, float* out_dx, float* out_dy,
-                               cudaStream_t stream) {
-  if (npatch <= 0) return cudaSuccess;
-  k_get_patches<<<npatch, 128, 0, stream>>>(I, dx, dy, width, psz, pszd2, patchnorm, mids, out_I, out_dx, out_dy);
-  count_launch();
-  return cudaGetLastError();
-}
-
-// ==================================================================================================
-// NCC hypothesis scoring, run_track_nposes.cpp:271-355.  One CTA per point; three mean-subtracted psz x psz
-// patches (util_getPatch with dopatchnorm, :281) at level lv_l, each divided by its norm (:317-319),
-// corr = max(0, (max(0,<b,r>)*nback^2 + max(0,<r,f>)*nfwd^2) / (nback^2 + nfwd^2)) (:324-348).
-// Stale patches of invalid points never reach the output in the reference (their weight is 0), so points are
-// independent.
-// ==================================================================================================
-__device__ __forceinline__ float cta_sum(float v, float* s_red) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
-  v = warp_sum(v);
-  __syncthreads();
-  if (lane == 0) s_red[warp] = v;
-  __syncthreads();
-  float s = s_red[0];
-  for (int wv = 1; wv < nw; ++wv) s = s + s_red[wv];
-  return s;
-}
-
-__global__ void __launch_bounds__(128) k_ncc(ict_optparam op, CamLevels cam, const float* __restrict__ img_b,
-                                             const float* __restrict__ img_r, const float* __restrict__ img_f,
-                                             int nback, int nfwd, const int64_t* __restrict__ pt_off, int T,
-                                             const float* __restrict__ pb, const float* __restrict__ pr,
-                                             const float* __restrict__ pf, float* __restrict__ out) {
-  extern __shared__ float sm[];
-  __shared__ float s_red[4];
-  __shared__ int s_t;
-  const int n = op.novals, psz = op.psz, l = op.lv_l;
-  const long long g = blockIdx.x;   // global point index
-  if (threadIdx.x == 0) {
-    int lo = 0, hi = T;             // track with pt_off[t] <= g < pt_off[t+1]
-    while (hi - lo > 1) { const int mid = (lo + hi) >> 1; if (pt_off[mid] <= g) lo = mid; else hi = mid; }
-    s_t = lo;
-  }
-  __syncthreads();
-  const int t = s_t;
-  const int64_t off = pt_off[t];
-  const int n_t = (int)(pt_off[t + 1] - off);
-  const int i = (int)(g - off);
-  const float swo = cam.swo[l], sho = cam.sho[l];
-  const int width = cam.width[l];
-  const float* imgs[3] = {img_b, img_r, img_f};
-  const float* pts[3] = {pb, pr, pf};
-  bool val[3];
-  float nrm[3];
-  for (int k = 0; k < 3; ++k) {
-    float* buf = sm + k * n;
-    const float mx = pts[k][2 * off + i], my = pts[k][2 * off + n_t + i];
-    val[k] = (mx > 0) & (my > 0) & (mx < swo) & (my < sho);   // strict, :292,299,307
-    float ss = 0.0f;
-    if (val[k]) {
-      const PatchPlace q = patch_place(mx, my, op.pszd2, width);
-      float s = 0.0f;
-      for (int e = threadIdx.x; e < n; e += blockDim.x) {
-        const int r = e / psz, c = e - r * psz;
-        const float v = bilin4(imgs[k], q.base + r * width + c, width, q.w0, q.w1, q.w2, q.w3);
-        buf[e] = v;
-        s = s + v;
-      }
-      const float m = cta_sum(s, s_red) / n;
-      for (int e = threadIdx.x; e < n; e += blockDim.x) {
-        const float v = buf[e] - m;
-        buf[e] = v;
-        ss = ss + v * v;
-      }
-    } else {
-      for (int e = threadIdx.x; e < n; e += blockDim.x) buf[e] = 0.0f;
-    }
-    nrm[k] = sqrtf(cta_sum(ss, s_red));
-  }
-  float corr = -1.0f;
-  if (val[1]) {
-    float d0 = 0.0f, d1 = 0.0f;
-    for (int e = threadIdx.x; e < n; e += blockDim.x) {
-      const float b = sm[e] / nrm[0], r = sm[n + e] / nrm[1], f = sm[2 * n + e] / nrm[2];
-      d0 = d0 + b * r;
-      d1 = d1 + r * f;
-    }
-    d0 = cta_sum(d0, s_red);
-    d1 = cta_sum(d1, s_red);
-    float corr_br, corr_rf, w0, w1;
-    if (val[0]) { corr_br = 0.0f < d0 ? d0 : 0.0f; w0 = (float)(nback * nback); } else { corr_br = -1.0f; w0 = 0.0f; }
-    if (val[2]) { corr_rf = 0.0f < d1 ? d1 : 0.0f; w1 = (float)(nfwd * nfwd); } else { corr_rf = -1.0f; w1 = 0.0f; }
-    const float v = (corr_br * w0 + corr_rf * w1) / (w0 + w1);
-    corr = 0.0f < v ? v : 0.0f;
-  }
-  if (threadIdx.x == 0) out[g] = corr;
-}
-
-cudaError_t launch_ncc(const ict_optparam& op, const CamLevels& cam, const float* img_b, const float* img_r,
-                       const float* img_f, int nback, int nfwd, const int64_t* pt_off, int T, const float* pb,
-                       const float* pr, const float* pf, float* out, cudaStream_t stream) {
-  // total points = pt_off[T] lives on the device; the caller passes host-known totals through T tracks
-  int64_t total = 0;
-  cudaError_t e = cudaMemcpyAsync(&total, pt_off + T, sizeof(int64_t), cudaMemcpyDeviceToHost, stream);
-  if (e != cudaSuccess) return e;
-  e = cudaStreamSynchronize(stream);
-  if (e != cudaSuccess) return e;
-  if (total <= 0) return cudaSuccess;
-  const size_t smem = sizeof(float) * 3 * (size_t)op.novals;
-  if (smem > 200 * 1024) return cudaErrorInvalidConfiguration;
-  e = set_kernel_attrs<k_ncc>(200 * 1024, -1);
-  if (e != cudaSuccess) return e;
-  k_ncc<<<(unsigned)total, 128, smem, stream>>>(op, cam, img_b, img_r, img_f, nback, nfwd, pt_off, T, pb, pr, pf, out);
-  count_launch();
-  return cudaGetLastError();
+cudaError_t launch_track_big(const TrackParams& prm, int t, int64_t npts, void* work, cudaStream_t st) {
+  BigArgs a;
+  a.prm = prm;
+  bigtrack_work_bytes(prm.op, npts, prm.eigen_packet, work, &a.w);
+  a.t = t;
+  a.n_in = (int)npts;
+  a.P = (int)(npts < prm.op.maxpttrack ? npts : prm.op.maxpttrack);
+  a.E = (long long)a.P * prm.op.novals;
+  return prm.eigen_packet == 8 ? track_big<16>(a, st) : track_big<8>(a, st);
 }
 
 }  // namespace ict

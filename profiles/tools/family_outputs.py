@@ -28,6 +28,12 @@ CASES = {
     "general_o0": (4, 50, FAST, 0, 3), "general_o1": (4, 50, SSE, 1, 3), "general_o2": (8, 100, GENERAL, 0, 3),
     "general_o3": (4, 50, AVX, 0, 3), "general_pn32": (32, 13, FAST, 1, 3),
     "multi_psz1": (1, 3000, FAST, 0, 1), "multi_psz1_sse": (1, 3000, SSE, 0, 1), "multi_psz8": (8, 261, FAST, 0, 2),
+    # the other multi-CTA launch sequences: k_dense_iter (point count not a multiple of 4), the non-fused tree order,
+    # dopatchnorm in both orders, the streaming reference-order iteration (more than 2^18 pixel slots), 8-float packets
+    "multi_psz1_ldg": (1, 3001, FAST, 0, 1), "multi_psz1_o2": (1, 3000, GENERAL, 0, 1),
+    "multi_psz8_pn": (8, 261, FAST, 1, 2), "multi_psz8_sse_pn": (8, 261, SSE, 1, 2),
+    "multi_psz8_sse_big": (8, 4200, SSE, 0, 1), "multi_psz8_avx": (8, 261, AVX, 0, 2),
+    "multi_psz8_avx_big": (8, 4200, AVX, 0, 1),
 }
 TRACE_CAP = 64
 

@@ -214,7 +214,8 @@ def test_chain_in_one_launch_equals_per_frame_launches(ict, kw):
 @pytest.mark.parametrize("kw", [dict(seed=61, w=320, h=240, lv_f=2, psz=1, dense_border=8, tilt=(0.15, -0.1)),
                                 dict(seed=62, w=320, h=240, lv_f=2, psz=1, dense_border=6, tilt=(0.1, 0.2), donorm=1),
                                 dict(seed=63, w=160, h=120, lv_f=1, psz=8, npts=900),
-                                dict(seed=64, w=160, h=120, lv_f=1, psz=8, npts=700, donorm=1, dopatchnorm=1)])
+                                dict(seed=64, w=160, h=120, lv_f=1, psz=8, npts=700, donorm=1, dopatchnorm=1),
+                                dict(seed=65, w=640, h=480, psz=8, npts=4200)])   # 268 800 slots: streaming ref. order
 def test_dense_alignment_multi_cta_path(ict, orc, kw):
     """BASELINE config 4 geometry (reduced): one track with one point per pixel and per-pixel depth, psz = 1 — too
     large for a CTA, so the multi-CTA path runs.  Bit-exact against the oracle in reference order; within fp32

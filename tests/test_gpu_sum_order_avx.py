@@ -91,11 +91,12 @@ def test_k2x8(ict, orc, kw):
                                 dict(seed=61, w=320, h=240, lv_f=2, psz=1, dense_border=8, tilt=(0.15, -0.1)),
                                 dict(seed=62, w=320, h=240, lv_f=2, psz=1, dense_border=6, tilt=(0.1, 0.2), donorm=1),
                                 dict(seed=63, w=160, h=120, lv_f=1, psz=8, npts=900),
-                                dict(seed=64, w=160, h=120, lv_f=1, psz=8, npts=700, donorm=1, dopatchnorm=1)],
-                         ids=["psz8-230", "psz8-240-pn", "dense", "dense-donorm", "psz8-900", "psz8-700-pn"])
+                                dict(seed=64, w=160, h=120, lv_f=1, psz=8, npts=700, donorm=1, dopatchnorm=1),
+                                dict(seed=65, w=640, h=480, psz=8, npts=4200)],
+                         ids=["psz8-230", "psz8-240-pn", "dense", "dense-donorm", "psz8-900", "psz8-700-pn", "psz8-4200"])
 def test_multi_cta_path(ict, orc, kw):
     """Tracks too large for one CTA (dense psz 1 among them): the multi-CTA path with sixteen chains per sum, in its
-    three-launch (no dopatchnorm, small tracks) and five-launch iteration forms."""
+    three-launch (no dopatchnorm, up to 2^18 pixel slots) and five-launch (dopatchnorm, or more slots) iteration forms."""
     case = make_case(**kw)
     check(ict, orc, case, trace_cap=48)
 
