@@ -198,6 +198,52 @@ def teacher_forced_errors(g, o):
     return worst_jtr, worst_dp, nrec
 
 
+def replay_models(orc, case, pyr, p_in=None):
+    """evaluate_model.TrackModel of every track of a case, on the pyramids pyr = ((I, dx, dy) of A, of B) the run
+    used."""
+    from evaluate_model import track_models
+    c = case
+    pa, pb = pyr
+    T = c["T"]
+    p_in = np.zeros((T, 6)) if p_in is None else p_in
+    return track_models(orc, c["op"], c["sc"].fc, c["sc"].cc, c["sc"].wh, [pa[0], pb[0]], [pa[1], pb[1]],
+                        [pa[2], pb[2]], c["pt_off"], c["pts"], np.zeros(T, np.int32), np.ones(T, np.int32), p_in)
+
+
+def check_trajectory(run, op):
+    """Exact checks of a traced run against its own records, for any kernel and sum order:
+      * the records of each track are levels lv_f .. lv_l in turn, the iterations of a level run 0 .. n-1 and n is
+        iters[t, level]; none was cut off (a record is left free);
+      * normdp (rec[14]) is delta_p's l1 norm in the reference's association;
+      * each level went on exactly while keep_iterating(it + 1, normdp, normdp of iteration 0) held;
+      * npixres = novals * sum of the records' visible points."""
+    from evaluate_model import normdp_l1, keep_iterating
+    tr, iters, npix = run["trace"], run["iters"], run["npixres"]
+    T, cap = tr.shape[:2]
+    for t in range(T):
+        n_rec = int((tr[t, :, 0] >= 0).sum())
+        assert n_rec < cap, (t, "trace_cap too small: the trace may be truncated")
+        assert (tr[t, :n_rec, 0] >= 0).all() and (tr[t, n_rec:, 0] == -1).all(), t
+        recs = tr[t, :n_rec]
+        k = 0
+        for j, lv in enumerate(range(op.lv_f, op.lv_l - 1, -1)):
+            n = int(iters[t, j])
+            lr = recs[k:k + n]
+            k += n
+            assert n >= 1 and len(lr) == n, (t, lv, n, len(lr))
+            assert (lr[:, 0] == lv).all() and (lr[:, 1] == np.arange(n)).all(), (t, lv, lr[:, :2])
+            for i, r in enumerate(lr):
+                assert r[14] == normdp_l1(r[8:14]), (t, lv, i, r[14], r[8:14])
+                assert keep_iterating(op, i + 1, r[14], lr[0, 14]) == (i + 1 < n), (t, lv, i, r[14], lr[0, 14])
+        assert k == n_rec, (t, k, n_rec)
+        assert int(npix[t]) == op.novals * int(recs[:, 15].astype(np.int64).sum()), (t, npix[t])
+
+
+def replay_trace_cap(op):
+    """A trace_cap with room for every iteration of every level and one free record."""
+    return (op.lv_f - op.lv_l + 1) * op.maxiter + 1
+
+
 # ---- the seeded cases on which the oracle is compared with the reference's own sources (tests/golden/vs_ref.npz) ----
 REF_CASES = [dict(seed=11), dict(seed=12, donorm=1), dict(seed=13, dopatchnorm=1), dict(seed=14, psz=4, npts=64),
              dict(seed=15, psz=16, npts=12), dict(seed=16, psz=7, npts=20, donorm=1, dopatchnorm=1),
