@@ -231,6 +231,29 @@ int ict_track_batch_dev(ict_tracker* tr, const ict_frames* fs, const int* ref_fr
                         const double* p_in_dev, double* p_out_dev, int* iters_dev, float* trace_dev,
                         int trace_cap, int64_t* npixres_dev, void* stream);
 
+/* SetPose at one pose and TrackPose from another.  For each track t, SetPose runs exactly as in ict_track_batch at
+ * p_ref[t]: donorm's normalisation, the template and steepest-descent state, Get2DPoints.  TrackPose then runs with
+ * the fp32 pose coefficients starting at setpose_se3(p_start[t]), normalised with the same track's (meanshift,
+ * varval), instead of at setpose_se3(p_ref[t]) — what a caller of the reference's classes gets from
+ * pose.setpose_se3(p_start, ...) between SetPose and TrackPose.  Use it to start from a better guess than the
+ * reference frame's pose: a constant-velocity or IMU prediction, a hypothesis of ict_pose_hypotheses, the best
+ * candidate of ict_track_evaluate_poses.  Nothing else changes: the stop rule, the trace, iters, npixres,
+ * p_out = getPose_se3 of the final coefficients, keep_state (the carried template depends on p_ref only), teacher
+ * forcing, the robustness flags, the sum orders, empty tracks, NaN one-point donorm tracks and the maxpttrack cap.
+ *   p_start == NULL, or a row with p_start[t] == p_ref[t], gives the same bits as ict_track_batch in every output.
+ *   A non-finite row of p_start places every point of the track outside the new image, as a NaN placement does: the
+ *   track runs one iteration per level on no pixel and returns a non-finite pose.
+ * p_ref, p_start, p_out: double[T*6]; the other arguments and the errors are those of ict_track_batch, and so are
+ * the kernels: a start pose adds no launch. */
+int ict_track_batch_from(ict_tracker* tr, const ict_frames* fs, const int* ref_frame, const int* new_frame,
+                         const double* p_ref, const double* p_start, double* p_out, int* iters, float* trace,
+                         int trace_cap, int64_t* npixres);
+/* Device-pointer form of ict_track_batch_from (p_start_dev may be NULL), as ict_track_batch_dev. */
+int ict_track_batch_from_dev(ict_tracker* tr, const ict_frames* fs, const int* ref_frame_dev,
+                             const int* new_frame_dev, const double* p_ref_dev, const double* p_start_dev,
+                             double* p_out_dev, int* iters_dev, float* trace_dev, int trace_cap,
+                             int64_t* npixres_dev, void* stream);
+
 /* One forward (step=+1) or backward (step=-1) chain of run_track_nposes.cpp:232-239 / :251-258 for all T tracks:
  * for k in 0..nsteps-1: SetPose(p, frame[first+k*step] as ref, frame[first+(k+1)*step] as new); TrackPose(p).
  * poses_out: double[(nsteps+1)*T*6], entry 0 = p_in. Host buffers.  The poses of the chain never leave the device

@@ -74,6 +74,10 @@ SIGNATURES = {
                                   C.c_void_p, C.c_int, C.c_void_p]),
     "ict_track_batch_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                       C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
+    "ict_track_batch_from": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
+    "ict_track_batch_from_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "ict_frames_upload_u8_stream": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "ict_tracker_set_points_stream": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "ict_track_batch_stream": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
@@ -299,23 +303,35 @@ class Tracker:
         _check(lib().ict_tracker_set_points_dev(self.h_, T, C.c_void_p(pt_off_ptr), C.c_void_p(pts_ptr), total,
                                                 max_pts, C.c_void_p(stream)))
 
-    def track_batch(self, frames, ref_frame, new_frame, p_in, trace_cap=0):
+    def track_batch(self, frames, ref_frame, new_frame, p_in, trace_cap=0, p_start=None):
+        """SetPose at p_in and TrackPose from there; with p_start (broadcast like p_in), TrackPose starts from p_start
+        instead while the template stays at p_in (ict_track_batch_from)."""
         T, L = self.T, self.L
         ref_frame = np.ascontiguousarray(np.broadcast_to(ref_frame, (T,)), np.int32)
         new_frame = np.ascontiguousarray(np.broadcast_to(new_frame, (T,)), np.int32)
         p_in = np.ascontiguousarray(np.broadcast_to(p_in, (T, 6)), np.float64)
         p_out = np.zeros((T, 6), np.float64); iters = np.zeros((T, L), np.int32); npix = np.zeros(T, np.int64)
         trace = np.zeros((T, trace_cap, TRACE_FLOATS), np.float32) if trace_cap else None
-        _check(lib().ict_track_batch(self.h_, frames.h_, _p(ref_frame), _p(new_frame), _p(p_in), _p(p_out), _p(iters),
-                                     _p(trace), trace_cap, _p(npix)))
+        tail = (_p(p_out), _p(iters), _p(trace), trace_cap, _p(npix))
+        if p_start is None:
+            _check(lib().ict_track_batch(self.h_, frames.h_, _p(ref_frame), _p(new_frame), _p(p_in), *tail))
+        else:
+            p_start = np.ascontiguousarray(np.broadcast_to(p_start, (T, 6)), np.float64)
+            _check(lib().ict_track_batch_from(self.h_, frames.h_, _p(ref_frame), _p(new_frame), _p(p_in), _p(p_start),
+                                              *tail))
         return dict(p_out=p_out, iters=iters, npixres=npix, trace=trace)
 
     def track_batch_dev(self, frames, ref_ptr, new_ptr, p_in_ptr, p_out_ptr, iters_ptr=0, npix_ptr=0, trace_ptr=0,
-                        trace_cap=0, stream=0):
+                        trace_cap=0, stream=0, p_start_ptr=0):
+        """Device-pointer form of track_batch; p_start_ptr: device double[T*6] start poses, or 0."""
         v = C.c_void_p
-        _check(lib().ict_track_batch_dev(self.h_, frames.h_, v(ref_ptr), v(new_ptr), v(p_in_ptr), v(p_out_ptr),
-                                         v(iters_ptr) if iters_ptr else None, v(trace_ptr) if trace_ptr else None,
-                                         trace_cap, v(npix_ptr) if npix_ptr else None, v(stream)))
+        tail = (v(p_out_ptr), v(iters_ptr) if iters_ptr else None, v(trace_ptr) if trace_ptr else None, trace_cap,
+                v(npix_ptr) if npix_ptr else None, v(stream))
+        if p_start_ptr:
+            _check(lib().ict_track_batch_from_dev(self.h_, frames.h_, v(ref_ptr), v(new_ptr), v(p_in_ptr),
+                                                  v(p_start_ptr), *tail))
+        else:
+            _check(lib().ict_track_batch_dev(self.h_, frames.h_, v(ref_ptr), v(new_ptr), v(p_in_ptr), *tail))
 
     def track_sequence(self, frames, first, nsteps, step, p_in):
         T, L = self.T, self.L

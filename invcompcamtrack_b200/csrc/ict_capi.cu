@@ -469,7 +469,7 @@ struct ict_tracker {
   unsigned robust = 0;         // ict_tracker_set_robust
   int keep_state = 0;          // knob "keep_state": template arrays persist between TrackPose calls until the next Set3Dpoints
   bool state_valid = false;
-  DevBuf pt_off, pts, pt3d, norm, p_in, p_out, iters, npix, trace, pt2d, rf, nf, big, teacher, state;
+  DevBuf pt_off, pts, pt3d, norm, p_in, p_start, p_out, iters, npix, trace, pt2d, rf, nf, big, teacher, state;
   DevBuf ev, ev_in;              // ict_track_evaluate: scratch + outputs, per-call inputs (its own: no other call's data)
   int teacher_cap = 0;           // ict_tracker_set_teacher: records per track of the staged teacher poses (0: none)
   // several multi-CTA tracks in one call run on up to ICT_BIG_LANES streams side by side (each track is a chain of a few
@@ -682,6 +682,7 @@ struct TrackCall {
   int seq_n = 0, seq_step = 0;
   const int *h_rf = nullptr, *h_nf = nullptr;
   const double* p_in = nullptr;
+  const double* p_start = nullptr;   // null: TrackPose starts at p_in
   double* p_out = nullptr;
   int* iters = nullptr;
   float* trace = nullptr;
@@ -741,6 +742,7 @@ static int run_tracks(ict_tracker* tr, const TrackCall& c, cudaStream_t st) {
   prm.fixed_ref = c.fixed_ref;
   prm.fixed_new = c.fixed_new;
   prm.p_in = c.p_in;
+  prm.p_start = c.p_start;
   prm.p_out = c.p_out;
   prm.iters = c.iters;
   prm.trace = c.trace;
@@ -776,15 +778,16 @@ static int run_tracks(ict_tracker* tr, const TrackCall& c, cudaStream_t st) {
   return ICT_OK;
 }
 
-int ict_track_batch_dev(ict_tracker* tr, const ict_frames* fs, const int* ref_frame_dev, const int* new_frame_dev,
-                        const double* p_in_dev, double* p_out_dev, int* iters_dev, float* trace_dev, int trace_cap,
-                        int64_t* npixres_dev, void* stream) {
-  if (!ref_frame_dev || !new_frame_dev || !p_in_dev || !p_out_dev) return fail(ICT_ERR_BAD_ARG, "null device pointer");
+int ict_track_batch_from_dev(ict_tracker* tr, const ict_frames* fs, const int* ref_frame_dev, const int* new_frame_dev,
+                             const double* p_ref_dev, const double* p_start_dev, double* p_out_dev, int* iters_dev,
+                             float* trace_dev, int trace_cap, int64_t* npixres_dev, void* stream) {
+  if (!ref_frame_dev || !new_frame_dev || !p_ref_dev || !p_out_dev) return fail(ICT_ERR_BAD_ARG, "null device pointer");
   TrackCall c;
   c.fs = fs;
   c.rf = ref_frame_dev;
   c.nf = new_frame_dev;
-  c.p_in = p_in_dev;
+  c.p_in = p_ref_dev;
+  c.p_start = p_start_dev;
   c.p_out = p_out_dev;
   c.iters = iters_dev;
   c.trace = trace_dev;
@@ -793,16 +796,24 @@ int ict_track_batch_dev(ict_tracker* tr, const ict_frames* fs, const int* ref_fr
   return run_tracks(tr, c, (cudaStream_t)stream);
 }
 
+int ict_track_batch_dev(ict_tracker* tr, const ict_frames* fs, const int* ref_frame_dev, const int* new_frame_dev,
+                        const double* p_in_dev, double* p_out_dev, int* iters_dev, float* trace_dev, int trace_cap,
+                        int64_t* npixres_dev, void* stream) {
+  return ict_track_batch_from_dev(tr, fs, ref_frame_dev, new_frame_dev, p_in_dev, nullptr, p_out_dev, iters_dev,
+                                  trace_dev, trace_cap, npixres_dev, stream);
+}
+
 // The per-call inputs of ict_track_batch*: checks the frame indices, reserves the buffers of T tracks (and c.trace_cap
-// trace records per track), copies the frame indices and start poses in (on `lane` when one is given, on st otherwise)
-// and points c at the buffers.
+// trace records per track), copies the frame indices, the SetPose poses and the TrackPose start poses (when p_start is
+// set) in (on `lane` when one is given, on st otherwise) and points c at the buffers.
 static int stage_batch(ict_tracker* tr, TrackCall& c, const int* ref_frame, const int* new_frame, const double* p_in,
-                       CopyLane* lane, cudaStream_t st) {
+                       const double* p_start, CopyLane* lane, cudaStream_t st) {
   const int T = tr->T, L = tr->op.lv_f - tr->op.lv_l + 1;
   if (frames_in_range(c.fs, T, ref_frame, new_frame)) return ICT_ERR_BAD_ARG;
   CU(tr->rf.reserve(sizeof(int) * (size_t)T));
   CU(tr->nf.reserve(sizeof(int) * (size_t)T));
   CU(tr->p_in.reserve(sizeof(double) * 6 * (size_t)T));
+  if (p_start) CU(tr->p_start.reserve(sizeof(double) * 6 * (size_t)T));
   CU(tr->p_out.reserve(sizeof(double) * 6 * (size_t)T));
   CU(tr->iters.reserve(sizeof(int) * (size_t)T * L));
   CU(tr->npix.reserve(sizeof(long long) * (size_t)T));
@@ -812,10 +823,12 @@ static int stage_batch(ict_tracker* tr, TrackCall& c, const int* ref_frame, cons
   CU(cudaMemcpyAsync(tr->rf.p, ref_frame, sizeof(int) * (size_t)T, cudaMemcpyHostToDevice, cs));
   CU(cudaMemcpyAsync(tr->nf.p, new_frame, sizeof(int) * (size_t)T, cudaMemcpyHostToDevice, cs));
   CU(cudaMemcpyAsync(tr->p_in.p, p_in, sizeof(double) * 6 * (size_t)T, cudaMemcpyHostToDevice, cs));
+  if (p_start) CU(cudaMemcpyAsync(tr->p_start.p, p_start, sizeof(double) * 6 * (size_t)T, cudaMemcpyHostToDevice, cs));
   if (lane) CU(lane->publish(st));
   c.rf = tr->rf.as<int>();
   c.nf = tr->nf.as<int>();
   c.p_in = tr->p_in.as<double>();
+  c.p_start = p_start ? tr->p_start.as<double>() : nullptr;
   c.p_out = tr->p_out.as<double>();
   c.iters = tr->iters.as<int>();
   c.npix = tr->npix.as<long long>();
@@ -823,16 +836,17 @@ static int stage_batch(ict_tracker* tr, TrackCall& c, const int* ref_frame, cons
   return ICT_OK;
 }
 
-int ict_track_batch(ict_tracker* tr, const ict_frames* fs, const int* ref_frame, const int* new_frame,
-                    const double* p_in, double* p_out, int* iters, float* trace, int trace_cap, int64_t* npixres) {
-  if (!tr || !fs || !ref_frame || !new_frame || !p_in || !p_out) return fail(ICT_ERR_BAD_ARG, "null argument");
+int ict_track_batch_from(ict_tracker* tr, const ict_frames* fs, const int* ref_frame, const int* new_frame,
+                         const double* p_ref, const double* p_start, double* p_out, int* iters, float* trace,
+                         int trace_cap, int64_t* npixres) {
+  if (!tr || !fs || !ref_frame || !new_frame || !p_ref || !p_out) return fail(ICT_ERR_BAD_ARG, "null argument");
   const int T = tr->T;
   if (points_current(tr)) return ICT_ERR_BAD_ARG;
   const int L = tr->op.lv_f - tr->op.lv_l + 1;
   TrackCall c;
   c.fs = fs;
   c.trace_cap = trace && trace_cap > 0 ? trace_cap : 0;
-  if (int rc = stage_batch(tr, c, ref_frame, new_frame, p_in, nullptr, 0)) return rc;
+  if (int rc = stage_batch(tr, c, ref_frame, new_frame, p_ref, p_start, nullptr, 0)) return rc;
   c.h_rf = ref_frame;   // the multi-CTA path runs the tracks one after the other, each with its own frame pair
   c.h_nf = new_frame;
   if (int rc = run_tracks(tr, c, 0)) return rc;
@@ -846,6 +860,11 @@ int ict_track_batch(ict_tracker* tr, const ict_frames* fs, const int* ref_frame,
   return ICT_OK;
 }
 
+int ict_track_batch(ict_tracker* tr, const ict_frames* fs, const int* ref_frame, const int* new_frame,
+                    const double* p_in, double* p_out, int* iters, float* trace, int trace_cap, int64_t* npixres) {
+  return ict_track_batch_from(tr, fs, ref_frame, new_frame, p_in, nullptr, p_out, iters, trace, trace_cap, npixres);
+}
+
 int ict_track_batch_stream(ict_tracker* tr, const ict_frames* fs, const int* ref_frame, const int* new_frame,
                            const double* p_in, double* p_out, int* iters, int64_t* npixres, void* stream) {
   if (!tr || !fs || !ref_frame || !new_frame || !p_in || !p_out) return fail(ICT_ERR_BAD_ARG, "null argument");
@@ -857,7 +876,7 @@ int ict_track_batch_stream(ict_tracker* tr, const ict_frames* fs, const int* ref
   const int L = tr->op.lv_f - tr->op.lv_l + 1;
   TrackCall c;
   c.fs = fs;
-  if (int rc = stage_batch(tr, c, ref_frame, new_frame, p_in, &tr->lane_in, st)) return rc;
+  if (int rc = stage_batch(tr, c, ref_frame, new_frame, p_in, nullptr, &tr->lane_in, st)) return rc;
   if (int rc = run_tracks(tr, c, st)) return rc;
   CU(tr->lane.done(st));
   CU(tr->lane_in.done(st));

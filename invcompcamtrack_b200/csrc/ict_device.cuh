@@ -317,6 +317,21 @@ __device__ __forceinline__ void track_setpose(const double* p_in, const double* 
   setpose_se3(p_in + 6 * (int64_t)t, donorm, norm + 4 * (int64_t)t, norm[4 * (int64_t)t + 3], p, G);
 }
 
+// SetPose of track t at row t of p_ref with TrackPose's start of its own (prm.p_start, ict_track_batch_from).  One
+// thread.  Gt receives the G of p_ref, the pose save_rotated_point projects the template at; p/G receive the
+// coefficients TrackPose starts from: setpose_se3 of row t of p_start, normalised with the track's own (meanshift,
+// varval), or without p_start those of p_ref.  The kernels pass as Gt 12 floats of storage that no thread touches
+// before the first level writes it (the level's Hessian sums, the LU factors of the multi-CTA path), so the start
+// pose costs no shared memory and no barrier.  The template is always projected from Gt: choosing between G and Gt
+// per call would cost the register-bound kernels (K2v2) spills in their iteration loops.
+__device__ __forceinline__ void track_setpose_from(const TrackParams& prm, const double* p_ref, int t, bool donorm,
+                                                   float* p, float* G, float* Gt) {
+  track_setpose(p_ref, prm.norm, t, donorm, p, G);
+#pragma unroll
+  for (int k = 0; k < 12; ++k) Gt[k] = G[k];
+  if (prm.p_start) track_setpose(prm.p_start, prm.norm, t, donorm, p, G);
+}
+
 // project_pt_save_rotated (pose.cpp:400-488) of point i at the SetPose pose G: the camera-frame point into Xc/Yc/Zc
 // (SAVE), and Get2DPoints() (odometer.h:30), the point at level lv_l, into pt2d_out (when set)
 template <bool SAVE = true, typename I>

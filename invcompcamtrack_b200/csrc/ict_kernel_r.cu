@@ -230,7 +230,7 @@ __global__ void __launch_bounds__((NPROD + 2) * 32, NPROD == 4 ? 2 : 1) k_track_
       S.Z[i] = q[2 * (int64_t)n_in + i];
     }
   }
-  if (tid == 0) track_setpose(prm.p_in, prm.norm, t, donorm, S.p, S.G);
+  if (tid == 0) track_setpose_from(prm, prm.p_in, t, donorm, S.p, S.G, S.Hsum);
   if (tid >= 32 && tid < 32 + KR_MAXU) {
     mbar_init(&S.win_full[tid - 32], 1);
     S.pd_flag[tid - 32] = 0u;
@@ -245,7 +245,7 @@ __global__ void __launch_bounds__((NPROD + 2) * 32, NPROD == 4 ? 2 : 1) k_track_
   }
   mbar_fence_init();
   __syncthreads();
-  for (int i = tid; i < P; i += nt) save_rotated_point(prm, S.G, off, n_in, i, S.X[i], S.Y[i], S.Z[i], S.Xc, S.Yc, S.Zc);
+  for (int i = tid; i < P; i += nt) save_rotated_point(prm, S.Hsum, off, n_in, i, S.X[i], S.Y[i], S.Z[i], S.Xc, S.Yc, S.Zc);
   __syncthreads();
 
   float* trace = track_trace(prm, t);

@@ -134,9 +134,9 @@ __global__ void __launch_bounds__(32 * NW, NW == 8 ? 2 : 1) k_track_v8(const Tra
       for (int k = 0; k < 12; ++k) s_AB[i * 12 + k] = 0.0f;
     }
   }
-  if (tid == 0) track_setpose(step_p_in, prm.norm, t, donorm, S.p, S.G);
+  if (tid == 0) track_setpose_from(prm, step_p_in, t, donorm, S.p, S.G, S.Hsum);   // K2v8 leaves S.Hsum unused
   __syncthreads();
-  for (int i = tid; i < P; i += nt) save_rotated_point(prm, S.G, off, n_in, i, s_X[i], s_Y[i], s_Z[i], s_Xc, s_Yc, s_Zc);
+  for (int i = tid; i < P; i += nt) save_rotated_point(prm, S.Hsum, off, n_in, i, s_X[i], s_Y[i], s_Z[i], s_Xc, s_Yc, s_Zc);
   __syncthreads();
 
   float* trace = TRACE ? track_trace(prm, t) : nullptr;

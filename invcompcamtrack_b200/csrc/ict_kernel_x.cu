@@ -135,13 +135,13 @@ __global__ void __launch_bounds__(256, 2) k_track_x(const TrackParams prm) {
       for (int k = 0; k < 12; ++k) s_AB[i * 12 + k] = 0.0f;
     }
   }
-  if (tid == 0) track_setpose(prm.p_in, prm.norm, t, donorm, S.p, S.G);
+  if (tid == 0) track_setpose_from(prm, prm.p_in, t, donorm, S.p, S.G, S.Hsum);
   if (tid >= 32 && tid < 34) {
     mbar_init(&S.full[tid - 32], 32 * KX_PROD);
     mbar_init(&S.empty[tid - 32], 32);
   }
   __syncthreads();
-  for (int i = tid; i < P; i += nt) save_rotated_point(prm, S.G, off, n_in, i, s_X[i], s_Y[i], s_Z[i], s_Xc, s_Yc, s_Zc);
+  for (int i = tid; i < P; i += nt) save_rotated_point(prm, S.Hsum, off, n_in, i, s_X[i], s_Y[i], s_Z[i], s_Xc, s_Yc, s_Zc);
   __syncthreads();
 
   float* trace = track_trace(prm, t);

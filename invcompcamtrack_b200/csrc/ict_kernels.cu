@@ -478,13 +478,13 @@ __global__ void __launch_bounds__(256) k_track(const TrackParams prm) {
   }
   // ---- SetPose: setpose_se3 (pose.cpp:25-76) ----------------------------------------------------------
   if (tid == 0) {
-    track_setpose(prm.p_in, prm.norm, t, donorm, S.p, S.G);
+    track_setpose_from(prm, prm.p_in, t, donorm, S.p, S.G, S.Hsum);
     S.npix = 0;
     S.nvis = 0;
   }
   __syncthreads();
   // project_pt_save_rotated: camera-frame points frozen for the whole TrackPose
-  for (int i = tid; i < P; i += nt) save_rotated_point(prm, S.G, off, n_in, i, s_X[i], s_Y[i], s_Z[i], s_Xc, s_Yc, s_Zc);
+  for (int i = tid; i < P; i += nt) save_rotated_point(prm, S.Hsum, off, n_in, i, s_X[i], s_Y[i], s_Z[i], s_Xc, s_Yc, s_Zc);
   __syncthreads();
 
   float* trace = track_trace(prm, t);
@@ -832,11 +832,11 @@ __global__ void __launch_bounds__(256, MINB) k_track_fast(const TrackParams prm)
     }
   }
   if (tid == 0) {
-    track_setpose(prm.p_in, prm.norm, t, donorm, S.p, S.G);
+    track_setpose_from(prm, prm.p_in, t, donorm, S.p, S.G, S.Hsum);
     S.npix = 0;
   }
   __syncthreads();
-  for (int i = tid; i < P; i += nt) save_rotated_point(prm, S.G, off, n_in, i, s_X[i], s_Y[i], s_Z[i], s_Xc, s_Yc, s_Zc);
+  for (int i = tid; i < P; i += nt) save_rotated_point(prm, S.Hsum, off, n_in, i, s_X[i], s_Y[i], s_Z[i], s_Xc, s_Yc, s_Zc);
   __syncthreads();
 
   float* trace = track_trace(prm, t);
@@ -1118,6 +1118,7 @@ TrackKernel select_track_kernel(const ict_optparam& op, int max_pts, int sum_mod
 cudaError_t launch_track(const TrackParams& prm, TrackKernel k, int max_pts, cudaStream_t stream) {
   if (prm.T <= 0) return cudaSuccess;
   if (prm.seq_n > 1 && k != TrackKernel::V8) return cudaErrorInvalidConfiguration;   // only K2v8 loops over frames
+  if (prm.seq_n > 1 && prm.p_start) return cudaErrorInvalidConfiguration;         // a chain starts each step at p_in
   const int P = track_pcap(prm.op, max_pts);
   const long long E = (long long)P * prm.op.novals;
   const int nt = E >= 2048 ? 256 : (E >= 512 ? 128 : 64);

@@ -33,7 +33,8 @@ struct TrackParams {
   const int64_t* pt_off;           // [T+1]
   const float* pt3d;               // per track: X block, Y block, Z block (n_t each) at 3*pt_off[t]
   const double* norm;              // per track: meanshift[3], varval
-  const double* p_in;              // [T*6]
+  const double* p_in;              // [T*6] the SetPose pose: the template is projected at it
+  const double* p_start;           // [T*6] or null (p_in): the pose TrackPose starts from (ict_track_batch_from)
   double* p_out;                   // [T*6]
   int* iters;                      // [T*L] or null
   float* trace;                    // [T*trace_cap*16] or null
@@ -123,7 +124,7 @@ TrackKernel select_track_kernel(const ict_optparam& op, int max_pts, int sum_mod
                                 int no_k2r, int tma_ok);
 size_t track_smem_bytes(const ict_optparam& op, int max_pts, int sum_mode);
 // Launches kernel k, which select_track_kernel chose for max_pts; cudaErrorInvalidConfiguration for MultiCta (the
-// caller runs launch_track_big) and for a chain (seq_n > 1) on any kernel but V8.
+// caller runs launch_track_big), for a chain (seq_n > 1) on any kernel but V8 and for a chain with start poses.
 cudaError_t launch_track(const TrackParams& prm, TrackKernel k, int max_pts, cudaStream_t stream);
 
 // Each kernel's own constraints: *_supported / *_smem_bytes.  The launchers assume select_track_kernel chose them.

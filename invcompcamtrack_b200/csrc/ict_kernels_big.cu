@@ -17,7 +17,7 @@ namespace ict {
 struct BigState {
   float G[12];
   float p[6];
-  Lu6 lu;
+  Lu6 lu;                   // before the first level: lu.lu[0..11] = the template's pose (track_setpose_from)
   float normdp, normdp_init;
   int cont, it, nvis, trace_n, level_it;
   unsigned ticket;          // CTAs that have published their partial sums in the running fused-iteration launch
@@ -272,7 +272,7 @@ __global__ void k_big_init(const BigArgs a, int fused) {
   if (gid == 0) {
     BigState* S = a.w.st;
     const ict_optparam& op = a.prm.op;
-    track_setpose(a.prm.p_in, a.prm.norm, a.t, op.donorm != 0, S->p, S->G);
+    track_setpose_from(a.prm, a.prm.p_in, a.t, op.donorm != 0, S->p, S->G, S->lu.lu);
     S->npix = 0;
     S->nvis = 0;
     S->trace_n = 0;
@@ -287,7 +287,7 @@ __global__ void k_big_project_ref(const BigArgs a) {
   const int64_t off = a.prm.pt_off[a.t];
   const float* q = a.prm.pt3d + 3 * off;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < a.P; i += (long long)gridDim.x * blockDim.x)
-    save_rotated_point(a.prm, S->G, off, a.n_in, i, q[i], q[a.n_in + i], q[2 * (int64_t)a.n_in + i], a.w.Xc, a.w.Yc,
+    save_rotated_point(a.prm, S->lu.lu, off, a.n_in, i, q[i], q[a.n_in + i], q[2 * (int64_t)a.n_in + i], a.w.Xc, a.w.Yc,
                        a.w.Zc);
 }
 
